@@ -8,8 +8,11 @@ Headline workload at any N: BASELINE config 2 per GPU -- 1M synthetic 150 bp x 1
 local (Smith-Waterman) score + end cell + traceback ops; even pairs mutated copies, odd pairs random
 (seed 20250002 + rank).  Shards are independent: no data-path collective ("weak" scaling).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--pairs P] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--pairs P] [--impl ours|reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
+
+--dump-outputs DIR writes what the last timed step returned (see write_outputs), so that two builds can be compared
+output for output on the same seeded inputs.
 
 One JSON line on stdout (rank 0):
   value      device-resident inputs, CUDA-event timed, max over ranks
@@ -58,7 +61,13 @@ def parse():
     ap.add_argument("--extra-timeout", type=int, default=420, help="seconds the sub-records may take before the headline is printed without them")
     ap.add_argument("--c4-len", type=int, default=1_000_000)
     ap.add_argument("--c5-pairs", type=int, default=100_000)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's results as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's results; it cannot be combined with --impl reference")
+    return args
 
 
 def config_dict(args, world):
@@ -221,6 +230,44 @@ class Timer:
         self.barrier()
         ms = e0.elapsed_time(e1) / steps
         return sharding.max_over_ranks(ms, self.dev) if self.world > 1 else ms      # a rank-local timer must not enter a collective
+
+
+DUMP_BYTES = 60_000_000     # the data of all files of one --dump-outputs run: under 64 MB with the .npy headers
+DUMP_SEED = 20250010
+
+
+def snapshot_outputs(torch, dItems, dOps, n, stride, world):
+    """What the headline call hands back to its caller after a step: every pair's result record (psa_batch_item) and
+    its traceback op words, copied to the host.  When all pairs do not fit in DUMP_BYTES, a seeded sample of them (the
+    same on every run).  Returns (pair index, records [k, 10] int32, op words [k, stride] uint32)."""
+    from cse305_parallel_sequence_alignment_b200.capi import ITEM_DTYPE
+    fields = len(ITEM_DTYPE.names)
+    per_pair = 8 * (1 + fields + stride)
+    k = min(n, DUMP_BYTES // world // per_pair)
+    idx = np.arange(n) if k == n else np.sort(np.random.default_rng(DUMP_SEED).choice(n, k, replace=False))
+    sel = torch.from_numpy(idx).to(dItems.device)
+    items = dItems.view(n, fields).index_select(0, sel).cpu().numpy()
+    ops = dOps.view(n, stride).index_select(0, sel).cpu().numpy().view(np.uint32)
+    return idx, items, ops
+
+
+def write_outputs(path, snapshot, n, rank, world, dist):
+    """DIR/<name>.npy as float64, which holds every int32 and uint32 exactly: one file per field of psa_batch_item,
+    ops.npy ([pairs, stride] op words) and pair_index.npy (which pairs were kept).  With several ranks, rank 0 writes
+    every rank's pairs, rank r's pair i as pair_index r * n + i."""
+    from cse305_parallel_sequence_alignment_b200.capi import ITEM_DTYPE
+    idx, items, ops = snapshot
+    if world > 1:
+        parts = [None] * world if rank == 0 else None
+        dist.gather_object((idx + rank * n, items, ops), parts, dst=0)
+        if rank != 0:
+            return
+        idx, items, ops = (np.concatenate(x) for x in zip(*parts))
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "pair_index.npy"), idx.astype(np.float64))
+    for c, name in enumerate(ITEM_DTYPE.names):
+        np.save(os.path.join(path, f"{name}.npy"), items[:, c].astype(np.float64))
+    np.save(os.path.join(path, "ops.npy"), ops.astype(np.float64))
 
 
 def host_pack_record(psa, A, B):
@@ -504,6 +551,9 @@ def main():
     launches0 = ctx.launches
     kernel_ms = T.run(step_device, args.steps, 0)
     launches = ctx.launches - launches0
+    snapshot = None
+    if args.dump_outputs:                # before the fill-only loop below overwrites the records
+        snapshot = snapshot_outputs(torch, dItems, dOps, n, stride, world)
 
     # ---- the dominant kernel alone: same fill launches (direction codes included), walk kernels not launched ----
     ctx.set_option("pack_skip_walk", 1)      # measurement hook (csrc/psa_internal.h), not an environment switch
@@ -532,6 +582,8 @@ def main():
         ctx.set_option("pack_serial_fills", default_serial)
     e2e_bytes_ms = wall(step_e2e_bytes, max(3, args.steps // 2))
     clocks = sampler.stop()              # sampled while the GPU was busy (device-timed loop + e2e loops)
+    if snapshot is not None:             # written once the clocks are no longer sampled
+        write_outputs(args.dump_outputs, snapshot, n, rank, world, dist)
     same_bytes = bool(np.array_equal(items_np["score"], items16_np["score"]) and
                       np.array_equal(items_np["aln_len"].astype(np.int64), items16_np["aln_len"].astype(np.int64)))
 

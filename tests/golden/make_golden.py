@@ -10,8 +10,12 @@ Runs only in the build container (needs /root/reference and oracle/_ref built by
                     md5 + op counts for long ones) as produced by the reference's Subproblem
   random_small.json 400 seeded random/mutated pairs with the reference's full answers
   typed_small.json  the 36 (start_type, end_type) border variants of Subproblem, 8 pairs each
+  ref_tables.json   the inputs of tests/test_oracle_golden.py's two full-table comparisons, each with an md5 of
+                    T1, T2 and T3, the corner, the end state, the node states and (random pairs) an md5 of the printed rows;
+                    taken from the reference when oracle/_ref is built, else from the oracle, and the file's
+                    "source" says which (ref_tables_fixture, which can run on its own)
 
-Usage:  python tests/golden/make_golden.py
+Usage:  python tests/golden/make_golden.py [tables]
 """
 import hashlib
 import json
@@ -25,6 +29,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
 from oracle import pyoracle as po  # noqa: E402
+from tests.helpers import py_random_pair, table_record  # noqa: E402
 
 REF_DATA = "/root/reference/gene_sequences_test"
 HEAD = 13400
@@ -130,6 +135,7 @@ def main():
         cases.append(c)
     json.dump(cases, open(os.path.join(HERE, "random_small.json"), "w"))
     typed_fixture()
+    ref_tables_fixture()
     print("golden fixtures written:", len(kat), "KATs,", len(cases), "random cases")
 
 
@@ -159,5 +165,48 @@ def typed_fixture():
     print("typed fixture written:", len(cases), "cases")
 
 
+def _ref_record(a, b, g, h, p, start_type=-1, end_type=-1):
+    if po.have_ref():
+        corner, end_state, nodes, tables = po.ref_subproblem(a, b, g, h, p=p, start_type=start_type, end_type=end_type,
+                                                             want_tables=True)
+        ra, rb = po.ref_rows(a, b, nodes)
+        return table_record(tables, corner, end_state, bytes(int(x) for x in nodes[:, 2]), ra, rb)
+    al, tables = po.align(a, b, g, h, start_type=start_type, end_type=end_type, want_tables=True)
+    return table_record(tables, (al.t1, al.t2, al.t3), al.end_state, al.ops, al.row_a, al.row_b)
+
+
+def ref_tables_fixture():
+    """The exact seeded draws of test_oracle_equals_reference_random (random.Random(7)) and
+    test_oracle_equals_reference_typed_tables (random.Random(5)), with their answers."""
+    out = {"source": "reference (oracle/_ref)" if po.have_ref() else
+           "oracle (gotoh_oracle.c): the compiled reference was not available when this file was written",
+           "random": [], "typed": []}
+    rnd = random.Random(7)
+    for t in range(400):
+        a, b = py_random_pair(rnd, alpha=rnd.choice([b"ACGT", b"AC", b"ACGTN"]))
+        g, h = rnd.choice([(1, 2), (1, 2), (2, 1), (1, 0), (0, 3), (4, 7), (0, 0)])
+        p = rnd.choice([1, 2, 5, 32])
+        out["random"].append(dict(a=a.decode(), b=b.decode(), g=g, h=h, p=p, **_ref_record(a, b, g, h, p)))
+    rnd = random.Random(5)
+    for st in (-1, -2, -3, 1, 2, 3):
+        for et in (-1, -2, -3, 1, 2, 3):
+            for t in range(6):
+                m = rnd.randint(1, 30)
+                n = rnd.randint(m, 36)
+                a = bytes(rnd.choice(b"ACGT") for _ in range(m))
+                b = bytes(rnd.choice(b"ACGT") for _ in range(n))
+                g, h = rnd.choice([(1, 2), (2, 1), (1, 0), (0, 2)])
+                p = rnd.choice([1, 3])
+                rec = _ref_record(a, b, g, h, p, st, et)
+                del rec["rows_md5"]                 # the typed comparison checks tables, end state and node states
+                out["typed"].append(dict(a=a.decode(), b=b.decode(), g=g, h=h, p=p, start_type=st, end_type=et, **rec))
+    json.dump(out, open(os.path.join(HERE, "ref_tables.json"), "w"), separators=(",", ":"))
+    print("full-table fixture written:", len(out["random"]), "random,", len(out["typed"]), "typed cases;", out["source"])
+
+
 if __name__ == "__main__":
-    main()
+    if sys.argv[1:] == ["tables"]:
+        po.build()
+        ref_tables_fixture()
+    else:
+        main()

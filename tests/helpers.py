@@ -1,4 +1,5 @@
 """Shared test helpers: FASTA fixture reader and seeded sequence generators (SURVEY 8d)."""
+import hashlib
 import os
 import random
 
@@ -76,3 +77,10 @@ def py_random_pair(rnd: random.Random, max_m=40, max_n=48, alpha=b"ACGT"):
     else:
         b = bytes(rnd.choice(alpha) for _ in range(n))
     return a, b
+
+
+def table_record(tables, corner, end_state, ops: bytes, row_a: bytes, row_b: bytes):
+    """What the full-table comparisons check, small enough to store: tables [3, m+1, n+1] int32 (-inf = NEG)."""
+    return {"tables_md5": [hashlib.md5(t.astype("<i4").tobytes()).hexdigest() for t in tables],
+            "corner": [int(x) for x in corner], "end_state": int(end_state), "ops": "".join(str(x) for x in ops),
+            "rows_md5": hashlib.md5(row_a + b"\n" + row_b + b"\n").hexdigest()}
