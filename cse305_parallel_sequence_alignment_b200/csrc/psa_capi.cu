@@ -49,9 +49,9 @@ int dispatch_batch(psa_ctx* ctx, const psa_batch_args& args, int max_m, int max_
         return psa_fail(ctx, PSA_ERR_CAPACITY, "ops_stride_words < ceil((max m + max n)/16)");
     if (args.start_type != -1 || args.end_type != -1 || args.types != nullptr) {
         if (mode != PSA_GLOBAL) return psa_fail(ctx, PSA_ERR_ARG, "start/end types apply to global alignment only");
-        if (!psa_short_supported(max_m, max_n, tb))
-            return psa_fail(ctx, PSA_ERR_RANGE, "typed subproblems are implemented by the short-pair kernel (n <= 256)");
-        return psa_launch_short(ctx, args, max_m, max_n, mode, tb, stream);
+        if (psa_short_supported(max_m, max_n, tb)) return psa_launch_short(ctx, args, max_m, max_n, mode, tb, stream);
+        if (tb) return psa_launch_long_batch_tb(ctx, args, max_m, max_n, mode, stream);
+        return psa_fail(ctx, PSA_ERR_RANGE, "typed subproblems wider than 256 columns need PSA_WANT_TRACEBACK on the device entry");
     }
     if (psa_short_supported(max_m, max_n, tb)) {
         // DNA fast path (two pairs per register, .S16x2); non-ACGT members fall through to the generic kernel inside
@@ -64,8 +64,7 @@ int dispatch_batch(psa_ctx* ctx, const psa_batch_args& args, int max_m, int max_
             return psa_launch_pack_long(ctx, args, max_m, max_n, mode, stream);
         return psa_launch_long_batch(ctx, args, max_m, max_n, mode, stream);
     }
-    return psa_fail(ctx, PSA_ERR_RANGE, "device batches of long pairs support score only; use psa_align_long_device "
-                                        "(or the host-buffer calls) for a checkpointed traceback");
+    return psa_launch_long_batch_tb(ctx, args, max_m, max_n, mode, stream);
 }
 
 }  // namespace
@@ -115,6 +114,7 @@ int psa_ctx_set_option(psa_ctx* ctx, const char* name, long long value) {
     else if (k == "long_geometry") o.long_geometry = (int)value;
     else if (k == "long_ctas_per_sm") o.long_ctas_per_sm = (int)value;
     else if (k == "long_band") o.long_band = (int)value;
+    else if (k == "long_tb_chunk") o.long_tb_chunk = value;
     else if (k == "long_systolic") o.long_systolic = (int)value;
     else if (k == "systolic_warps_per_sm") o.systolic_warps_per_sm = (int)value;
     else if (k == "systolic_kc") o.systolic_kc = (int)value;
@@ -200,6 +200,12 @@ int psa_align_batch_device(psa_ctx* ctx, const uint8_t* d_bases_a, const int64_t
 }
 
 }  // extern "C"
+
+// Pairs of a host-buffer traceback batch of long pairs from which the batched path (one warp per pair) replaces the
+// per-pair loop (each pair over the whole GPU).  Sweep of 1 - 64 pairs (profiles/r03_long_tb.json, same box): at 16 pairs
+// the batch is at least as fast in every series (5 kbp local 38.6 vs 38.7 ms, global 28.9 vs 40.0; 1 kbp local 2.9 vs
+// 8.1, global 1.4 vs 8.3); at 8 pairs the per-pair loop still wins at 5 kbp (19.4 vs 34.9 ms local, 20.0 vs 21.2 global).
+constexpr int kLongTbBatchMin = 16;
 
 // Host-buffer batch with an optional border variant per call or per pair; psa_align_batch is the -1/-1 case.
 static int align_batch_host(psa_ctx* ctx, const uint8_t* bases_a, const int64_t* off_a, const int32_t* len_a,
@@ -311,7 +317,14 @@ static int align_batch_host(psa_ctx* ctx, const uint8_t* bases_a, const int64_t*
     PSA_CUDA_OK(ctx, cudaMemcpyAsync(d + o_lb, len_b, n_pairs * 4, cudaMemcpyHostToDevice, st));
     const bool is_short = psa_short_supported(max_m, max_n, tb);
     if (typed && mode != PSA_GLOBAL) return psa_fail(ctx, PSA_ERR_ARG, "start/end types apply to global alignment only");
-    if (is_short || (!typed && !tb && n_pairs > 8)) {
+    // long pairs with traceback: from kLongTbBatchMin pairs on, one warp per pair (checkpointed batch fill + batched walk)
+    // unless one pair's checkpoints exceed the memory budget
+    long long tb_chunk = 0;
+    if (!is_short && tb && n_pairs >= (size_t)kLongTbBatchMin) {
+        rc = psa_long_batch_tb_chunk(ctx, (long long)n_pairs, max_m, max_n, mode, &tb_chunk);
+        if (rc) return rc;
+    }
+    if (is_short || (!typed && !tb && n_pairs > 8) || tb_chunk > 0) {
         rc = dispatch_batch(ctx, args, max_m, max_n, mode, flags, st);
         if (rc) return rc;
     } else {

@@ -32,6 +32,7 @@ struct psa_options {
     int long_geometry = -1;       // >= 0: force the tile geometry of the single long pair kernel (score only)
     int long_ctas_per_sm = 0;
     int long_band = 1;            // 0: no ahead-of-time band recompute before the checkpointed traceback walk
+    long long long_tb_chunk = 0;  // > 0: cap of the pairs per chunk of a long traceback batch (tests: several chunks in one call)
     int long_systolic = -1;       // -1 auto, 0 never, 1 always: column-stationary systolic kernel for one long pair (score only)
     int systolic_warps_per_sm = 0;   // resident strips per SM (default 8)
     int systolic_kc = 8;          // columns per lane of the systolic kernel (4 or 8): 8 measured faster on 1 and on 8 GPUs (fewer strips = a
@@ -161,5 +162,9 @@ int psa_launch_long_batch(psa_ctx* ctx, const psa_batch_args& args, int max_m, i
 size_t psa_long_batch_scratch_bytes(psa_ctx* ctx, long long n_pairs, int max_n);
 int psa_launch_long_batch_at(psa_ctx* ctx, const psa_batch_args& args, int max_m, int max_n, int mode,
                              const uint8_t* d_flags, uint8_t* scratch, cudaStream_t st);
+// Batch of long pairs with traceback: chunks of a checkpointed one-warp-per-pair fill + one-warp-per-pair walk (psa_long.cu).
+// psa_long_batch_tb_chunk: pairs per chunk for this batch shape (0: one checkpoint slot exceeds the memory budget).
+int psa_long_batch_tb_chunk(psa_ctx* ctx, long long n_pairs, int max_m, int max_n, int mode, long long* chunk);
+int psa_launch_long_batch_tb(psa_ctx* ctx, const psa_batch_args& args, int max_m, int max_n, int mode, cudaStream_t st);
 bool psa_pack_long_supported(int max_m, int max_n, int mode, int g, int h);
 int psa_launch_pack_long(psa_ctx* ctx, const psa_batch_args& args, int max_m, int max_n, int mode, cudaStream_t st);

@@ -380,20 +380,16 @@ __global__ void __launch_bounds__(BAND_WPB * 32) psa_long_band_kernel(TbArgs T) 
     for (int q = lane; q < nrows * 8; q += 32) out[q] = in[q];
 }
 
+// The walk from the end cell, lane 0 stepping through the codes of the tile held in `dirs` and the whole warp
+// recomputing the next tile whenever the path leaves it.  Writes the 2-bit ops to `ops` and completes `r`
+// (start cell, aln_len); `band` (optional) holds tiles psa_long_band_kernel recomputed ahead of time.
+// Shared by the single-pair kernel and the batched walk (one warp per pair).
 template <int MODE>
-__global__ void __launch_bounds__(32) psa_long_tb_kernel(TbArgs T) {
-    __shared__ uint32_t dirs[R * 32];
-    __shared__ int lbH[R], lbE[R];
-    __shared__ uint8_t sA[R];
-    const LongJob& J = T.J;
-    const int lane = threadIdx.x;
+__device__ void tb_walk(const LongJob& J, psa_batch_item& r, int state, uint32_t* ops, const uint32_t* band,
+                        uint32_t* dirs, int* lbH, int* lbE, uint8_t* sA) {
+    const int lane = threadIdx.x & 31;
     const int m = J.m;
-    psa_batch_item r;
-    int i, j, state;
-    tb_end<MODE>(J, r, state);
-    i = r.end_i; j = r.end_j;
-    if (T.ops == nullptr) { if (lane == 0) *T.item = r; return; }
-
+    int i = r.end_i, j = r.end_j;
     int trb = -1, ts = -1;      // tile currently held in `dirs`
     int len = 0;
     int hits = 0, misses = 0;
@@ -415,7 +411,7 @@ __global__ void __launch_bounds__(32) psa_long_tb_kernel(TbArgs T) {
                     code = (dirs[(si - 1 - rb * R) * 32 + cj / K] >> (4 * (cj % K))) & 15;
                 }
                 acc |= (uint32_t)state << (2 * (len & 15));
-                if ((len & 15) == 15) { T.ops[len >> 4] = acc; acc = 0; }
+                if ((len & 15) == 15) { ops[len >> 4] = acc; acc = 0; }
                 ++len;
                 r.start_i = i; r.start_j = j;
                 const int ns = next_state<MODE>(state, code, border);
@@ -429,11 +425,11 @@ __global__ void __launch_bounds__(32) psa_long_tb_kernel(TbArgs T) {
         const int rb = need_rb, s = need_s;
         const int need_row = __shfl_sync(0xffffffffu, (lane == 0) ? ((state == 2) ? i : i - 1) : 0, 0);   // source row of the pending step
         const int i0 = rb * R, nrows = min(min(R, m - i0), need_row - i0);      // rows below the entry row are never consulted
-        const int bt = (T.band != nullptr) ? s - band_first_strip<MODE>(J, r.end_i, r.end_j, rb) : -1;
+        const int bt = (band != nullptr) ? s - band_first_strip<MODE>(J, r.end_i, r.end_j, rb) : -1;
         if (bt >= 0 && bt < BAND_TILES) {
             // ---- the tile was recomputed ahead of time by psa_long_band_kernel: copy its codes in ----
             __syncwarp();
-            const uint4* in = reinterpret_cast<const uint4*>(T.band + ((long long)rb * BAND_TILES + bt) * (R * 32));
+            const uint4* in = reinterpret_cast<const uint4*>(band + ((long long)rb * BAND_TILES + bt) * (R * 32));
             uint4* out = reinterpret_cast<uint4*>(dirs);
             const int total = nrows * 8;                       // 16-byte pieces; eight loads in flight per lane
             for (int q0 = 0; q0 < total; q0 += 256) {
@@ -453,13 +449,127 @@ __global__ void __launch_bounds__(32) psa_long_tb_kernel(TbArgs T) {
         trb = rb; ts = s;
     }
 #ifdef PSA_TB_DEBUG
-    if (lane == 0) printf("psa_long_tb_kernel: %d band tiles, %d recomputed tiles, %d ops\n", hits, misses, len);
+    if (lane == 0) printf("tb_walk: %d band tiles, %d recomputed tiles, %d ops\n", hits, misses, len);
 #endif
     if (lane == 0) {
-        if (len & 15) T.ops[len >> 4] = acc;
+        if (len & 15) ops[len >> 4] = acc;
         r.aln_len = len;
-        *T.item = r;
     }
+}
+
+template <int MODE>
+__global__ void __launch_bounds__(32) psa_long_tb_kernel(TbArgs T) {
+    __shared__ uint32_t dirs[R * 32];
+    __shared__ int lbH[R], lbE[R];
+    __shared__ uint8_t sA[R];
+    psa_batch_item r;
+    int state;
+    tb_end<MODE>(T.J, r, state);
+    if (T.ops != nullptr) tb_walk<MODE>(T.J, r, state, T.ops, T.band, dirs, lbH, lbE, sA);
+    if (threadIdx.x == 0) *T.item = r;
+}
+
+// ---- batch of long pairs with traceback: checkpointed fill (one warp per pair), then one walk warp per pair ----
+// Pair p of the chunk [p0, p0 + count) owns slot p - p0 of the region: [best (8 B) | corner (3 x 4 B) | pad to 256 B |
+// row-block bottom rows H, F (NB rows of up256((n+1)*4) bytes each) | strip right columns H, E ([S][m+1] ints each)],
+// sized by the pair's own m, n inside slot_bytes (computed from the largest m, n of the batch).
+struct LongBatchTb {
+    psa_batch_args P;
+    long long p0, count;
+    uint8_t* region;
+    long long slot_bytes;
+    int* ticket;
+};
+
+__device__ __forceinline__ long long up256_d(long long x) { return (x + 255) / 256 * 256; }
+
+// The LongJob of pair p (its checkpoints in the slot); the same for the fill and the walk.
+__device__ __forceinline__ LongJob batch_tb_job(const LongBatchTb& Bt, long long p) {
+    const psa_batch_args& P = Bt.P;
+    LongJob J;
+    J.a = P.bases_a + P.off_a[p]; J.b = P.bases_b + P.off_b[p];
+    J.m = P.len_a[p]; J.n = P.len_b[p]; J.g = P.g; J.h = P.h; J.mul8 = key_mult(K);
+    uint8_t* slot = Bt.region + (p - Bt.p0) * Bt.slot_bytes;
+    const int NB = (J.m + R - 1) / R, S = (J.n + W - 1) / W;
+    const long long row = up256_d((long long)(J.n + 1) * 4), ckv = up256_d((long long)S * (J.m + 1) * 4);
+    J.best = (unsigned long long*)slot; J.corner = (int*)(slot + 8);
+    J.hbufH = (int*)(slot + 256); J.hbufF = (int*)(slot + 256 + row * NB); J.hb_stride = row / 4;
+    J.ckvH = (int*)(slot + 256 + 2 * row * NB); J.ckvE = (int*)(slot + 256 + 2 * row * NB + ckv);
+    J.progress = nullptr; J.ticket = nullptr;
+    J.col0 = 0; J.n_total = J.n; J.row_off = 0;
+    J.start_type = P.types ? (int)(P.types[p] & 15) - 3 : P.start_type;
+    J.end_type = P.types ? (int)(P.types[p] >> 4) - 3 : P.end_type;
+    return J;
+}
+
+// Fill: the <128, 8> tile grid the walk decodes (pairs are independent: no progress flags).
+template <int MODE>
+__global__ void __launch_bounds__(WPB * 32) psa_long_batch_tb_fill_kernel(LongBatchTb Bt) {
+    __shared__ WarpSmem<R> smem[WPB];
+    const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    WarpSmem<R>& sm = smem[w];
+    for (;;) {
+        long long q = 0;
+        if (lane == 0) q = atomicAdd(Bt.ticket, 1);
+        q = __shfl_sync(0xffffffffu, q, 0);
+        if (q >= Bt.count) break;
+        const long long p = Bt.p0 + q;
+        const LongJob J = batch_tb_job(Bt, p);
+        if (J.m <= 0 || J.n <= 0) continue;          // borders only: the walk kernel writes the item
+        if (lane == 0) { *J.best = 0ull; J.corner[0] = J.corner[1] = J.corner[2] = PSA_KNEG; }
+        __syncwarp();
+        Track tr{0, 0, 0};
+        const int NB = (J.m + R - 1) / R;
+        for (int rb = 0; rb < NB; ++rb) process_rowblock<MODE, R, K>(J, rb, sm, tr);
+        flush_track<MODE>(J, tr);
+        __syncwarp();
+    }
+}
+
+// Result of a member with m == 0 or n == 0: what the short kernel's degenerate branch returns (psa_short.cu).
+template <int MODE>
+__device__ __forceinline__ psa_batch_item degenerate_item(int m, int n, int g, int h, int st, int et) {
+    auto outv = [](int v) { return v < PSA_KNEG / 2 ? PSA_NEG_INF : v; };
+    psa_batch_item r;
+    r.t1 = r.t2 = r.t3 = PSA_NEG_INF;
+    if (MODE == PSA_LOCAL) r.t1 = 0;
+    else if (m == 0 && n == 0) {
+        if (st == -1 || st == 1) r.t1 = 0; else if (st == -2) r.t2 = 0; else if (st == -3) r.t3 = 0;
+    } else if (m == 0) r.t2 = outv(border_row0_H<PSA_GLOBAL>(n, g, h, st));
+    else r.t3 = outv(border_col0_H<PSA_GLOBAL>(m, g, h, st));
+    r.score = imax(r.t1, imax(r.t2, r.t3));
+    if (MODE == PSA_LOCAL) r.end_state = 1;
+    else if (et > 0) r.end_state = et;
+    else {
+        const int e2 = r.t2 + (et == -2 ? h : 0), e3 = r.t3 + (et == -3 ? h : 0);
+        r.end_state = (r.t1 >= e2 && r.t1 >= e3) ? 1 : ((e2 >= r.t1 && e2 >= e3) ? 2 : 3);
+    }
+    r.end_i = MODE == PSA_LOCAL ? 0 : m; r.end_j = MODE == PSA_LOCAL ? 0 : n;
+    r.start_i = 0; r.start_j = 0; r.aln_len = 0;
+    return r;
+}
+
+// Walk: one warp per pair of the chunk, the single-pair walk without the band (the other pairs are the parallelism).
+constexpr int WALK_WPB = 2;      // 2 x 17.3 KB of static shared memory per CTA
+template <int MODE>
+__global__ void __launch_bounds__(WALK_WPB * 32) psa_long_batch_tb_walk_kernel(LongBatchTb Bt) {
+    __shared__ uint32_t dirs[WALK_WPB][R * 32];
+    __shared__ int lbH[WALK_WPB][R], lbE[WALK_WPB][R];
+    __shared__ uint8_t sA[WALK_WPB][R];
+    const int w = threadIdx.x >> 5;
+    const long long q = (long long)blockIdx.x * WALK_WPB + w;
+    if (q >= Bt.count) return;
+    const long long p = Bt.p0 + q;
+    const LongJob J = batch_tb_job(Bt, p);
+    psa_batch_item r;
+    if (J.m <= 0 || J.n <= 0) {
+        r = degenerate_item<MODE>(J.m, J.n, J.g, J.h, J.start_type, J.end_type);
+    } else {
+        int state;
+        tb_end<MODE>(J, r, state);
+        tb_walk<MODE>(J, r, state, Bt.P.ops + p * Bt.P.ops_stride_words, nullptr, dirs[w], lbH[w], lbE[w], sA[w]);
+    }
+    if ((threadIdx.x & 31) == 0) Bt.P.items[p] = r;
 }
 
 }  // namespace
@@ -637,6 +747,75 @@ int psa_launch_long_batch(psa_ctx* ctx, const psa_batch_args& args, int max_m, i
     return psa_launch_long_batch_at(ctx, args, max_m, max_n, mode, nullptr, (uint8_t*)ctx->d_work, st);
 }
 
+
+// ---- batch of long pairs with traceback ----------------------------------------------------------------------------
+// The plan depends on n_pairs, max_m and max_n alone (nothing is read back from the device): every pair of a chunk owns a
+// checkpoint slot sized for the largest pair, a chunk holds at most one pair per resident fill warp and at most as many
+// slots as half of the device memory that is free at call time (plus the context's own work buffer, which it may
+// replace).  Chunks run fill -> walk on the caller's stream, one after the other.
+namespace {
+size_t long_tb_slot_bytes(int max_m, int max_n) {
+    const size_t NB = ((size_t)max_m + R - 1) / R, S = ((size_t)max_n + W - 1) / W;
+    return 256 + 2 * NB * up256((size_t)(max_n + 1) * 4) + 2 * up256(S * ((size_t)max_m + 1) * 4);
+}
+int long_tb_fill_ctas(psa_ctx* ctx, int mode, int* ctas) {
+    int per_sm = 0;
+    const void* kern = mode == PSA_LOCAL ? (const void*)psa_long_batch_tb_fill_kernel<PSA_LOCAL>
+                                         : (const void*)psa_long_batch_tb_fill_kernel<PSA_GLOBAL>;
+    PSA_CUDA_OK(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, WPB * 32, 0));
+    if (per_sm > 4) per_sm = 4;
+    *ctas = std::max(1, per_sm * ctx->sm_count);
+    return PSA_OK;
+}
+}  // namespace
+
+int psa_long_batch_tb_chunk(psa_ctx* ctx, long long n_pairs, int max_m, int max_n, int mode, long long* chunk) {
+    *chunk = 0;
+    int ctas = 1;
+    int rc = long_tb_fill_ctas(ctx, mode, &ctas);
+    if (rc) return rc;
+    size_t free_b = 0, total_b = 0;
+    PSA_CUDA_OK(ctx, cudaMemGetInfo(&free_b, &total_b));
+    const size_t budget = (free_b + ctx->d_work_bytes) / 2;
+    const size_t slot = long_tb_slot_bytes(max_m, max_n);
+    long long c = std::min<long long>(n_pairs, (long long)ctas * WPB);
+    c = std::min<long long>(c, (long long)((budget > 256 ? budget - 256 : 0) / slot));
+    if (ctx->opt.long_tb_chunk > 0) c = std::min<long long>(c, ctx->opt.long_tb_chunk);
+    *chunk = std::max(0LL, c);
+    return PSA_OK;
+}
+
+int psa_launch_long_batch_tb(psa_ctx* ctx, const psa_batch_args& args, int max_m, int max_n, int mode, cudaStream_t st) {
+    if (max_m >= 0x1FFFFF || max_n >= 0x1FFFFF) return psa_fail(ctx, PSA_ERR_RANGE, "long path: lengths must be < 2^21 - 1");
+    long long chunk = 0;
+    int rc = psa_long_batch_tb_chunk(ctx, args.n_pairs, max_m, max_n, mode, &chunk);
+    if (rc) return rc;
+    if (chunk < 1) chunk = 1;          // one slot over the budget: try it anyway (the per-pair path needs the same checkpoints)
+    int ctas = 1;
+    rc = long_tb_fill_ctas(ctx, mode, &ctas);
+    if (rc) return rc;
+    const size_t slot = long_tb_slot_bytes(max_m, max_n);
+    rc = ensure_work(ctx, 256 + (size_t)chunk * slot);
+    if (rc) return rc;
+    uint8_t* d = (uint8_t*)ctx->d_work;
+    for (long long p0 = 0; p0 < args.n_pairs; p0 += chunk) {
+        const long long cnt = std::min(chunk, args.n_pairs - p0);
+        LongBatchTb Bt{args, p0, cnt, d + 256, (long long)slot, (int*)d};
+        PSA_CUDA_OK(ctx, cudaMemsetAsync(d, 0, 256, st));
+        const int fill_grid = (int)std::min<long long>((cnt + WPB - 1) / WPB, ctas);
+        const int walk_grid = (int)((cnt + WALK_WPB - 1) / WALK_WPB);
+        if (mode == PSA_LOCAL) {
+            psa_long_batch_tb_fill_kernel<PSA_LOCAL><<<fill_grid, WPB * 32, 0, st>>>(Bt);
+            psa_long_batch_tb_walk_kernel<PSA_LOCAL><<<walk_grid, WALK_WPB * 32, 0, st>>>(Bt);
+        } else {
+            psa_long_batch_tb_fill_kernel<PSA_GLOBAL><<<fill_grid, WPB * 32, 0, st>>>(Bt);
+            psa_long_batch_tb_walk_kernel<PSA_GLOBAL><<<walk_grid, WALK_WPB * 32, 0, st>>>(Bt);
+        }
+        PSA_CUDA_OK(ctx, cudaGetLastError());
+        ctx->launches += 2;
+    }
+    return PSA_OK;
+}
 
 // ---- partition finder (SURVEY 8 f-3; the role of sequence_alignment/partial.cpp:81-163) ---------------------------
 // Forward sweep of (A, B) and reverse sweep of (reverse A, reverse B), both score-only fills that keep the bottom row

@@ -107,8 +107,8 @@ int psa_align_pair_typed(psa_ctx* ctx, const char* a, const char* b, size_t m, s
  * two-point partition {(0,0,-1), (m,n,1)} (:392-398), for which this equals psa_align_pair.
  * out: ops/rows/aln_len of the linked alignment, start cell of its first column, t1..t3/end_state
  * of the last piece, score = score of the linked alignment as printed.  If every piece is at most 256
- * columns wide they all run in one launch; otherwise the pieces run one after the other, each on the
- * whole GPU. */
+ * columns wide they all run in one launch; otherwise a handful of pieces run one after the other, each on
+ * the whole GPU, and more of them run as one batch of long pairs (one warp per piece, as psa_align_batch). */
 typedef struct psa_bp {
     int64_t i, j;
     int32_t t;
@@ -148,8 +148,13 @@ typedef struct {
 
 /* ops, if requested, are 2-bit codes (1/2/3; 0 = unused), 16 per uint32 starting at bit 0, in
  * TRACEBACK order (first code = the end cell), ops_stride_words words per pair; the caller must
- * give ops_stride_words >= ceil((max m + max n) / 16).  psa_ops_unpack turns one pair's words
- * into forward-order bytes. */
+ * give ops_stride_words >= ceil((max m + max n) / 16), for short and long pairs alike.  Words past
+ * ceil(aln_len / 16) of a pair are not written.  psa_ops_unpack turns one pair's words into
+ * forward-order bytes.
+ * Long pairs (wider than 256 columns) with PSA_WANT_TRACEBACK: a few pairs run one after the other, each
+ * over the whole GPU (psa_align_long_device); larger batches run one warp per pair -- a fill that keeps
+ * tile-boundary checkpoints, then a walk that recomputes only the tiles the path crosses -- in chunks
+ * sized by the device memory free at call time.  Lengths < 2^21 - 1. */
 int psa_align_batch(psa_ctx* ctx, const uint8_t* bases_a, const int64_t* off_a, const int32_t* len_a,
                     const uint8_t* bases_b, const int64_t* off_b, const int32_t* len_b, size_t n_pairs,
                     size_t bytes_a, size_t bytes_b, int mode, int g, int h, unsigned flags,
@@ -157,7 +162,10 @@ int psa_align_batch(psa_ctx* ctx, const uint8_t* bases_a, const int64_t* off_a, 
 
 /* Same computation with every buffer already resident in device memory (the caller's
  * allocations, e.g. torch tensors) on the given cudaStream_t (NULL = the context's stream);
- * asynchronous: the caller synchronises.  max_len_a/max_len_b bound the lengths in the batch. */
+ * asynchronous: the caller synchronises.  max_len_a/max_len_b bound the lengths in the batch.
+ * Long pairs accept PSA_WANT_TRACEBACK: always the one-warp-per-pair batch path (checkpointed fill +
+ * batched walk), planned from n_pairs, max_len_a and max_len_b alone, so nothing is read back and the
+ * call stays asynchronous; results are identical to psa_align_pair on each pair. */
 int psa_align_batch_device(psa_ctx* ctx, const uint8_t* d_bases_a, const int64_t* d_off_a, const int32_t* d_len_a,
                            const uint8_t* d_bases_b, const int64_t* d_off_b, const int32_t* d_len_b,
                            size_t n_pairs, int max_len_a, int max_len_b, int mode, int g, int h, unsigned flags,
