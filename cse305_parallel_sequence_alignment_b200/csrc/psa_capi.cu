@@ -515,6 +515,20 @@ void psa_render_rows(const char* a, const char* b, const uint8_t* ops, int64_t l
 
 }  // extern "C"
 
+// Gives *out library-owned ops and rows for `len` alignment columns (rows NUL-terminated) and sets aln_len; the caller
+// fills ops and renders the rows.  On allocation failure frees what was allocated.
+static int alloc_alignment(psa_ctx* ctx, psa_result* out, int64_t len) {
+    out->ops = (uint8_t*)malloc((size_t)len + 1);
+    out->row_a = (char*)malloc((size_t)len + 1);
+    out->row_b = (char*)malloc((size_t)len + 1);
+    if (!out->ops || !out->row_a || !out->row_b) { psa_result_free(out); return psa_fail(ctx, PSA_ERR_NOMEM, "malloc"); }
+    out->row_a[len] = 0; out->row_b[len] = 0;
+    out->aln_len = len;
+    return PSA_OK;
+}
+
+static bool ok_type(int t) { return t == -1 || t == -2 || t == -3 || t == 1 || t == 2 || t == 3; }
+
 static int align_pair_impl(psa_ctx* ctx, const char* a, const char* b, size_t m, size_t n, int mode, int g, int h,
                            unsigned flags, psa_result* out, const psa_piece_types& ty) {
     if (!ctx) return PSA_ERR_ARG;
@@ -534,14 +548,10 @@ static int align_pair_impl(psa_ctx* ctx, const char* a, const char* b, size_t m,
     out->end_i = it.end_i; out->end_j = it.end_j; out->start_i = it.start_i; out->start_j = it.start_j;
     out->aln_len = it.aln_len;
     if (tb) {
-        out->ops = (uint8_t*)malloc((size_t)it.aln_len + 1);
-        out->row_a = (char*)malloc((size_t)it.aln_len + 1);
-        out->row_b = (char*)malloc((size_t)it.aln_len + 1);
-        if (!out->ops || !out->row_a || !out->row_b) { psa_result_free(out); return psa_fail(ctx, PSA_ERR_NOMEM, "malloc"); }
+        rc = alloc_alignment(ctx, out, it.aln_len);
+        if (rc) return rc;
         psa_ops_unpack(words.data(), it.aln_len, out->ops);
         psa_render_rows(a, b, out->ops, it.aln_len, it.start_i, it.start_j, out->row_a, out->row_b);
-        out->row_a[it.aln_len] = 0;
-        out->row_b[it.aln_len] = 0;
     }
     return PSA_OK;
 }
@@ -556,7 +566,6 @@ int psa_align_pair(psa_ctx* ctx, const char* a, const char* b, size_t m, size_t 
 int psa_align_pair_typed(psa_ctx* ctx, const char* a, const char* b, size_t m, size_t n, int start_type, int end_type,
                          int g, int h, unsigned flags, psa_result* out) {
     if (!ctx) return PSA_ERR_ARG;
-    auto ok_type = [](int t) { return t == -1 || t == -2 || t == -3 || t == 1 || t == 2 || t == 3; };
     if (!ok_type(start_type) || !ok_type(end_type)) return psa_fail(ctx, PSA_ERR_ARG, "start/end type must be one of -1,-2,-3,1,2,3");
     if (m == 0 || n == 0) return psa_fail(ctx, PSA_ERR_ARG, "typed subproblems need m, n >= 1");
     psa_piece_types ty;
@@ -569,7 +578,6 @@ int psa_align_partition(psa_ctx* ctx, const char* a, const char* b, size_t m, si
     if (!ctx) return PSA_ERR_ARG;
     if (!out || !bp || (!a && m) || (!b && n)) return psa_fail(ctx, PSA_ERR_ARG, "null pointer");
     if (n_bp < 2) return psa_fail(ctx, PSA_ERR_ARG, "a partition needs at least two points");
-    auto ok_type = [](int t) { return t == -1 || t == -2 || t == -3 || t == 1 || t == 2 || t == 3; };
     const size_t np = n_bp - 1;
     std::vector<int64_t> off_a(np), off_b(np);
     std::vector<int32_t> len_a(np), len_b(np);
@@ -597,16 +605,14 @@ int psa_align_partition(psa_ctx* ctx, const char* a, const char* b, size_t m, si
     std::vector<uint32_t> words(np * stride);
     psa_piece_types ty;
     ty.per_pair = types.data();
-    const int rc = align_batch_host(ctx, (const uint8_t*)a, off_a.data(), len_a.data(), (const uint8_t*)b, off_b.data(),
-                                    len_b.data(), np, m, n, PSA_GLOBAL, g, h, PSA_WANT_SCORE | PSA_WANT_TRACEBACK,
-                                    items.data(), words.data(), stride, ty);
+    int rc = align_batch_host(ctx, (const uint8_t*)a, off_a.data(), len_a.data(), (const uint8_t*)b, off_b.data(),
+                              len_b.data(), np, m, n, PSA_GLOBAL, g, h, PSA_WANT_SCORE | PSA_WANT_TRACEBACK,
+                              items.data(), words.data(), stride, ty);
     if (rc) return rc;
     int64_t total = 0;
     for (size_t k = 0; k < np; ++k) total += items[k].aln_len;
-    out->ops = (uint8_t*)malloc((size_t)total + 1);
-    out->row_a = (char*)malloc((size_t)total + 1);
-    out->row_b = (char*)malloc((size_t)total + 1);
-    if (!out->ops || !out->row_a || !out->row_b) { psa_result_free(out); return psa_fail(ctx, PSA_ERR_NOMEM, "malloc"); }
+    rc = alloc_alignment(ctx, out, total);
+    if (rc) return rc;
     int64_t at = 0;
     bool first = true;
     for (size_t k = 0; k < np; ++k) {            // link the pieces in order (main_alignment.cpp:343-347)
@@ -618,8 +624,6 @@ int psa_align_partition(psa_ctx* ctx, const char* a, const char* b, size_t m, si
         if (first) { out->start_i = off_a[k] + it.start_i; out->start_j = off_b[k] + it.start_j; first = false; }
         at += it.aln_len;
     }
-    out->row_a[total] = 0; out->row_b[total] = 0;
-    out->aln_len = total;
     const psa_batch_item& last = items[np - 1];
     out->t1 = last.t1; out->t2 = last.t2; out->t3 = last.t3; out->end_state = last.end_state;
     out->end_i = bp[n_bp - 1].i; out->end_j = bp[n_bp - 1].j;
@@ -733,16 +737,12 @@ int psa_align_long_partitioned(psa_ctx* ctx, const char* a, const char* b, size_
             const int64_t sc = rescore(ops);
             if (sc != INT64_MIN && (opt == INT64_MIN || sc == opt || Q.size() == 2)) {
                 P = Q;
-                out->aln_len = (int64_t)ops.size();
-                out->ops = (uint8_t*)malloc(ops.size() + 1);
-                out->row_a = (char*)malloc(ops.size() + 1);
-                out->row_b = (char*)malloc(ops.size() + 1);
-                if (!out->ops || !out->row_a || !out->row_b) { psa_result_free(out); return psa_fail(ctx, PSA_ERR_NOMEM, "malloc"); }
+                rc = alloc_alignment(ctx, out, (int64_t)ops.size());
+                if (rc) return rc;
                 memcpy(out->ops, ops.data(), ops.size());
                 // cell of the first column in print_seq's convention: a leading gap sits on the border row / column 0
                 const int64_t si = (!ops.empty() && ops[0] == 2) ? 0 : 1, sj = (!ops.empty() && ops[0] == 3) ? 0 : 1;
                 psa_render_rows(a, b, out->ops, out->aln_len, si, sj, out->row_a, out->row_b);
-                out->row_a[ops.size()] = 0; out->row_b[ops.size()] = 0;
                 out->score = (int32_t)sc;
                 out->t1 = last.t1; out->t2 = last.t2; out->t3 = last.t3; out->end_state = last.end_state;
                 out->end_i = (int64_t)m; out->end_j = (int64_t)n; out->start_i = si; out->start_j = sj;

@@ -51,11 +51,6 @@ struct LongJob {
     int row_off;                // ROWOFF instantiation only: height of the FIRST row block (partition sweeps); else 0
 };
 
-__device__ __forceinline__ unsigned long long pack_best(int score, int i, int j) {
-    return ((unsigned long long)(unsigned)score << 42) | ((unsigned long long)(0x1FFFFF - i) << 21) |
-           (unsigned long long)(0x1FFFFF - j);
-}
-
 // Polling load: relaxed at gpu scope (served by L2, no L1 invalidate).  ld.acquire would emit a
 // CCTL.IVALL per poll, and a few spinning warps then starve the shared-memory pipe of the working
 // warps on the same SM (measured: 1.35e9 invalidates, 4x slower tiles).  One fence follows the
@@ -171,7 +166,7 @@ __device__ void process_rowblock(const LongJob& J, int rb, WarpSmem<RR>& sm, Tra
 template <int MODE>
 __device__ void flush_track(const LongJob& J, Track& tr) {
     if (MODE != PSA_LOCAL) return;
-    unsigned long long key = tr.best > 0 ? pack_best(tr.best, tr.bi, J.col0 + tr.bj) : 0ull;
+    unsigned long long key = tr.best > 0 ? best_key(tr.best, tr.bi, J.col0 + tr.bj) : 0ull;
 #pragma unroll
     for (int off = 16; off >= 1; off >>= 1) {
         const unsigned long long o = __shfl_xor_sync(0xffffffffu, key, off);
@@ -232,8 +227,6 @@ __global__ void __launch_bounds__(WPB * 32) psa_long_batch_kernel(LongBatch Bt) 
         J.start_type = -1; J.end_type = -1;
         if (lane == 0) { s_best[w] = 0ull; s_corner[w][0] = s_corner[w][1] = s_corner[w][2] = PSA_KNEG; }
         __syncwarp();
-        psa_batch_item r;
-        r.start_i = 0; r.start_j = 0; r.aln_len = 0;
         if (J.m > 0 && J.n > 0) {
             Track tr{0, 0, 0};
             const int NB = (J.m + R - 1) / R;
@@ -242,25 +235,10 @@ __global__ void __launch_bounds__(WPB * 32) psa_long_batch_kernel(LongBatch Bt) 
             __syncwarp();
         }
         if (lane == 0) {
-            const int m = J.m, n = J.n, g = J.g, h = J.h;
-            if (MODE == PSA_LOCAL) {
-                const unsigned long long key = s_best[w];
-                const int sc = (int)(key >> 42);
-                r.t1 = sc; r.t2 = PSA_NEG_INF; r.t3 = PSA_NEG_INF; r.score = sc; r.end_state = 1;
-                r.end_i = sc > 0 ? 0x1FFFFF - (int)((key >> 21) & 0x1FFFFF) : 0;
-                r.end_j = sc > 0 ? 0x1FFFFF - (int)(key & 0x1FFFFF) : 0;
-            } else {
-                int c1, c2, c3;
-                if (m > 0 && n > 0) { c1 = s_corner[w][0]; c2 = s_corner[w][1]; c3 = s_corner[w][2]; }
-                else {
-                    c1 = (m == 0 && n == 0) ? 0 : PSA_NEG_INF;
-                    c2 = (m == 0 && n > 0) ? -h - g * n : PSA_NEG_INF;
-                    c3 = (n == 0 && m > 0) ? -h - g * m : PSA_NEG_INF;
-                }
-                r.t1 = c1; r.t2 = c2; r.t3 = c3; r.score = imax(c1, imax(c2, c3));
-                r.end_state = (c1 >= c2 && c1 >= c3) ? 1 : ((c2 >= c1 && c2 >= c3) ? 2 : 3);
-                r.end_i = m; r.end_j = n;
-            }
+            psa_batch_item r;
+            if (J.m <= 0 || J.n <= 0) r = empty_item<MODE>(J.m, J.n, J.g, J.h, -1, -1);
+            else if (MODE == PSA_LOCAL) r = local_item_from_key(s_best[w]);
+            else r = global_item(s_corner[w][0], s_corner[w][1], s_corner[w][2], J.m, J.n, J.h, -1);
             Bt.P.items[p] = r;
         }
         __syncwarp();
@@ -277,30 +255,11 @@ struct TbArgs {
 
 constexpr int BAND_TILES = 3;
 
-// End cell and end state of the traceback (find_alignment, subproblem_alignment.cpp:112-145).
+// Result record the traceback starts from: end cell and end state (find_alignment, subproblem_alignment.cpp:112-145).
 template <int MODE>
-__device__ __forceinline__ void tb_end(const LongJob& J, psa_batch_item& r, int& state) {
-    if (MODE == PSA_LOCAL) {
-        const unsigned long long key = *J.best;
-        const int sc = (int)(key >> 42);
-        r.t1 = sc; r.t2 = PSA_NEG_INF; r.t3 = PSA_NEG_INF; r.score = sc;
-        r.end_i = sc > 0 ? 0x1FFFFF - (int)((key >> 21) & 0x1FFFFF) : 0;
-        r.end_j = sc > 0 ? 0x1FFFFF - (int)(key & 0x1FFFFF) : 0;
-        state = 1;
-    } else {
-        const int c1 = J.corner[0], c2 = J.corner[1], c3 = J.corner[2];
-        auto outv = [](int v) { return v < PSA_KNEG / 2 ? PSA_NEG_INF : v; };      // sentinel drift -> the ABI's -inf
-        r.t1 = outv(c1); r.t2 = outv(c2); r.t3 = outv(c3); r.score = outv(imax(c1, imax(c2, c3)));
-        // a positive end type forces the state; -2 / -3 credit h to T2 / T3 in the pick (cpp:112-146, h_prime)
-        if (J.end_type > 0) state = J.end_type;
-        else {
-            const int e2 = c2 + (J.end_type == -2 ? J.h : 0), e3 = c3 + (J.end_type == -3 ? J.h : 0);
-            state = (c1 >= e2 && c1 >= e3) ? 1 : ((e2 >= c1 && e2 >= e3) ? 2 : 3);
-        }
-        r.end_i = J.m; r.end_j = J.n_total;
-    }
-    r.end_state = state;
-    r.start_i = 0; r.start_j = 0; r.aln_len = 0;
+__device__ __forceinline__ psa_batch_item tb_end(const LongJob& J) {
+    if (MODE == PSA_LOCAL) return local_item_from_key(*J.best);
+    return global_item(J.corner[0], J.corner[1], J.corner[2], J.m, J.n_total, J.h, J.end_type);
 }
 
 // First strip of the band in row block rb: the tiles around the straight line the path is expected to
@@ -367,9 +326,7 @@ __global__ void __launch_bounds__(BAND_WPB * 32) psa_long_band_kernel(TbArgs T) 
     const int u = blockIdx.x * BAND_WPB + w;
     if (u >= NB * BAND_TILES) return;
     const int rb = u / BAND_TILES, bt = u % BAND_TILES;
-    psa_batch_item r;
-    int state;
-    tb_end<MODE>(J, r, state);
+    const psa_batch_item r = tb_end<MODE>(J);
     if (rb * R >= r.end_i) return;                       // rows below the end cell are never visited
     const int s = band_first_strip<MODE>(J, r.end_i, r.end_j, rb) + bt;
     if (s >= S) return;
@@ -380,16 +337,16 @@ __global__ void __launch_bounds__(BAND_WPB * 32) psa_long_band_kernel(TbArgs T) 
     for (int q = lane; q < nrows * 8; q += 32) out[q] = in[q];
 }
 
-// The walk from the end cell, lane 0 stepping through the codes of the tile held in `dirs` and the whole warp
-// recomputing the next tile whenever the path leaves it.  Writes the 2-bit ops to `ops` and completes `r`
+// The walk from the end cell and end state of `r`, lane 0 stepping through the codes of the tile held in `dirs` and the
+// whole warp recomputing the next tile whenever the path leaves it.  Writes the 2-bit ops to `ops` and completes `r`
 // (start cell, aln_len); `band` (optional) holds tiles psa_long_band_kernel recomputed ahead of time.
 // Shared by the single-pair kernel and the batched walk (one warp per pair).
 template <int MODE>
-__device__ void tb_walk(const LongJob& J, psa_batch_item& r, int state, uint32_t* ops, const uint32_t* band,
-                        uint32_t* dirs, int* lbH, int* lbE, uint8_t* sA) {
+__device__ void tb_walk(const LongJob& J, psa_batch_item& r, uint32_t* ops, const uint32_t* band, uint32_t* dirs, int* lbH,
+                        int* lbE, uint8_t* sA) {
     const int lane = threadIdx.x & 31;
     const int m = J.m;
-    int i = r.end_i, j = r.end_j;
+    int i = r.end_i, j = r.end_j, state = r.end_state;
     int trb = -1, ts = -1;      // tile currently held in `dirs`
     int len = 0;
     int hits = 0, misses = 0;
@@ -462,10 +419,8 @@ __global__ void __launch_bounds__(32) psa_long_tb_kernel(TbArgs T) {
     __shared__ uint32_t dirs[R * 32];
     __shared__ int lbH[R], lbE[R];
     __shared__ uint8_t sA[R];
-    psa_batch_item r;
-    int state;
-    tb_end<MODE>(T.J, r, state);
-    if (T.ops != nullptr) tb_walk<MODE>(T.J, r, state, T.ops, T.band, dirs, lbH, lbE, sA);
+    psa_batch_item r = tb_end<MODE>(T.J);
+    if (T.ops != nullptr) tb_walk<MODE>(T.J, r, T.ops, T.band, dirs, lbH, lbE, sA);
     if (threadIdx.x == 0) *T.item = r;
 }
 
@@ -526,29 +481,6 @@ __global__ void __launch_bounds__(WPB * 32) psa_long_batch_tb_fill_kernel(LongBa
     }
 }
 
-// Result of a member with m == 0 or n == 0: what the short kernel's degenerate branch returns (psa_short.cu).
-template <int MODE>
-__device__ __forceinline__ psa_batch_item degenerate_item(int m, int n, int g, int h, int st, int et) {
-    auto outv = [](int v) { return v < PSA_KNEG / 2 ? PSA_NEG_INF : v; };
-    psa_batch_item r;
-    r.t1 = r.t2 = r.t3 = PSA_NEG_INF;
-    if (MODE == PSA_LOCAL) r.t1 = 0;
-    else if (m == 0 && n == 0) {
-        if (st == -1 || st == 1) r.t1 = 0; else if (st == -2) r.t2 = 0; else if (st == -3) r.t3 = 0;
-    } else if (m == 0) r.t2 = outv(border_row0_H<PSA_GLOBAL>(n, g, h, st));
-    else r.t3 = outv(border_col0_H<PSA_GLOBAL>(m, g, h, st));
-    r.score = imax(r.t1, imax(r.t2, r.t3));
-    if (MODE == PSA_LOCAL) r.end_state = 1;
-    else if (et > 0) r.end_state = et;
-    else {
-        const int e2 = r.t2 + (et == -2 ? h : 0), e3 = r.t3 + (et == -3 ? h : 0);
-        r.end_state = (r.t1 >= e2 && r.t1 >= e3) ? 1 : ((e2 >= r.t1 && e2 >= e3) ? 2 : 3);
-    }
-    r.end_i = MODE == PSA_LOCAL ? 0 : m; r.end_j = MODE == PSA_LOCAL ? 0 : n;
-    r.start_i = 0; r.start_j = 0; r.aln_len = 0;
-    return r;
-}
-
 // Walk: one warp per pair of the chunk, the single-pair walk without the band (the other pairs are the parallelism).
 constexpr int WALK_WPB = 2;      // 2 x 17.3 KB of static shared memory per CTA
 template <int MODE>
@@ -563,11 +495,10 @@ __global__ void __launch_bounds__(WALK_WPB * 32) psa_long_batch_tb_walk_kernel(L
     const LongJob J = batch_tb_job(Bt, p);
     psa_batch_item r;
     if (J.m <= 0 || J.n <= 0) {
-        r = degenerate_item<MODE>(J.m, J.n, J.g, J.h, J.start_type, J.end_type);
+        r = empty_item<MODE>(J.m, J.n, J.g, J.h, J.start_type, J.end_type);
     } else {
-        int state;
-        tb_end<MODE>(J, r, state);
-        tb_walk<MODE>(J, r, state, Bt.P.ops + p * Bt.P.ops_stride_words, nullptr, dirs[w], lbH[w], lbE[w], sA[w]);
+        r = tb_end<MODE>(J);
+        tb_walk<MODE>(J, r, Bt.P.ops + p * Bt.P.ops_stride_words, nullptr, dirs[w], lbH[w], lbE[w], sA[w]);
     }
     if ((threadIdx.x & 31) == 0) Bt.P.items[p] = r;
 }

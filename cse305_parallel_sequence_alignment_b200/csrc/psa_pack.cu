@@ -27,7 +27,7 @@
 //     running score.  The scratch is O(chunk), not O(batch): it is recycled every chunk.
 // Pairs that are not plain upper-case ACGT are flagged and recomputed by the generic int32 kernel
 // (psa_short.cu) -- results stay bit-exact for any alphabet.
-#include "psa_common.cuh"
+#include "psa_result.cuh"
 #include <chrono>
 #include <vector>
 
@@ -502,33 +502,16 @@ __global__ void __launch_bounds__(128) psa_pack_fill_kernel(PackArgs A) {
                 fb = max(fb, __shfl_xor_sync(0xffffffffu, fb, off));
             }
             if (t == 0 && have) {
-                psa_batch_item it;
-                it.t2 = PSA_NEG_INF; it.t3 = PSA_NEG_INF; it.end_state = 1; it.start_i = 0; it.start_j = 0; it.aln_len = 0;
-                it.t1 = it.score = (int)(fa >> 20);
-                it.end_i = fa ? 1023 - (int)((fa >> 10) & 1023u) : 0;
-                it.end_j = fa ? 1023 - (int)(fa & 1023u) : 0;
-                if (mA > 0 && nA > 0) P.items[pA] = it;
-                if (haveB && mB > 0 && nB > 0) {
-                    it.t1 = it.score = (int)(fb >> 20);
-                    it.end_i = fb ? 1023 - (int)((fb >> 10) & 1023u) : 0;
-                    it.end_j = fb ? 1023 - (int)(fb & 1023u) : 0;
-                    P.items[pB] = it;
-                }
+                auto item = [](uint32_t f) {
+                    return local_item((int)(f >> 20), f ? 1023 - (int)((f >> 10) & 1023u) : 0, f ? 1023 - (int)(f & 1023u) : 0);
+                };
+                if (mA > 0 && nA > 0) P.items[pA] = item(fa);
+                if (haveB && mB > 0 && nB > 0) P.items[pB] = item(fb);
             }
         } else {
             // the capturing lane of each pair writes its corner (exactly one lane per pair)
-            auto emit = [&](long long p, int m, int n, int sh, const uint32_t* c3) {
-                const int t1 = (int)((c3[0] >> sh) & 0xffffu) - C.bias;
-                const int t2 = (int)((c3[1] >> sh) & 0xffffu) - C.bias;
-                const int t3 = (int)((c3[2] >> sh) & 0xffffu) - C.bias;
-                psa_batch_item it;
-                it.t1 = t1; it.t2 = t2; it.t3 = t3; it.score = max(t1, max(t2, t3));
-                it.end_state = (t1 >= t2 && t1 >= t3) ? 1 : ((t2 >= t1 && t2 >= t3) ? 2 : 3);
-                it.end_i = m; it.end_j = n; it.start_i = 0; it.start_j = 0; it.aln_len = 0;
-                P.items[p] = it;
-            };
-            if (have && mA > 0 && nA > 0 && t == tcapA) emit(pA, mA, nA, 0, cap);
-            if (haveB && mB > 0 && nB > 0 && t == tcapB) emit(pB, mB, nB, 16, cap + 3);
+            if (have && mA > 0 && nA > 0 && t == tcapA) P.items[pA] = packed_corner_item(cap, 0, C.bias, mA, nA);
+            if (haveB && mB > 0 && nB > 0 && t == tcapB) P.items[pB] = packed_corner_item(cap + 3, 16, C.bias, mB, nB);
         }
         if (t == 0 && have) {
             // degenerate members (a zero length) and non-ACGT members go to the generic kernel

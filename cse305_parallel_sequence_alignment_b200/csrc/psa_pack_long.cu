@@ -15,7 +15,7 @@
 // bias, so the clamp never touches them and plain 32-bit adds cannot borrow between the halves.
 // Local mode finds the end cell with the packed key T1*8 + (7 - k%8) (VIMNMX3.U16x2), one running key per
 // 8 columns, folded after every strip into a 64-bit (T1 desc, i asc, j asc) key.
-#include "psa_common.cuh"
+#include "psa_result.cuh"
 
 namespace {
 
@@ -118,7 +118,7 @@ __global__ void __launch_bounds__(WPB * 32) psa_pack_long_kernel(PLArgs A) {
             const int t1v = (int)(best >> 3) - A.bias;
             if (t1v <= 0) return 0ull;
             const int j = (bs >> 1) * W + lane * K + (bs & 1) * 8 + (7 - (int)(best & 7u)) + 1;
-            return ((unsigned long long)t1v << 42) | ((unsigned long long)(0x1FFFFF - bi) << 21) | (unsigned long long)(0x1FFFFF - j);
+            return best_key(t1v, bi, j);
         };
         uint32_t cap[6] = {0, 0, 0, 0, 0, 0};
         const int S = (npp + W - 1) / W;
@@ -215,30 +215,12 @@ __global__ void __launch_bounds__(WPB * 32) psa_pack_long_kernel(PLArgs A) {
                 fa = oa > fa ? oa : fa; fb = ob > fb ? ob : fb;
             }
             if (lane == 0) {
-                auto put = [&](long long p, unsigned long long key) {
-                    psa_batch_item it;
-                    it.t1 = it.score = (int)(key >> 42); it.t2 = PSA_NEG_INF; it.t3 = PSA_NEG_INF; it.end_state = 1;
-                    it.end_i = key ? 0x1FFFFF - (int)((key >> 21) & 0x1FFFFF) : 0;
-                    it.end_j = key ? 0x1FFFFF - (int)(key & 0x1FFFFF) : 0;
-                    it.start_i = 0; it.start_j = 0; it.aln_len = 0;
-                    P.items[p] = it;
-                };
-                if (mA > 0 && nA > 0) put(pA, fa);
-                if (haveB && mB > 0 && nB > 0) put(pB, fb);
+                if (mA > 0 && nA > 0) P.items[pA] = local_item_from_key(fa);
+                if (haveB && mB > 0 && nB > 0) P.items[pB] = local_item_from_key(fb);
             }
         } else {
-            auto emit = [&](long long p, int m, int n, int sh, const uint32_t* c3) {
-                const int t1 = (int)((c3[0] >> sh) & 0xffffu) - A.bias;
-                const int t2 = (int)((c3[1] >> sh) & 0xffffu) - A.bias;
-                const int t3 = (int)((c3[2] >> sh) & 0xffffu) - A.bias;
-                psa_batch_item it;
-                it.t1 = t1; it.t2 = t2; it.t3 = t3; it.score = max(t1, max(t2, t3));
-                it.end_state = (t1 >= t2 && t1 >= t3) ? 1 : ((t2 >= t1 && t2 >= t3) ? 2 : 3);
-                it.end_i = m; it.end_j = n; it.start_i = 0; it.start_j = 0; it.aln_len = 0;
-                P.items[p] = it;
-            };
-            if (mA > 0 && nA > 0 && lane == tcA) emit(pA, mA, nA, 0, cap);
-            if (haveB && mB > 0 && nB > 0 && lane == tcB) emit(pB, mB, nB, 16, cap + 3);
+            if (mA > 0 && nA > 0 && lane == tcA) P.items[pA] = packed_corner_item(cap, 0, A.bias, mA, nA);
+            if (haveB && mB > 0 && nB > 0 && lane == tcB) P.items[pB] = packed_corner_item(cap + 3, 16, A.bias, mB, nB);
         }
         if (lane == 0) {
             A.fallback[pA] = (!okA || mA == 0 || nA == 0) ? 1 : 0;

@@ -17,30 +17,11 @@
 //     z2 = d1==1 ? (E + h > H) : (E + h >= H)    (bit 2)  -> predecessor of a T2 state to the right
 //     e3 = (F + h > H)                           (bit 3)  -> predecessor of a T3 state below
 // Lane 0 then walks the codes and writes 2-bit ops.
-#include "psa_common.cuh"
+#include "psa_result.cuh"
 
 namespace {
 
 constexpr int kMaxK = 8;
-
-__device__ __forceinline__ int imax(int a, int b) { return a > b ? a : b; }
-
-// Borders by start type, global mode (ComputeFirstRowMapThread / compute_row, subproblem_alignment.cpp:
-// 212-227, 259-292).  H = max(T1,T2,T3) of the border cell; on row 0 only T2 can be finite (plus the
-// single 0 at (0,0)), on column 0 only T3.
-__device__ __forceinline__ int row0_H(int st, int j, int g, int h) {
-    if (j == 0) return (st == 2 || st == 3) ? PSA_KNEG : 0;          // T1/T2/T3[0][0] = 0 for -1,1 / -2 / -3
-    if (st == -2) return -g * j;
-    if (st == 1 || st == 3) return PSA_KNEG;
-    return -h - g * j;
-}
-__device__ __forceinline__ int col0_H(int st, int i, int g, int h) {
-    if (i == 0) return (st == 2 || st == 3) ? PSA_KNEG : 0;
-    if (st == -3) return -g * i;
-    if (st == 1 || st == 2) return PSA_KNEG;
-    return -h - g * i;
-}
-__device__ __forceinline__ int out_val(int v) { return v < PSA_KNEG / 2 ? PSA_NEG_INF : v; }
 
 template <int K, int MODE, bool TB>
 __global__ void __launch_bounds__(256) psa_short_kernel(psa_batch_args P, int sa_stride, int sb_stride,
@@ -63,25 +44,7 @@ __global__ void __launch_bounds__(256) psa_short_kernel(psa_batch_args P, int sa
         const int st = P.types ? (int)(P.types[p] & 15) - 3 : P.start_type;
         const int et = P.types ? (int)(P.types[p] >> 4) - 3 : P.end_type;
         if (m <= 0 || n <= 0) {   // degenerate: borders only (subproblem_alignment.cpp:259-292)
-            if (lane == 0) {
-                psa_batch_item r;
-                r.t1 = r.t2 = r.t3 = PSA_NEG_INF;
-                if (LOCAL) r.t1 = 0;
-                else if (m == 0 && n == 0) {
-                    if (st == -1 || st == 1) r.t1 = 0; else if (st == -2) r.t2 = 0; else if (st == -3) r.t3 = 0;
-                } else if (m == 0) r.t2 = out_val(row0_H(st, n, g, h));
-                else if (n == 0) r.t3 = out_val(col0_H(st, m, g, h));
-                r.score = imax(r.t1, imax(r.t2, r.t3));
-                if (LOCAL) r.end_state = 1;
-                else if (et > 0) r.end_state = et;
-                else {
-                    const int e2 = r.t2 + (et == -2 ? h : 0), e3 = r.t3 + (et == -3 ? h : 0);
-                    r.end_state = (r.t1 >= e2 && r.t1 >= e3) ? 1 : ((e2 >= r.t1 && e2 >= e3) ? 2 : 3);
-                }
-                r.end_i = LOCAL ? 0 : m; r.end_j = LOCAL ? 0 : n;
-                r.start_i = 0; r.start_j = 0; r.aln_len = 0;
-                *item = r;
-            }
+            if (lane == 0) *item = empty_item<MODE>(m, n, g, h, st, et);
             continue;
         }
         // ---- stage both sequences (coalesced byte loads) ----
@@ -99,10 +62,10 @@ __global__ void __launch_bounds__(256) psa_short_kernel(psa_batch_args P, int sa
         for (int k = 0; k < K; ++k) {
             const int j = c0 + k + 1;
             bcol[k] = (j <= n) ? (int)sB[j - 1] : 256;          // 256 never equals a byte
-            Hc[k] = LOCAL ? PSA_KNEG : row0_H(st, j, g, h);       // row 0: T2[0][j] (cpp:216-224)
+            Hc[k] = LOCAL ? PSA_KNEG : border_row0_H<PSA_GLOBAL>(j, g, h, st);     // row 0: T2[0][j] (cpp:216-224)
             Fc[k] = PSA_KNEG;
         }
-        int hd = LOCAL ? PSA_KNEG : row0_H(st, c0, g, h);   // H[0][c0]; the single 0 of row 0 sits at (0,0) (cpp:261-272)
+        int hd = LOCAL ? PSA_KNEG : border_row0_H<PSA_GLOBAL>(c0, g, h, st);   // H[0][c0]; the single 0 of row 0 sits at (0,0) (cpp:261-272)
         int recv_h = PSA_KNEG, recv_e = PSA_KNEG;
         int best = 0, bi = 0, bj = 0;           // local: best T1 and its first cell in this lane
         int c1 = PSA_KNEG, c2 = PSA_KNEG, c3 = PSA_KNEG;   // global: corner capture
@@ -111,7 +74,7 @@ __global__ void __launch_bounds__(256) psa_short_kernel(psa_batch_args P, int sa
         for (int s = 0; s < steps; ++s) {
             const int i = s - lane + 1;
             int hl, el;
-            if (lane == 0) { hl = LOCAL ? PSA_KNEG : col0_H(st, i, g, h); el = PSA_KNEG; }   // T3[i][0] (cpp:284-292)
+            if (lane == 0) { hl = LOCAL ? PSA_KNEG : border_col0_H<PSA_GLOBAL>(i, g, h, st); el = PSA_KNEG; }   // T3[i][0] (cpp:284-292)
             else { hl = recv_h; el = recv_e; }
             if (i >= 1 && i <= m) {
                 const int a = sA[i - 1];
@@ -146,7 +109,6 @@ __global__ void __launch_bounds__(256) psa_short_kernel(psa_batch_args P, int sa
         }
 
         // ---- gather the result ----
-        int state, ti, tj;
         psa_batch_item r;
         if (LOCAL) {
 #pragma unroll
@@ -157,26 +119,14 @@ __global__ void __launch_bounds__(256) psa_short_kernel(psa_batch_args P, int sa
                 const bool take = (ob > best) || (ob == best && (oi < bi || (oi == bi && oj < bj)));
                 if (take) { best = ob; bi = oi; bj = oj; }
             }
-            r.t1 = best; r.t2 = PSA_NEG_INF; r.t3 = PSA_NEG_INF; r.score = best;
-            r.end_i = best > 0 ? bi : 0; r.end_j = best > 0 ? bj : 0;
-            state = 1; ti = r.end_i; tj = r.end_j;
+            r = local_item(best, best > 0 ? bi : 0, best > 0 ? bj : 0);
         } else {
             const int src = (n - 1) / K;
             c1 = __shfl_sync(0xffffffffu, c1, src);
             c2 = __shfl_sync(0xffffffffu, c2, src);
             c3 = __shfl_sync(0xffffffffu, c3, src);
-            r.t1 = out_val(c1); r.t2 = out_val(c2); r.t3 = out_val(c3); r.score = out_val(imax(c1, imax(c2, c3)));
-            // end state: find_alignment() (cpp:112-145): forced by a positive end type, else the first of
-            // T1, T2 + h', T3 + h' that is >= the others (h' = h only for the matching end type -2 / -3)
-            if (et > 0) state = et;
-            else {
-                const int e2 = c2 + (et == -2 ? h : 0), e3 = c3 + (et == -3 ? h : 0);
-                state = (c1 >= e2 && c1 >= e3) ? 1 : ((e2 >= c1 && e2 >= e3) ? 2 : 3);
-            }
-            r.end_i = m; r.end_j = n; ti = m; tj = n;
+            r = global_item(c1, c2, c3, m, n, h, et);
         }
-        r.end_state = state;
-        r.start_i = 0; r.start_j = 0; r.aln_len = 0;
 
         if (TB) {
             __syncwarp();
@@ -184,7 +134,7 @@ __global__ void __launch_bounds__(256) psa_short_kernel(psa_batch_args P, int sa
                 uint32_t* ow = P.ops + p * P.ops_stride_words;
                 uint32_t acc = 0;
                 int len = 0;
-                int i = ti, j = tj;
+                int i = (int)r.end_i, j = (int)r.end_j, state = r.end_state;
                 while (i > 0 && j > 0) {
                     acc |= (uint32_t)state << (2 * (len & 15));
                     if ((len & 15) == 15) { ow[len >> 4] = acc; acc = 0; }
@@ -196,15 +146,8 @@ __global__ void __launch_bounds__(256) psa_short_kernel(psa_batch_args P, int sa
                     int code = 0;
                     const bool border = (si == 0 || sj == 0);
                     if (!border) code = (dirs[(si - 1) * 32 + (sj - 1) / K] >> (4 * ((sj - 1) % K))) & 15;
-                    const int d1 = code & 3, z2 = (code >> 2) & 1, e3 = (code >> 3) & 1;
-                    if (state == 1) {
-                        if (LOCAL && (border || d1 == 0)) break;     // T1[i][j] == f: the 0 floor, stop here
-                        state = d1;
-                    } else if (state == 2) {
-                        state = (d1 == 1) ? (z2 ? 2 : 1) : (z2 ? 2 : 3);
-                    } else {
-                        state = e3 ? 3 : d1;
-                    }
+                    state = next_state<MODE>(state, code, border);
+                    if (state == 0) break;     // nothing precedes this column: the 0 floor of a local alignment, or a border source
                     i = si; j = sj;
                     // on the border the predecessor node is the one find_alignment() drops (cpp:170)
                 }

@@ -331,7 +331,7 @@ __global__ void __launch_bounds__(SWPB * 32) psa_systolic_kernel(SysJob J) {
         const int j = cg + kk + 1;
         unsigned long long key = 0ull;
         if (t1v > 0 && j <= J.n_total)
-            key = ((unsigned long long)(unsigned)t1v << 42) | ((unsigned long long)(0x1FFFFF - besti) << 21) | (unsigned long long)(0x1FFFFF - j);
+            key = best_key(t1v, besti, j);
 #pragma unroll
         for (int off = 16; off >= 1; off >>= 1) {
             const unsigned long long o = __shfl_xor_sync(0xffffffffu, key, off);
@@ -346,22 +346,9 @@ __global__ void __launch_bounds__(SWPB * 32) psa_systolic_kernel(SysJob J) {
 // Result record of a systolic run: the local best / the global corner accumulated by the panel launches.
 __global__ void psa_systolic_result_kernel(const unsigned long long* best, const int* corner, int mode, int m, int n_total,
                                            int has_corner, psa_batch_item* item) {
-    psa_batch_item r;
-    r.start_i = 0; r.start_j = 0; r.aln_len = 0;
-    if (mode == PSA_LOCAL) {
-        const unsigned long long key = *best;
-        const int sc = (int)(key >> 42);
-        r.t1 = sc; r.t2 = PSA_NEG_INF; r.t3 = PSA_NEG_INF; r.score = sc; r.end_state = 1;
-        r.end_i = sc > 0 ? 0x1FFFFF - (int)((key >> 21) & 0x1FFFFF) : 0;
-        r.end_j = sc > 0 ? 0x1FFFFF - (int)(key & 0x1FFFFF) : 0;
-    } else {
-        auto outv = [](int v) { return v < PSA_KNEG / 2 ? PSA_NEG_INF : v; };
-        const int c1 = has_corner ? corner[0] : PSA_KNEG, c2 = has_corner ? corner[1] : PSA_KNEG, c3 = has_corner ? corner[2] : PSA_KNEG;
-        r.t1 = outv(c1); r.t2 = outv(c2); r.t3 = outv(c3); r.score = outv(imax(c1, imax(c2, c3)));
-        r.end_state = (c1 >= c2 && c1 >= c3) ? 1 : ((c2 >= c1 && c2 >= c3) ? 2 : 3);
-        r.end_i = m; r.end_j = n_total;
-    }
-    *item = r;
+    if (mode == PSA_LOCAL) { *item = local_item_from_key(*best); return; }
+    const int c1 = has_corner ? corner[0] : PSA_KNEG, c2 = has_corner ? corner[1] : PSA_KNEG, c3 = has_corner ? corner[2] : PSA_KNEG;
+    *item = global_item(c1, c2, c3, m, n_total, 0, -1);      // untyped: h is not read
 }
 
 struct SysLayout {

@@ -12,11 +12,9 @@
 // Recurrence and 4-bit direction codes exactly as in psa_short.cu (reference:
 // subproblem_alignment.cpp:229-249 for the fill, :147-169 for the predecessor order).
 #pragma once
-#include "psa_common.cuh"
+#include "psa_result.cuh"
 
 namespace psa_tile {
-
-__device__ __forceinline__ int imax(int a, int b) { return a > b ? a : b; }
 
 template <int K>
 struct Cols {
@@ -86,30 +84,6 @@ __device__ __forceinline__ void sweep(Cols<K>& cs, int hd, const int* lbH, const
         recv_h = __shfl_up_sync(0xffffffffu, hl, 1);
         recv_e = __shfl_up_sync(0xffffffffu, el, 1);
     }
-}
-
-// Border values for start_type = -1 (subproblem_alignment.cpp:259-292, :212-227).
-// Local mode uses H = 0 on the borders (E, F stay -inf): with T1 = f + max(0, .) every interior
-// T1 is >= 0, so H = max(0, H_spec) everywhere and score, end cell and path flags are those of the
-// -inf-border spec (DESIGN.md section 3) -- and no explicit 0-floor is needed in the fill.
-// st = start type of the subproblem (subproblem_alignment.cpp:212-227, 259-292): -1 the live case; -2 / -3
-// continue an open gap along row 0 / column 0 (no h on that border); 1, 2, 3 force the first state, which
-// leaves only T1[0][0] (1), row 0 (2) or column 0 (3) finite.
-template <int MODE>
-__device__ __forceinline__ int border_row0_H(int j, int g, int h, int st = -1) {   // H[0][j] = T2[0][j]; (0,0): the table st selects
-    if (MODE == PSA_LOCAL) return 0;
-    if (j == 0) return (st == 2 || st == 3) ? PSA_KNEG : 0;
-    if (st == -2) return -g * j;
-    if (st == 1 || st == 3) return PSA_KNEG;
-    return -h - g * j;
-}
-template <int MODE>
-__device__ __forceinline__ int border_col0_H(int i, int g, int h, int st = -1) {   // H[i][0] = T3[i][0]
-    if (MODE == PSA_LOCAL) return 0;
-    if (i == 0) return (st == 2 || st == 3) ? PSA_KNEG : 0;
-    if (st == -3) return -g * i;
-    if (st == 1 || st == 2) return PSA_KNEG;
-    return -h - g * i;
 }
 
 // ---- lean score-only sweep (fill kernels) ----------------------------------------------------
@@ -253,20 +227,6 @@ __device__ __forceinline__ void sweep_score(ColsS<K>& cs, int hd, const int* lbH
         recv_x = __shfl_up_sync(0xffffffffu, x, 1);
         recv_e = __shfl_up_sync(0xffffffffu, el, 1);
     }
-}
-
-// Traceback decode shared by every kernel that walks direction codes.
-// state: current state; code: 4-bit code of the SOURCE cell (0 when the source is on the border).
-// Returns the next state, or 0 when a local alignment stops at this column.
-template <int MODE>
-__device__ __forceinline__ int next_state(int state, int code, bool border) {
-    const int d1 = code & 3, z2 = (code >> 2) & 1, e3 = (code >> 3) & 1;
-    if (state == 1) {
-        if (MODE == PSA_LOCAL && (border || d1 == 0)) return 0;
-        return d1;
-    }
-    if (state == 2) return (d1 == 1) ? (z2 ? 2 : 1) : (z2 ? 2 : 3);
-    return e3 ? 3 : d1;
 }
 
 }  // namespace psa_tile

@@ -114,7 +114,7 @@ def test_long_batch_score_only(ctx, mode):
         assert it["score"] == lin.score, k
         assert (it["end_i"], it["end_j"]) == (lin.end_i, lin.end_j), k
         if mode == psa.GLOBAL:
-            assert (it["t1"], it["t2"], it["t3"]) == (lin.t1, lin.t2, lin.t3), k
+            assert (it["t1"], it["t2"], it["t3"], it["end_state"]) == (lin.t1, lin.t2, lin.t3, lin.end_state), k
 
 
 @pytest.mark.parametrize("mode", [psa.GLOBAL, psa.LOCAL])
