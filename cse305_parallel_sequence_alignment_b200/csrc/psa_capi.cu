@@ -106,9 +106,6 @@ int psa_ctx_set_option(psa_ctx* ctx, const char* name, long long value) {
     else if (k == "pack_skip_walk") o.pack_skip_walk = (int)value;
     else if (k == "pack_ctas_per_sm") o.pack_ctas_per_sm = (int)value;
     else if (k == "pack_chunk") o.pack_chunk = value < 1024 ? 1024 : value;
-    else if (k == "pack_ramp") o.pack_ramp = (int)value;
-    else if (k == "pack_streams") o.pack_streams = (int)value;
-    else if (k == "pack_compact_probe") o.pack_compact_probe = (int)value;
     else if (k == "pack_serial_fills") o.pack_serial_fills = (int)value;
     else if (k == "pack_long_k") o.pack_long_k = (int)value;
     else if (k == "long_geometry") o.long_geometry = (int)value;
@@ -264,6 +261,8 @@ static int align_batch_host(psa_ctx* ctx, const uint8_t* bases_a, const int64_t*
     }
     int rc = check_scoring(ctx, mode, g, h, max_m, max_n);
     if (rc) return rc;
+    if (tb && ops_stride_words * 16 < (size_t)max_m + max_n)
+        return psa_fail(ctx, PSA_ERR_CAPACITY, "ops_stride_words < ceil((max m + max n)/16)");
     PSA_CUDA_OK(ctx, cudaSetDevice(ctx->device));
     // an asynchronous device call of this context may still be using the shared scratch on a user stream
     if (ctx->last_valid) { PSA_CUDA_OK(ctx, cudaEventSynchronize(ctx->last_event)); ctx->last_valid = false; }
@@ -292,13 +291,11 @@ static int align_batch_host(psa_ctx* ctx, const uint8_t* bases_a, const int64_t*
         PSA_CUDA_OK(ctx, cudaMemcpyAsync(d + o_ty, ty.per_pair, n_pairs, cudaMemcpyHostToDevice, st));
     }
     const bool typed = ty.any();
-    // large DNA batches laid out back to back: chunked copy/compute pipeline on two streams
+    // large DNA batches laid out back to back: chunked copy/compute pipeline on the four aux streams
     if (!typed && contiguous && n_pairs > (size_t)ctx->opt.pack_chunk && psa_short_supported(max_m, max_n, tb) &&
         psa_pack_supported(max_m, max_n, mode, g, h) && ctx->opt.pack && ctx->opt.pipeline) {
         psa_batch_args host{bases_a, off_a, len_a, bases_b, off_b, len_b, (int64_t)n_pairs, g, h, items, ops,
                             (int64_t)ops_stride_words};
-        if (tb && ops_stride_words * 16 < (size_t)max_m + max_n)
-            return psa_fail(ctx, PSA_ERR_CAPACITY, "ops_stride_words < ceil((max m + max n)/16)");
         const auto t_valid = std::chrono::steady_clock::now();
         rc = psa_pack_pipeline(ctx, args, host, bytes_a, bytes_b, max_m, max_n, mode, tb);
         if (ctx->opt.timing) {
@@ -491,7 +488,7 @@ int psa_align_batch_packed(psa_ctx* ctx, const uint32_t* a2, const uint32_t* b2,
                         (psa_batch_item*)(d + o_it), tb ? (uint32_t*)(d + o_op) : nullptr, (int64_t)ops_stride_words};
     args.a2 = (const uint32_t*)(d + o_a); args.b2 = (const uint32_t*)(d + o_b);
     args.wa = wa; args.wb = wb; args.fixed_m = len_a; args.fixed_n = len_b;
-    return psa_pack_pipeline_packed(ctx, args, a2, b2, (psa_packed_item*)(d + o_i16), items, ops, mode, tb, compact, d + o_cp, nullptr);
+    return psa_pack_pipeline_packed(ctx, args, a2, b2, (psa_packed_item*)(d + o_i16), items, ops, mode, tb, compact, d + o_cp);
 }
 
 void psa_ops_unpack(const uint32_t* words, int32_t aln_len, uint8_t* ops_forward) {

@@ -21,11 +21,8 @@ struct psa_options {
     int pack_traceback = 0;       // 0: per-cell direction codes in a recycled global ring (faster: DESIGN.md section 4);
                                   // 1: tile-boundary checkpoints + per-tile recompute (no code stream at all)
     int pack_skip_walk = 0;       // measurement only: fill launches without the traceback walk (results lack ops)
-    int pack_streams = 4;         // chunks in flight in psa_align_batch_packed's host pipeline (2 - 4)
-    int pack_compact_probe = 0;   // measurement only: 1 = PSA_OPS_COMPACT without the packing kernel, 2 = also without the scan (results lack ops)
     int pack_ctas_per_sm = 0;     // > 0: cap of resident CTAs per SM of the packed fill kernel
     long long pack_chunk = 131072;
-    int pack_ramp = 1;            // ramped chunk sizes at both ends of the host pipeline
     int pack_serial_fills = 0;    // 1: host pipelines start fill(c) when fill(c-1) has finished, so chunks complete evenly spaced, in
                                   // order (0: the four in-flight fills share the SMs and finish together, their D2H in one burst)
     int pack_long_k = 0;          // 8 / 16: force the lane width of the packed long-batch kernel
@@ -138,13 +135,13 @@ int psa_launch_short_flagged(psa_ctx* ctx, const psa_batch_args& args, int max_m
 bool psa_pack_supported(int max_m, int max_n, int mode, int g, int h);
 int psa_launch_pack(psa_ctx* ctx, const psa_batch_args& args, int max_m, int max_n, int mode, bool traceback,
                     cudaStream_t stream);
-// host-buffer pipeline: per-chunk H2D -> fill -> traceback -> D2H on two alternating streams
+// host-buffer pipelines over one chunk driver: per-chunk H2D -> fill -> traceback -> D2H, chunk c on aux stream c % 4
 int psa_pack_pipeline(psa_ctx* ctx, const psa_batch_args& dev, const psa_batch_args& host, size_t bytes_a, size_t bytes_b,
                       int max_m, int max_n, int mode, bool traceback);
 // the same pipeline for 2-bit packed fixed-stride input and 16-byte result records (psa_align_batch_packed)
 int psa_pack_pipeline_packed(psa_ctx* ctx, const psa_batch_args& dev, const uint32_t* h_a2, const uint32_t* h_b2,
                              psa_packed_item* d_items16, psa_packed_item* h_items16, uint32_t* h_ops, int mode, bool traceback,
-                             bool compact, uint8_t* d_compact, uint64_t* total_words);
+                             bool compact, uint8_t* d_compact);
 int psa_launch_peak(psa_ctx* ctx, int kind, double* lane_ops_per_s, double* ms);
 int psa_launch_similarity(psa_ctx* ctx, const psa_batch_args& args, int max_len, double* d_out, cudaStream_t st);
 // column-stationary systolic kernel (psa_systolic.cu): the panels first_panel, first_panel + panel_step, ... of one pair

@@ -13,9 +13,9 @@
 extern "C" {
 #endif
 
-/* name: pack, pipeline, pack_traceback, pack_skip_walk, pack_ctas_per_sm, pack_chunk, pack_ramp, pack_serial_fills,
- *       pack_streams, pack_compact_probe, pack_long_k, long_geometry, long_ctas_per_sm, long_band, long_tb_chunk,
- *       long_systolic, systolic_warps_per_sm, systolic_kc, systolic_rb, timing
+/* name: pack, pipeline, pack_traceback, pack_skip_walk, pack_ctas_per_sm, pack_chunk, pack_serial_fills, pack_long_k,
+ *       long_geometry, long_ctas_per_sm, long_band, long_tb_chunk, long_systolic, systolic_warps_per_sm, systolic_kc,
+ *       systolic_rb, timing
  * (struct psa_options in psa_common.cuh).  Returns PSA_ERR_ARG for an unknown name. */
 int psa_ctx_set_option(psa_ctx* ctx, const char* name, long long value);
 

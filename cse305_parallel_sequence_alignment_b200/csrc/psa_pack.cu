@@ -29,6 +29,8 @@
 // (psa_short.cu) -- results stay bit-exact for any alphabet.
 #include "psa_result.cuh"
 #include <chrono>
+#include <functional>
+#include <type_traits>
 #include <vector>
 
 namespace {
@@ -230,8 +232,8 @@ __device__ __forceinline__ void pack_walk(const uint32_t* __restrict__ dbase, in
 
 // Traceback flavours of the fill kernel.
 //   TB_CODES : every cell leaves a 5-bit direction code in a global ring (20 KB per 150 x 150 pair), walked by
-//              psa_pack_tb_kernel -- the round-1 design, kept for comparison (option pack_traceback = 1).
-//   TB_CKPT  : the fill keeps only tile-boundary checkpoints (11 KB per pair): the (H-(g+h), E) every lane receives
+//              psa_pack_tb_kernel -- the default (option pack_traceback = 0), faster than TB_CKPT (DESIGN.md section 4).
+//   TB_CKPT  : (option pack_traceback = 1) the fill keeps only tile-boundary checkpoints (11 KB per pair): the (H-(g+h), E) every lane receives
 //              from its left neighbour at every step (= the boundary column between two lanes' strips) and, every
 //              PACK_RS wavefront steps, every lane's column state (H-(g+h), F).  psa_pack_rwalk_kernel then
 //              recomputes only the <= PACK_RS x K tiles the path crosses, codes in shared memory -- no O(mn)
@@ -861,6 +863,23 @@ bool pick_shape(int max_n, Shape& s) {
     return true;
 }
 
+// Calls f(integral_constant<int, G>, integral_constant<int, K>) for the shape pick_shape chose: the one list of the
+// (G, K) instantiations of the fill and walk kernels.
+template <class F>
+int with_shape(const Shape& s, F&& f) {
+    using std::integral_constant;
+    switch (s.G * 100 + s.K) {
+        case 804: return f(integral_constant<int, 8>{}, integral_constant<int, 4>{});
+        case 808: return f(integral_constant<int, 8>{}, integral_constant<int, 8>{});
+        case 812: return f(integral_constant<int, 8>{}, integral_constant<int, 12>{});
+        case 816: return f(integral_constant<int, 8>{}, integral_constant<int, 16>{});
+        case 819: return f(integral_constant<int, 8>{}, integral_constant<int, 19>{});
+        case 820: return f(integral_constant<int, 8>{}, integral_constant<int, 20>{});
+        case 1612: return f(integral_constant<int, 16>{}, integral_constant<int, 12>{});
+        default: return f(integral_constant<int, 16>{}, integral_constant<int, 16>{});
+    }
+}
+
 }  // namespace
 
 bool psa_pack_supported(int max_m, int max_n, int mode, int g, int h) {
@@ -874,42 +893,58 @@ bool psa_pack_supported(int max_m, int max_n, int mode, int g, int h) {
     return top < 32000;
 }
 
-// One chunk [pair0, pair0+pairs) of the batch on `st`, using direction-code ring `ring` (0/1).
-// `flags` = fallback bytes for the WHOLE batch (indexed by absolute pair).
-static int tb_flavour(const psa_ctx* ctx, bool traceback) {
-    if (!traceback) return TB_NONE;
-    return ctx->opt.pack_traceback == 1 ? TB_CKPT : TB_CODES;
-}
+namespace {
 
-static long long pairs_cap_round(long long pairs) { return (pairs + 63) / 64 * 64; }
+constexpr int kInFlight = 4;     // chunks in flight: rings, perm buffers and aux streams (DESIGN.md section 5)
+constexpr int kCounters = 4096;  // flagged-pair counters, one per chunk
+
+// What every chunk of one packed batch shares, decided once per call by pack_plan: the kernel shape and constants,
+// the traceback flavour and the scratch in ctx->d_work.  Chunk c uses ring and perm buffer c % kInFlight and, for
+// byte input, flagged-pair counter c.
+struct PackPlan {
+    psa_batch_args args;               // device view of the whole batch
+    int max_m, max_n, mode;
+    int flavour;                       // TB_NONE (score only), TB_CODES or TB_CKPT
+    Shape sh;
+    PackConsts C;
+    uint8_t* flags;                    // fallback bytes of the WHOLE batch (indexed by absolute pair)
+    int* counters;                     // [kCounters]
+    uint32_t* rings[kInFlight];        // direction codes or checkpoints of one chunk
+    int* perms[kInFlight];             // visiting order of the tile-recompute walk (TB_CKPT only, else null)
+    long long slot_words;              // ring words per pair-of-pairs
+};
+
+long long pairs_cap_round(long long pairs) { return (pairs + 63) / 64 * 64; }
 
 template <int G, int K>
-static int launch_walk(psa_ctx* ctx, int flavour, const psa_batch_args& args, const PackConsts& C, const uint32_t* ring,
-                       long long slot_words, int m_cap, int n_cap, long long pair0, long long pairs, const uint8_t* flags, int mode,
-                       int span, int* perm, cudaStream_t st) {
-    if (flavour == TB_CODES) {
+int launch_walk(psa_ctx* ctx, const PackPlan& P, const uint32_t* ring, int* perm, long long pair0, long long pairs,
+                cudaStream_t st) {
+    const psa_batch_args& args = P.args;
+    const bool local = P.mode == PSA_LOCAL;
+    if (P.flavour == TB_CODES) {
         PackTbArgs T;
-        T.P = args; T.C = C; T.dirs = ring; T.dirs_slot_words = slot_words; T.pair0 = pair0; T.pairs = pairs;
-        T.fallback = flags; T.local = (mode == PSA_LOCAL);
-        pack_tb_lut(C.h, T.lut);
+        T.P = args; T.C = P.C; T.dirs = ring; T.dirs_slot_words = P.slot_words; T.pair0 = pair0; T.pairs = pairs;
+        T.fallback = P.flags; T.local = local;
+        pack_tb_lut(P.C.h, T.lut);
         psa_pack_tb_kernel<G, K><<<(int)((pairs + 127) / 128), 128, 0, st>>>(T);
         PSA_CUDA_OK(ctx, cudaGetLastError());
         ctx->launches += 1;
         return PSA_OK;
     }
     // visiting order, then the tile-recompute walk
+    const int span = local ? std::min(P.max_m, P.max_n) : (P.max_m + P.max_n) / 2;
     int* hist = perm + pairs_cap_round(pairs);          // 64 ints behind the permutation
     PSA_CUDA_OK(ctx, cudaMemsetAsync(hist, 0, 64 * sizeof(int), st));
     for (int pass = 0; pass < 2; ++pass)
         psa_pack_perm_kernel<<<(int)((pairs + 255) / 256), 256, 0, st>>>(args.items, args.len_a, args.len_b, pair0, (int)pairs,
-                                                                          mode == PSA_LOCAL ? 1 : 0, span, hist, perm, pass);
+                                                                          local ? 1 : 0, span, hist, perm, pass);
     PSA_CUDA_OK(ctx, cudaGetLastError());
     PackWalkArgs W;
-    W.P = args; W.C = C; W.ck = reinterpret_cast<const uint2*>(ring); W.ck_slot = slot_words / 2; W.ck_col = ck_col_u2(m_cap, G);
-    W.pair0 = pair0; W.pairs = pairs; W.fallback = flags; W.perm = perm; W.local = (mode == PSA_LOCAL);
-    pack_tb_lut(C.h, W.lut);
-    W.m_cap = m_cap;
-    const size_t smem = rwalk_smem_words(K, m_cap, n_cap) * 128 * sizeof(uint32_t);
+    W.P = args; W.C = P.C; W.ck = reinterpret_cast<const uint2*>(ring); W.ck_slot = P.slot_words / 2; W.ck_col = ck_col_u2(P.max_m, G);
+    W.pair0 = pair0; W.pairs = pairs; W.fallback = P.flags; W.perm = perm; W.local = local;
+    pack_tb_lut(P.C.h, W.lut);
+    W.m_cap = P.max_m;
+    const size_t smem = rwalk_smem_words(K, P.max_m, P.max_n) * 128 * sizeof(uint32_t);
     if (smem + 1024 > (size_t)ctx->smem_optin) return psa_fail(ctx, PSA_ERR_RANGE, "tile-recompute walk does not fit in shared memory");
     auto kern = psa_pack_rwalk_kernel<G, K>;
     const int orc = psa_kernel_optin_smem(ctx, (const void*)kern);
@@ -920,65 +955,54 @@ static int launch_walk(psa_ctx* ctx, int flavour, const psa_batch_args& args, co
     return PSA_OK;
 }
 
-static int pack_chunk(psa_ctx* ctx, const psa_batch_args& args, long long pair0, long long pairs, int max_m, int max_n,
-                      int mode, bool traceback, const Shape& sh, const PackConsts& C, uint8_t* flags, uint32_t* ring,
-                      long long slot_words, cudaStream_t st, int* flag_count = nullptr, int* perm = nullptr,
-                      cudaEvent_t fill_after = nullptr, cudaEvent_t fill_done = nullptr) {
-    // fill_after / fill_done: optional ordering of the fills of consecutive chunks that run on different streams
-    const int flavour = tb_flavour(ctx, traceback);
+// Chunk c, the pairs [pair0, pair0 + pairs) of the planned batch, on stream `st`: fill, traceback walk and, for byte
+// input, the generic kernel on the members the fill flagged.  fill_after / fill_done optionally order the fills of
+// consecutive chunks that run on different streams (option pack_serial_fills).
+int pack_chunk(psa_ctx* ctx, const PackPlan& P, int c, long long pair0, long long pairs, cudaStream_t st,
+               cudaEvent_t fill_after = nullptr, cudaEvent_t fill_done = nullptr) {
+    const bool bytes = P.args.a2 == nullptr;         // 2-bit input is plain ACGT: nothing can be flagged
+    const bool traceback = P.flavour != TB_NONE;
+    uint32_t* ring = P.rings[c % kInFlight];
+    int* flag_count = (bytes && c < kCounters) ? P.counters + c : nullptr;
     PackArgs A;
-    A.P = args; A.C = C; A.m_cap = max_m;
+    A.P = P.args; A.C = P.C; A.m_cap = P.max_m;
     A.dirs = traceback ? ring : nullptr;
-    A.dirs_slot_words = slot_words; A.pair0 = pair0; A.pairs = pairs;
-    A.fallback = flags;
+    A.dirs_slot_words = P.slot_words; A.pair0 = pair0; A.pairs = pairs;
+    A.fallback = P.flags;
     A.flag_count = flag_count;
     if (flag_count) PSA_CUDA_OK(ctx, cudaMemsetAsync(flag_count, 0, sizeof(int), st));
     if (fill_after) PSA_CUDA_OK(ctx, cudaStreamWaitEvent(st, fill_after, 0));
-    int rc;
-    switch (sh.G * 100 + sh.K) {
-        case 804: rc = launch_fill<8, 4>(ctx, A, mode, flavour, st); break;
-        case 808: rc = launch_fill<8, 8>(ctx, A, mode, flavour, st); break;
-        case 812: rc = launch_fill<8, 12>(ctx, A, mode, flavour, st); break;
-        case 816: rc = launch_fill<8, 16>(ctx, A, mode, flavour, st); break;
-        case 819: rc = launch_fill<8, 19>(ctx, A, mode, flavour, st); break;
-        case 820: rc = launch_fill<8, 20>(ctx, A, mode, flavour, st); break;
-        case 1612: rc = launch_fill<16, 12>(ctx, A, mode, flavour, st); break;
-        default: rc = launch_fill<16, 16>(ctx, A, mode, flavour, st); break;
-    }
+    int rc = with_shape(P.sh, [&](auto G, auto K) {
+        return launch_fill<decltype(G)::value, decltype(K)::value>(ctx, A, P.mode, P.flavour, st);
+    });
     if (rc) return rc;
     if (fill_done) PSA_CUDA_OK(ctx, cudaEventRecord(fill_done, st));
     // opt.pack_skip_walk: measurement hook (psa_internal.h) -- bench.py times the fill launches alone with it
     if (traceback && !ctx->opt.pack_skip_walk) {
-        const int span = (mode == PSA_LOCAL) ? std::min(max_m, max_n) : (max_m + max_n) / 2;
-        switch (sh.G * 100 + sh.K) {
-            case 804: rc = launch_walk<8, 4>(ctx, flavour, args, C, ring, slot_words, max_m, max_n, pair0, pairs, flags, mode, span, perm, st); break;
-            case 808: rc = launch_walk<8, 8>(ctx, flavour, args, C, ring, slot_words, max_m, max_n, pair0, pairs, flags, mode, span, perm, st); break;
-            case 812: rc = launch_walk<8, 12>(ctx, flavour, args, C, ring, slot_words, max_m, max_n, pair0, pairs, flags, mode, span, perm, st); break;
-            case 816: rc = launch_walk<8, 16>(ctx, flavour, args, C, ring, slot_words, max_m, max_n, pair0, pairs, flags, mode, span, perm, st); break;
-            case 819: rc = launch_walk<8, 19>(ctx, flavour, args, C, ring, slot_words, max_m, max_n, pair0, pairs, flags, mode, span, perm, st); break;
-            case 820: rc = launch_walk<8, 20>(ctx, flavour, args, C, ring, slot_words, max_m, max_n, pair0, pairs, flags, mode, span, perm, st); break;
-            case 1612: rc = launch_walk<16, 12>(ctx, flavour, args, C, ring, slot_words, max_m, max_n, pair0, pairs, flags, mode, span, perm, st); break;
-            default: rc = launch_walk<16, 16>(ctx, flavour, args, C, ring, slot_words, max_m, max_n, pair0, pairs, flags, mode, span, perm, st); break;
-        }
+        rc = with_shape(P.sh, [&](auto G, auto K) {
+            return launch_walk<decltype(G)::value, decltype(K)::value>(ctx, P, ring, P.perms[c % kInFlight], pair0, pairs, st);
+        });
         if (rc) return rc;
     }
-    if (args.a2 != nullptr) return PSA_OK;           // 2-bit input: nothing can be flagged
+    if (!bytes) return PSA_OK;
     // members flagged by the fill (non-ACGT bytes, zero lengths) are recomputed by the generic kernel
-    psa_batch_args sub = args;
+    psa_batch_args sub = P.args;
     sub.off_a += pair0; sub.len_a += pair0; sub.off_b += pair0; sub.len_b += pair0; sub.items += pair0;
-    if (sub.ops) sub.ops += pair0 * args.ops_stride_words;
+    if (sub.ops) sub.ops += pair0 * P.args.ops_stride_words;
     sub.n_pairs = pairs;
     sub.flagged_count = flag_count;
-    return psa_launch_short_flagged(ctx, sub, max_m, max_n, mode, traceback, flags + pair0, st);
+    return psa_launch_short_flagged(ctx, sub, P.max_m, P.max_n, P.mode, traceback, P.flags + pair0, st);
 }
 
-// Plans the scratch (fallback flags + two direction-code rings) for a batch; returns pointers.
-static int pack_plan(psa_ctx* ctx, const psa_batch_args& args, int max_m, int max_n, int mode, bool traceback,
-                     Shape& sh, PackConsts& C, uint8_t** flags, uint32_t** rings /*[nrings]*/, int nrings, long long* slot_words,
-                     int** counters, int** perms /*[nrings]*/) {
-    if (!pick_shape(max_n, sh)) return psa_fail(ctx, PSA_ERR_RANGE, "packed kernel: n > 256");
-    const int NWP = pad_words(words_for(sh.K));
+// Plans a batch: shape, constants and traceback flavour, and the scratch in ctx->d_work (fallback flags, counters and
+// kInFlight rings and perm buffers of one chunk each).
+int pack_plan(psa_ctx* ctx, const psa_batch_args& args, int max_m, int max_n, int mode, bool traceback, PackPlan& P) {
+    P.args = args; P.max_m = max_m; P.max_n = max_n; P.mode = mode;
+    P.flavour = !traceback ? TB_NONE : (ctx->opt.pack_traceback == 1 ? TB_CKPT : TB_CODES);
+    if (!pick_shape(max_n, P.sh)) return psa_fail(ctx, PSA_ERR_RANGE, "packed kernel: n > 256");
+    const int NWP = pad_words(words_for(P.sh.K));
     const int g = args.g, h = args.h;
+    PackConsts& C = P.C;
     C.g = g; C.h = h;
     C.bias = (int)pack_bias(mode, g, h, max_m, max_n);
     C.ng2 = (uint32_t)((-g) & 0xffff) * 0x00010001u;
@@ -990,16 +1014,14 @@ static int pack_plan(psa_ctx* ctx, const psa_batch_args& args, int max_m, int ma
         const uint32_t sc = x == 0 ? 1u : (x == 1 ? 32u : 1024u);
         C.cH[x] = 11u * sc; C.cT[x] = 0u - sc; C.cE[x] = 0u - 2u * sc; C.cF[x] = 0u - 8u * sc;
     }
-    const int flavour = tb_flavour(ctx, traceback);
-    *slot_words = flavour == TB_CKPT ? 2 * ck_slot_u2(max_m, sh.G, sh.K) : dirs_slot_words_for(max_m, sh.G, NWP);   // per pair-of-pairs
+    P.slot_words = P.flavour == TB_CKPT ? 2 * ck_slot_u2(max_m, P.sh.G, P.sh.K) : dirs_slot_words_for(max_m, P.sh.G, NWP);
     const long long chunk = std::min<long long>(ctx->opt.pack_chunk, args.n_pairs);
-    const size_t ring_bytes = traceback ? ((size_t)((chunk + 1) / 2) * (size_t)*slot_words * 4 + 255) / 256 * 256 : 0;
-    const size_t perm_bytes = flavour == TB_CKPT ? ((size_t)(pairs_cap_round(chunk) + 64) * sizeof(int) + 255) / 256 * 256 : 0;
-    constexpr size_t kCounters = 4096;                       // one flagged-pair counter per chunk
+    const size_t ring_bytes = traceback ? ((size_t)((chunk + 1) / 2) * (size_t)P.slot_words * 4 + 255) / 256 * 256 : 0;
+    const size_t perm_bytes = P.flavour == TB_CKPT ? ((size_t)(pairs_cap_round(chunk) + 64) * sizeof(int) + 255) / 256 * 256 : 0;
     const size_t o_cnt = ((size_t)args.n_pairs + 255) / 256 * 256;
     const size_t o_perm = o_cnt + kCounters * sizeof(int);
-    const size_t o_d0 = o_perm + (size_t)nrings * perm_bytes;
-    const size_t total = o_d0 + (size_t)nrings * ring_bytes + 256;
+    const size_t o_d0 = o_perm + (size_t)kInFlight * perm_bytes;
+    const size_t total = o_d0 + (size_t)kInFlight * ring_bytes + 256;
     if (total > ctx->d_work_bytes) {
         if (ctx->d_work) cudaFree(ctx->d_work);
         ctx->d_work = nullptr; ctx->d_work_bytes = 0;
@@ -1007,16 +1029,15 @@ static int pack_plan(psa_ctx* ctx, const psa_batch_args& args, int max_m, int ma
         ctx->d_work_bytes = total;
     }
     uint8_t* d = (uint8_t*)ctx->d_work;
-    *flags = d;
-    *counters = (int*)(d + o_cnt);
-    for (int k = 0; k < nrings; ++k) {
-        rings[k] = (uint32_t*)(d + o_d0 + (size_t)k * ring_bytes);
-        perms[k] = perm_bytes ? (int*)(d + o_perm + (size_t)k * perm_bytes) : nullptr;
+    P.flags = d;
+    P.counters = (int*)(d + o_cnt);
+    for (int k = 0; k < kInFlight; ++k) {
+        P.rings[k] = (uint32_t*)(d + o_d0 + (size_t)k * ring_bytes);
+        P.perms[k] = perm_bytes ? (int*)(d + o_perm + (size_t)k * perm_bytes) : nullptr;
     }
     return PSA_OK;
 }
 
-namespace {
 // events of one pipeline call (destroyed when the call returns, on every path)
 struct EventList {
     std::vector<cudaEvent_t> ev;
@@ -1028,24 +1049,97 @@ struct EventList {
     cudaEvent_t at(size_t k) const { return k < ev.size() ? ev[k] : nullptr; }
     ~EventList() { for (auto e : ev) if (e) cudaEventDestroy(e); }
 };
-}  // namespace
 
 int psa_ensure_aux(psa_ctx* ctx) {
     if (!ctx->aux_stream[0]) {
-        for (int k = 0; k < 4; ++k) PSA_CUDA_OK(ctx, cudaStreamCreateWithFlags(&ctx->aux_stream[k], cudaStreamNonBlocking));
+        for (int k = 0; k < kInFlight; ++k) PSA_CUDA_OK(ctx, cudaStreamCreateWithFlags(&ctx->aux_stream[k], cudaStreamNonBlocking));
         PSA_CUDA_OK(ctx, cudaStreamCreateWithFlags(&ctx->post_stream, cudaStreamNonBlocking));
         for (int k = 0; k < 3; ++k) PSA_CUDA_OK(ctx, cudaEventCreateWithFlags(&ctx->aux_event[k], cudaEventDisableTiming));
     }
     return PSA_OK;
 }
 
-// The whole device-resident batch, chunk by chunk; chunks alternate between two internal streams
-// so that the traceback of chunk c overlaps the fill of chunk c+1.  fork/join around `user`.
+// Chunk schedule of the host pipelines: full-size chunks in the middle, ramped down to chunk/8 at both ends -- the
+// first chunk's H2D copy and the last chunk's D2H copy are the only transfers nothing overlaps.
+std::vector<long long> chunk_sizes(long long chunk, long long n) {
+    const long long ramp[3] = {chunk / 8, chunk / 4, chunk / 2};
+    const long long ramp_sum = ramp[0] + ramp[1] + ramp[2];
+    const bool ramped = n >= 2 * ramp_sum + chunk && chunk >= 8192;
+    std::vector<long long> sizes;
+    if (ramped) sizes.assign(ramp, ramp + 3);
+    for (long long mid = ramped ? n - 2 * ramp_sum : n; mid > 0; mid -= chunk) sizes.push_back(std::min(chunk, mid));
+    if (ramped) sizes.insert(sizes.end(), {ramp[2], ramp[1], ramp[0]});
+    return sizes;
+}
+
+// The per-chunk steps in which the host pipelines differ.  Each gets the chunk index, its pairs [p0, p0 + cnt) and
+// its stream, and returns a psa_status.
+struct ChunkSteps {
+    std::function<int(size_t n_chunks)> begin;                        // once, before the first chunk (may be empty)
+    std::function<int(int c, long long p0, long long cnt, cudaStream_t st)> inputs, records, outputs;   // records may be empty
+    bool post = false;                                                // `records` enqueues work on ctx->post_stream
+};
+
+// Host-buffer pipeline: chunk c's H2D copies, fill, traceback, records and D2H copies all go to aux stream
+// c % kInFlight, so that the copies of one chunk overlap the kernels of the others.  Returns when every chunk's
+// results are on the host.
+int pack_pipeline(psa_ctx* ctx, const psa_batch_args& args, int max_m, int max_n, int mode, bool traceback, const ChunkSteps& s) {
+    PackPlan P;
+    int rc = pack_plan(ctx, args, max_m, max_n, mode, traceback, P);
+    if (rc) return rc;
+    rc = psa_ensure_aux(ctx);
+    if (rc) return rc;
+    const std::vector<long long> sizes = chunk_sizes(ctx->opt.pack_chunk, args.n_pairs);
+    EventList fills, marks;
+    rc = fills.create(ctx, ctx->opt.pack_serial_fills ? sizes.size() : 0);
+    if (rc) return rc;
+    if (s.begin && (rc = s.begin(sizes.size()))) return rc;
+    const bool tl = ctx->opt.timing >= 2;      // debugging aid: GPU-side timeline of every chunk
+    auto mark = [&](cudaStream_t st) {
+        if (tl) { cudaEvent_t e; cudaEventCreate(&e); cudaEventRecord(e, st); marks.ev.push_back(e); }
+    };
+    const auto t0 = std::chrono::steady_clock::now();
+    long long p0 = 0;
+    for (int c = 0; c < (int)sizes.size(); p0 += sizes[c], ++c) {
+        cudaStream_t st = ctx->aux_stream[c % kInFlight];
+        const long long cnt = sizes[c];
+        mark(st);
+        if ((rc = s.inputs(c, p0, cnt, st))) return rc;
+        mark(st);
+        if ((rc = pack_chunk(ctx, P, c, p0, cnt, st, c > 0 ? fills.at(c - 1) : nullptr, fills.at(c)))) return rc;
+        mark(st);
+        if (s.records && (rc = s.records(c, p0, cnt, st))) return rc;
+        mark(st);
+        if ((rc = s.outputs(c, p0, cnt, st))) return rc;
+        mark(st);
+    }
+    const auto t_enq = std::chrono::steady_clock::now();
+    for (int k = 0; k < kInFlight; ++k) PSA_CUDA_OK(ctx, cudaStreamSynchronize(ctx->aux_stream[k]));
+    if (s.post) PSA_CUDA_OK(ctx, cudaStreamSynchronize(ctx->post_stream));
+    if (tl) {
+        for (size_t c = 0; c < sizes.size(); ++c) {
+            float t[5];
+            for (int q = 0; q < 5; ++q) cudaEventElapsedTime(&t[q], marks.ev[0], marks.ev[5 * c + q]);
+            fprintf(stderr, "  chunk %2d (%6lld pairs): h2d %.3f-%.3f  fill+walk -%.3f  records -%.3f  d2h -%.3f\n", (int)c,
+                    sizes[c], t[0], t[1], t[2], t[3], t[4]);
+        }
+    }
+    if (ctx->opt.timing)
+        fprintf(stderr, "psa_pack_pipeline: %d chunks enqueued in %.3f ms, drained %.3f ms later\n", (int)sizes.size(),
+                std::chrono::duration<double, std::milli>(t_enq - t0).count(),
+                std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_enq).count());
+    return PSA_OK;
+}
+
+}  // namespace
+
+// The whole device-resident batch, chunk by chunk on the kInFlight aux streams, so that the traceback of one chunk
+// overlaps the fills of the others; fork / join around `user`, no host synchronisation.  Without traceback the batch
+// is one chunk on `user`.
 int psa_launch_pack(psa_ctx* ctx, const psa_batch_args& args, int max_m, int max_n, int mode, bool traceback,
                     cudaStream_t user) {
-    constexpr int NS = 4;       // chunks in flight: the latency-bound traceback of one chunk hides under the fills of the others
-    Shape sh; PackConsts C; uint8_t* flags; uint32_t* rr[NS]; long long slot_words; int* counters; int* perms[NS];
-    int rc = pack_plan(ctx, args, max_m, max_n, mode, traceback, sh, C, &flags, rr, NS, &slot_words, &counters, perms);
+    PackPlan P;
+    int rc = pack_plan(ctx, args, max_m, max_n, mode, traceback, P);
     if (rc) return rc;
     const long long chunk = traceback ? ctx->opt.pack_chunk : args.n_pairs;
     const bool split = args.n_pairs > chunk;
@@ -1053,16 +1147,15 @@ int psa_launch_pack(psa_ctx* ctx, const psa_batch_args& args, int max_m, int max
         rc = psa_ensure_aux(ctx);
         if (rc) return rc;
         PSA_CUDA_OK(ctx, cudaEventRecord(ctx->aux_event[0], user));
-        for (int k = 0; k < NS; ++k) PSA_CUDA_OK(ctx, cudaStreamWaitEvent(ctx->aux_stream[k], ctx->aux_event[0], 0));
+        for (int k = 0; k < kInFlight; ++k) PSA_CUDA_OK(ctx, cudaStreamWaitEvent(ctx->aux_stream[k], ctx->aux_event[0], 0));
     }
     int c = 0;
     for (long long p0 = 0; p0 < args.n_pairs; p0 += chunk, ++c) {
-        rc = pack_chunk(ctx, args, p0, std::min<long long>(chunk, args.n_pairs - p0), max_m, max_n, mode, traceback, sh, C,
-                        flags, rr[c % NS], slot_words, split ? ctx->aux_stream[c % NS] : user, c < 4096 ? counters + c : nullptr, perms[c % NS]);
+        rc = pack_chunk(ctx, P, c, p0, std::min<long long>(chunk, args.n_pairs - p0), split ? ctx->aux_stream[c % kInFlight] : user);
         if (rc) return rc;
     }
     if (split) {
-        for (int k = 0; k < NS; ++k) {          // join: one event, re-recorded per stream, waited on in order
+        for (int k = 0; k < kInFlight; ++k) {          // join: one event, re-recorded per stream, waited on in order
             PSA_CUDA_OK(ctx, cudaEventRecord(ctx->aux_event[1], ctx->aux_stream[k]));
             PSA_CUDA_OK(ctx, cudaStreamWaitEvent(user, ctx->aux_event[1], 0));
         }
@@ -1070,83 +1163,31 @@ int psa_launch_pack(psa_ctx* ctx, const psa_batch_args& args, int max_m, int max
     return PSA_OK;
 }
 
-// Host-buffer pipeline (psa_align_batch): chunk c's H2D copies, fill, traceback and D2H copies all
-// go to stream c%2, so copies of one chunk overlap the kernels of the other.  `h` = host arrays,
-// `args` = the device mirror (same layout).  contiguous = offsets are ascending and back to back,
-// so a chunk's bases are one contiguous range.
+// Byte input (psa_align_batch): `h` = host arrays, `args` = their device mirror (same layout).  The offsets are
+// ascending and back to back, so a chunk's bases are one contiguous range.
 int psa_pack_pipeline(psa_ctx* ctx, const psa_batch_args& args, const psa_batch_args& h, size_t bytes_a, size_t bytes_b,
                       int max_m, int max_n, int mode, bool traceback) {
-    // NS chunks in flight: with two, a stream's D2H + next H2D leave the SMs to a single chunk
-    constexpr int NS = 4;
-    Shape sh; PackConsts C; uint8_t* flags; uint32_t* rr[NS]; long long slot_words; int* counters; int* perms[NS];
-    int rc = pack_plan(ctx, args, max_m, max_n, mode, traceback, sh, C, &flags, rr, NS, &slot_words, &counters, perms);
-    if (rc) return rc;
-    rc = psa_ensure_aux(ctx);
-    if (rc) return rc;
-    const long long chunk = ctx->opt.pack_chunk;
-    const long long n = args.n_pairs;
-    // Chunk schedule: full-size chunks in the middle, ramped down to chunk/8 at both ends -- the first
-    // chunk's H2D copy and the last chunk's D2H copy are the only transfers nothing overlaps.
-    std::vector<long long> sizes;
-    {
-        const long long ramp[3] = {chunk / 8, chunk / 4, chunk / 2};
-        const long long ramp_sum = ramp[0] + ramp[1] + ramp[2];
-        if (n >= 2 * ramp_sum + chunk && chunk >= 8192 && ctx->opt.pack_ramp) {
-            for (int k = 0; k < 3; ++k) sizes.push_back(ramp[k]);
-            long long mid = n - 2 * ramp_sum;
-            while (mid > 0) { const long long t = std::min(chunk, mid); sizes.push_back(t); mid -= t; }
-            for (int k = 2; k >= 0; --k) sizes.push_back(ramp[k]);
-        } else {
-            for (long long p = 0; p < n; p += chunk) sizes.push_back(std::min(chunk, n - p));
-        }
-    }
-    EventList fills;
-    rc = fills.create(ctx, ctx->opt.pack_serial_fills ? sizes.size() : 0);
-    if (rc) return rc;
-    const auto t_pipe0 = std::chrono::steady_clock::now();
-    const bool tl = ctx->opt.timing >= 2;      // debugging aid: GPU-side timeline of every chunk
-    std::vector<cudaEvent_t> evs;
-    auto mark = [&](cudaStream_t s_) { if (tl) { cudaEvent_t e; cudaEventCreate(&e); cudaEventRecord(e, s_); evs.push_back(e); } };
-    long long p0 = 0;
-    for (int c = 0; c < (int)sizes.size(); p0 += sizes[c], ++c) {
-        cudaStream_t st = ctx->aux_stream[c % NS];
-        const long long cnt = sizes[c], p1 = p0 + cnt;
+    const long long n = args.n_pairs, stride = args.ops_stride_words;
+    ChunkSteps s;
+    s.inputs = [&](int, long long p0, long long cnt, cudaStream_t st) -> int {
+        const long long p1 = p0 + cnt;
         const size_t a0 = (size_t)h.off_a[p0], a1 = (p1 < n) ? (size_t)h.off_a[p1] : bytes_a;
         const size_t b0 = (size_t)h.off_b[p0], b1 = (p1 < n) ? (size_t)h.off_b[p1] : bytes_b;
-        mark(st);
         if (a1 > a0) PSA_CUDA_OK(ctx, cudaMemcpyAsync((void*)(args.bases_a + a0), h.bases_a + a0, a1 - a0, cudaMemcpyHostToDevice, st));
         if (b1 > b0) PSA_CUDA_OK(ctx, cudaMemcpyAsync((void*)(args.bases_b + b0), h.bases_b + b0, b1 - b0, cudaMemcpyHostToDevice, st));
         PSA_CUDA_OK(ctx, cudaMemcpyAsync((void*)(args.off_a + p0), h.off_a + p0, cnt * 8, cudaMemcpyHostToDevice, st));
         PSA_CUDA_OK(ctx, cudaMemcpyAsync((void*)(args.off_b + p0), h.off_b + p0, cnt * 8, cudaMemcpyHostToDevice, st));
         PSA_CUDA_OK(ctx, cudaMemcpyAsync((void*)(args.len_a + p0), h.len_a + p0, cnt * 4, cudaMemcpyHostToDevice, st));
         PSA_CUDA_OK(ctx, cudaMemcpyAsync((void*)(args.len_b + p0), h.len_b + p0, cnt * 4, cudaMemcpyHostToDevice, st));
-        mark(st);
-        rc = pack_chunk(ctx, args, p0, cnt, max_m, max_n, mode, traceback, sh, C, flags, rr[c % NS], slot_words, st,
-                        c < 4096 ? counters + c : nullptr, perms[c % NS], c > 0 ? fills.at(c - 1) : nullptr, fills.at(c));
-        if (rc) return rc;
-        mark(st);
+        return PSA_OK;
+    };
+    s.outputs = [&](int, long long p0, long long cnt, cudaStream_t st) -> int {
         PSA_CUDA_OK(ctx, cudaMemcpyAsync(h.items + p0, args.items + p0, cnt * sizeof(psa_batch_item), cudaMemcpyDeviceToHost, st));
         if (traceback)
-            PSA_CUDA_OK(ctx, cudaMemcpyAsync(h.ops + p0 * args.ops_stride_words, args.ops + p0 * args.ops_stride_words,
-                                             cnt * args.ops_stride_words * 4, cudaMemcpyDeviceToHost, st));
-        mark(st);
-    }
-    const auto t_enq = std::chrono::steady_clock::now();
-    for (int k = 0; k < NS; ++k) PSA_CUDA_OK(ctx, cudaStreamSynchronize(ctx->aux_stream[k]));
-    if (tl) {
-        for (size_t k = 0; k + 3 < evs.size(); k += 4) {
-            float a, b, c2, d;
-            cudaEventElapsedTime(&a, evs[0], evs[k]); cudaEventElapsedTime(&b, evs[0], evs[k + 1]);
-            cudaEventElapsedTime(&c2, evs[0], evs[k + 2]); cudaEventElapsedTime(&d, evs[0], evs[k + 3]);
-            fprintf(stderr, "  chunk %2d: h2d %.3f-%.3f  kernels -%.3f  d2h -%.3f\n", (int)(k / 4), a, b, c2, d);
-        }
-        for (auto e : evs) cudaEventDestroy(e);
-    }
-    if (ctx->opt.timing)
-        fprintf(stderr, "psa_pack_pipeline: %d chunks enqueued in %.3f ms, drained %.3f ms later\n", (int)sizes.size(),
-                std::chrono::duration<double, std::milli>(t_enq - t_pipe0).count(),
-                std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_enq).count());
-    return PSA_OK;
+            PSA_CUDA_OK(ctx, cudaMemcpyAsync(h.ops + p0 * stride, args.ops + p0 * stride, cnt * stride * 4, cudaMemcpyDeviceToHost, st));
+        return PSA_OK;
+    };
+    return pack_pipeline(ctx, args, max_m, max_n, mode, traceback, s);
 }
 
 // ---- 2-bit packed fixed-stride batches (psa_align_batch_packed) ------------------------------
@@ -1155,18 +1196,13 @@ __global__ void __launch_bounds__(256) psa_compact_items_kernel(const psa_batch_
     const long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (k >= n) return;
     const psa_batch_item it = in[k];
-    psa_packed_item o;
-    o.score = it.score;
-    o.end_i = (uint16_t)it.end_i; o.end_j = (uint16_t)it.end_j;
-    o.start_i = (uint16_t)it.start_i; o.start_j = (uint16_t)it.start_j;
-    o.aln_len = (uint16_t)it.aln_len; o.end_state = (uint16_t)it.end_state;
-    out[k] = o;
+    out[k] = packed_item(it);
 }
 
 // PSA_OPS_COMPACT: the op words of a chunk, back to back in pair order (pair k uses ceil(aln_len/16) words), packed on
 // the device so that only the words that carry ops cross PCIe (a 150 bp read pair needs 6 - 11 of its 20-word stride).
 // Two launches per chunk, one more than the fixed-stride path:
-//   psa_compact_items_scan_kernel: the 40 -> 16 byte records (as psa_compact_items_kernel) + per-CTA exclusive scan of
+//   psa_compact_items_scan_kernel: the 40 -> 16 byte records (packed_item) + per-CTA exclusive scan of
 //                                  the word counts -> offs[k] (CTA-local) and sums[cta]
 //   psa_ops_pack_kernel:           every CTA adds up the sums of the scan blocks before its pairs (at most 128) and the
 //                                  chunk's base (= end of the previous chunk, chained through `bases`), then one warp
@@ -1186,12 +1222,7 @@ __global__ void __launch_bounds__(SCAN_CT) psa_compact_items_scan_kernel(const p
         unsigned v = 0u;
         if (k < n) {
             const psa_batch_item it = in[k];
-            psa_packed_item o;
-            o.score = it.score;
-            o.end_i = (uint16_t)it.end_i; o.end_j = (uint16_t)it.end_j;
-            o.start_i = (uint16_t)it.start_i; o.start_j = (uint16_t)it.start_j;
-            o.aln_len = (uint16_t)it.aln_len; o.end_state = (uint16_t)it.end_state;
-            out[k] = o;
+            out[k] = packed_item(it);
             v = (unsigned)((it.aln_len + 15) >> 4);
         }
         unsigned x = v;                                     // inclusive scan inside the warp
@@ -1261,34 +1292,13 @@ __global__ void __launch_bounds__(SCAN_CT) psa_ops_pack_kernel(const psa_packed_
 }
 }  // namespace
 
-// Chunked copy/compute pipeline like psa_pack_pipeline, for 2-bit input: per chunk H2D of the two packed read
-// arrays (fixed stride: one contiguous range each, no offsets or lengths), fill + traceback, 40 -> 16 byte result
-// records, D2H of records and op words.  `args` = device mirror (a2/b2/items/ops device pointers).
+// 2-bit input (psa_align_batch_packed): per chunk H2D of the two packed read arrays (fixed stride: one contiguous range
+// each, no offsets or lengths), fill + traceback, 40 -> 16 byte result records, D2H of records and op words.  `args` =
+// device mirror (a2/b2/items/ops device pointers).
 int psa_pack_pipeline_packed(psa_ctx* ctx, const psa_batch_args& args, const uint32_t* h_a2, const uint32_t* h_b2,
                              psa_packed_item* d_items16, psa_packed_item* h_items16, uint32_t* h_ops, int mode, bool traceback,
-                             bool compact, uint8_t* d_compact /* scan scratch | bases | (staging buffer) */, uint64_t* total_words) {
-    constexpr int NS = 4;
-    const int max_m = args.fixed_m, max_n = args.fixed_n;
-    Shape sh; PackConsts C; uint8_t* flags; uint32_t* rr[NS]; long long slot_words; int* counters; int* perms[NS];
-    int rc = pack_plan(ctx, args, max_m, max_n, mode, traceback, sh, C, &flags, rr, NS, &slot_words, &counters, perms);
-    if (rc) return rc;
-    rc = psa_ensure_aux(ctx);
-    if (rc) return rc;
-    const int ns_used = std::max(2, std::min(NS, ctx->opt.pack_streams));
-    const long long chunk = ctx->opt.pack_chunk, n = args.n_pairs;
-    std::vector<long long> sizes;
-    {
-        const long long ramp[3] = {chunk / 8, chunk / 4, chunk / 2};
-        const long long ramp_sum = ramp[0] + ramp[1] + ramp[2];
-        if (n >= 2 * ramp_sum + chunk && chunk >= 8192 && ctx->opt.pack_ramp) {
-            for (int k = 0; k < 3; ++k) sizes.push_back(ramp[k]);
-            long long mid = n - 2 * ramp_sum;
-            while (mid > 0) { const long long t = std::min(chunk, mid); sizes.push_back(t); mid -= t; }
-            for (int k = 2; k >= 0; --k) sizes.push_back(ramp[k]);
-        } else {
-            for (long long p = 0; p < n; p += chunk) sizes.push_back(std::min(chunk, n - p));
-        }
-    }
+                             bool compact, uint8_t* d_compact /* scan scratch | bases | (staging buffer) */) {
+    const long long stride = args.ops_stride_words;
     // compact ops: the GPU packs each chunk's words back to back -- straight into the caller's buffer when that is
     // page-locked (zero-copy, whole 128-byte lines), else into a device buffer that is copied out once at the end
     compact = compact && traceback;
@@ -1298,14 +1308,17 @@ int psa_pack_pipeline_packed(psa_ctx* ctx, const psa_batch_args& args, const uin
     bool zero_copy = false;
     unsigned long long* h_bases = nullptr;
     unsigned long long* dh_bases = nullptr;
-    EventList chain, fills;
-    rc = fills.create(ctx, ctx->opt.pack_serial_fills ? sizes.size() : 0);
-    if (rc) return rc;
-    const size_t pack_smem = (size_t)(SCAN_CT / 32) * 32 * args.ops_stride_words * 4;
-    if (compact) {
-        if (sizes.size() + 1 > 4096) return psa_fail(ctx, PSA_ERR_RANGE, "compact ops: too many chunks");
+    size_t n_chunks = 0;
+    EventList chain;
+    const size_t pack_smem = (size_t)(SCAN_CT / 32) * 32 * stride * 4;
+    ChunkSteps s;
+    s.post = compact;
+    s.begin = [&](size_t nc) -> int {
+        n_chunks = nc;
+        if (!compact) return PSA_OK;
+        if (nc + 1 > 4096) return psa_fail(ctx, PSA_ERR_RANGE, "compact ops: too many chunks");
         if (pack_smem > 48 * 1024) return psa_fail(ctx, PSA_ERR_RANGE, "compact ops: ops_stride_words too large");
-        const size_t n_up = ((size_t)n + 255) / 256 * 256;
+        const size_t n_up = ((size_t)args.n_pairs + 255) / 256 * 256;
         d_offs = (unsigned*)d_compact;
         d_sums = (unsigned*)(d_compact + n_up * 4);                              // [chunks][128] scan-block sums
         d_bases = (unsigned long long*)(d_compact + n_up * 4 + 4096 * 128 * 4);
@@ -1324,30 +1337,16 @@ int psa_pack_pipeline_packed(psa_ctx* ctx, const psa_batch_args& args, const uin
         h_bases[0] = 0;
         PSA_CUDA_OK(ctx, cudaHostGetDevicePointer((void**)&dh_bases, ctx->h_pinned, 0));    // the GPU's view of the mirror
         PSA_CUDA_OK(ctx, cudaMemsetAsync(d_bases, 0, 8, ctx->post_stream));
-        rc = chain.create(ctx, sizes.size());
-        if (rc) return rc;
-    }
-    const bool tl = ctx->opt.timing >= 2;      // debugging aid: GPU-side timeline of every chunk
-    const auto t_host0 = std::chrono::steady_clock::now();
-    auto host_ms = [&]() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_host0).count(); };
-    std::vector<cudaEvent_t> evs;
-    auto mark = [&](cudaStream_t s_) { if (tl) { cudaEvent_t e; cudaEventCreate(&e); cudaEventRecord(e, s_); evs.push_back(e); } };
-    long long p0 = 0;
-    for (int c = 0; c < (int)sizes.size(); p0 += sizes[c], ++c) {
-        const int slot = c % ns_used;
-        cudaStream_t st = ctx->aux_stream[slot];
-        const long long cnt = sizes[c];
-        mark(st);
+        return chain.create(ctx, nc);
+    };
+    s.inputs = [&](int, long long p0, long long cnt, cudaStream_t st) -> int {
         PSA_CUDA_OK(ctx, cudaMemcpyAsync((void*)(args.a2 + p0 * args.wa), h_a2 + p0 * args.wa, (size_t)cnt * args.wa * 4, cudaMemcpyHostToDevice, st));
         PSA_CUDA_OK(ctx, cudaMemcpyAsync((void*)(args.b2 + p0 * args.wb), h_b2 + p0 * args.wb, (size_t)cnt * args.wb * 4, cudaMemcpyHostToDevice, st));
-        mark(st);
-        rc = pack_chunk(ctx, args, p0, cnt, max_m, max_n, mode, traceback, sh, C, flags, rr[slot], slot_words, st, nullptr, perms[slot],
-                        c > 0 ? fills.at(c - 1) : nullptr, fills.at(c));
-        if (rc) return rc;
-        mark(st);
+        return PSA_OK;
+    };
+    s.records = [&](int c, long long p0, long long cnt, cudaStream_t st) -> int {
         const int n_cta = (int)((cnt + SCAN_T - 1) / SCAN_T);
-        const int probe = ctx->opt.pack_compact_probe;
-        if (compact && probe < 2) {
+        if (compact) {
             if (n_cta > 128) return psa_fail(ctx, PSA_ERR_RANGE, "compact ops: chunk larger than 131 072 pairs");
             psa_compact_items_scan_kernel<<<n_cta, SCAN_CT, 0, st>>>(args.items + p0, d_items16 + p0, (int)cnt, d_offs + p0, d_sums + (size_t)c * 128);
         } else {
@@ -1355,41 +1354,27 @@ int psa_pack_pipeline_packed(psa_ctx* ctx, const psa_batch_args& args, const uin
         }
         PSA_CUDA_OK(ctx, cudaGetLastError());
         ctx->launches += 1;
-        if (compact && probe < 1) {
-            // The packing runs on a stream of its own, chunk after chunk (a chunk's base is the end of the previous one):
-            // chained inside the fill streams it made every later fill wait for the walks of ALL earlier chunks.
-            PSA_CUDA_OK(ctx, cudaEventRecord(chain.ev[c], st));
-            PSA_CUDA_OK(ctx, cudaStreamWaitEvent(ctx->post_stream, chain.ev[c], 0));
-            psa_ops_pack_kernel<<<(int)std::min<long long>((cnt + SCAN_CT - 1) / SCAN_CT, PACK_CTAS), SCAN_CT, pack_smem, ctx->post_stream>>>(
-                d_items16 + p0, args.ops + p0 * args.ops_stride_words, args.ops_stride_words, (int)cnt, d_offs + p0,
-                d_sums + (size_t)c * 128, n_cta, d_bases, dh_bases, c, cdst);
-            PSA_CUDA_OK(ctx, cudaGetLastError());
-            ctx->launches += 1;
-        }
-        mark(st);
+        if (!compact) return PSA_OK;
+        // The packing runs on a stream of its own, chunk after chunk (a chunk's base is the end of the previous one):
+        // chained inside the fill streams it made every later fill wait for the walks of ALL earlier chunks.
+        PSA_CUDA_OK(ctx, cudaEventRecord(chain.ev[c], st));
+        PSA_CUDA_OK(ctx, cudaStreamWaitEvent(ctx->post_stream, chain.ev[c], 0));
+        psa_ops_pack_kernel<<<(int)std::min<long long>((cnt + SCAN_CT - 1) / SCAN_CT, PACK_CTAS), SCAN_CT, pack_smem, ctx->post_stream>>>(
+            d_items16 + p0, args.ops + p0 * stride, stride, (int)cnt, d_offs + p0, d_sums + (size_t)c * 128, n_cta, d_bases,
+            dh_bases, c, cdst);
+        PSA_CUDA_OK(ctx, cudaGetLastError());
+        ctx->launches += 1;
+        return PSA_OK;
+    };
+    s.outputs = [&](int, long long p0, long long cnt, cudaStream_t st) -> int {
         PSA_CUDA_OK(ctx, cudaMemcpyAsync(h_items16 + p0, d_items16 + p0, (size_t)cnt * sizeof(psa_packed_item), cudaMemcpyDeviceToHost, st));
         if (traceback && !compact)
-            PSA_CUDA_OK(ctx, cudaMemcpyAsync(h_ops + p0 * args.ops_stride_words, args.ops + p0 * args.ops_stride_words,
-                                             (size_t)cnt * args.ops_stride_words * 4, cudaMemcpyDeviceToHost, st));
-        mark(st);
-    }
-    const double t_enq = host_ms();
-    for (int k = 0; k < NS; ++k) PSA_CUDA_OK(ctx, cudaStreamSynchronize(ctx->aux_stream[k]));
-    if (compact) {
-        PSA_CUDA_OK(ctx, cudaStreamSynchronize(ctx->post_stream));
-        const unsigned long long total = h_bases[sizes.size()];
-        if (!zero_copy && total) PSA_CUDA_OK(ctx, cudaMemcpy(h_ops, d_stage, (size_t)total * 4, cudaMemcpyDeviceToHost));
-        if (total_words) *total_words = total;
-    }
-    if (tl) {
-        for (size_t k = 0; k + 4 < evs.size(); k += 5) {
-            float t[5];
-            for (int q = 0; q < 5; ++q) cudaEventElapsedTime(&t[q], evs[0], evs[k + q]);
-            fprintf(stderr, "  chunk %2d (%6lld pairs): h2d %.3f-%.3f  fill+walk -%.3f  records/pack -%.3f  d2h -%.3f%s\n", (int)(k / 5),
-                    sizes[k / 5], t[0], t[1], t[2], t[3], t[4], compact ? "" : " (ops included)");
-        }
-        for (auto e : evs) cudaEventDestroy(e);
-        fprintf(stderr, "  host: enqueued at %.3f ms, all streams idle %.3f ms\n", t_enq, host_ms());
-    }
+            PSA_CUDA_OK(ctx, cudaMemcpyAsync(h_ops + p0 * stride, args.ops + p0 * stride, (size_t)cnt * stride * 4, cudaMemcpyDeviceToHost, st));
+        return PSA_OK;
+    };
+    const int rc = pack_pipeline(ctx, args, args.fixed_m, args.fixed_n, mode, traceback, s);
+    if (rc || !compact) return rc;
+    const unsigned long long total = h_bases[n_chunks];
+    if (!zero_copy && total) PSA_CUDA_OK(ctx, cudaMemcpy(h_ops, d_stage, (size_t)total * 4, cudaMemcpyDeviceToHost));
     return PSA_OK;
 }

@@ -55,6 +55,17 @@ __device__ __forceinline__ psa_batch_item packed_corner_item(const uint32_t* c3,
                        (int)((c3[2] >> sh) & 0xffffu) - bias, m, n, 0, -1);
 }
 
+// The 16-byte record of psa_align_batch_packed: score, cells, length and end state of the 40-byte record, the
+// coordinates and length narrowed to 16 bits (its reads are at most 512 x 256).
+__device__ __forceinline__ psa_packed_item packed_item(const psa_batch_item& it) {
+    psa_packed_item o;
+    o.score = it.score;
+    o.end_i = (uint16_t)it.end_i; o.end_j = (uint16_t)it.end_j;
+    o.start_i = (uint16_t)it.start_i; o.start_j = (uint16_t)it.start_j;
+    o.aln_len = (uint16_t)it.aln_len; o.end_state = (uint16_t)it.end_state;
+    return o;
+}
+
 // Border values by start type st (cpp:212-227, :259-292): H = max(T1,T2,T3) of the border cell; on row 0 only T2
 // can be finite, on column 0 only T3, besides the (0,0) cell.  -1 is the live case; -2 / -3 continue an open gap
 // along row 0 / column 0 (no h on that border); 1, 2, 3 force the first state, which leaves only T1[0][0] (1),

@@ -381,10 +381,12 @@ def test_packed_2bit_batch_equals_oracle_and_byte_api(ctx, mode, shape):
     c.close()
 
 
-@pytest.mark.parametrize("pinned", [False, True])
-def test_packed_2bit_compact_ops(ctx, pinned):
+@pytest.mark.parametrize("pinned, serial", [pytest.param(False, 0, id="False"), pytest.param(True, 0, id="True"),
+                                            pytest.param(True, 1, id="True-serial_fills")])
+def test_packed_2bit_compact_ops(ctx, pinned, serial):
     """PSA_OPS_COMPACT: op words back to back in pair order (page-locked and pageable
-    destination) hold exactly the words of the fixed-stride layout; several chunks, ramps, empty alignments."""
+    destination) hold exactly the words of the fixed-stride layout; several chunks, ramps, empty alignments;
+    fills of consecutive chunks concurrent or serialised (pack_serial_fills)."""
     import torch
     from cse305_parallel_sequence_alignment_b200 import synth
     npairs, L = 5000, 150
@@ -393,6 +395,7 @@ def test_packed_2bit_compact_ops(ctx, pinned):
     a2, b2 = psa.pack_reads_2bit(A), psa.pack_reads_2bit(B)
     c = psa.Context(0)
     c.set_option("pack_chunk", 1024)
+    c.set_option("pack_serial_fills", serial)
     items, ops = c.align_batch_packed(a2, b2, L, L, psa.LOCAL, 1, 2, traceback=True)
     stride = ops.shape[1]
     if pinned:

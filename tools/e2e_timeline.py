@@ -23,23 +23,19 @@ stride = (2 * L + 15) // 16 + 1
 items = pin(np.zeros(n * 4, dtype=np.int32)).view(psa.capi.PACKED_ITEM_DTYPE)
 ops = pin(np.zeros(n * stride, dtype=np.int32)).view(np.uint32).reshape(n, stride)
 ctx = psa.Context(0)
-probes = [int(x) for x in os.environ.get("PROBES", "0").split(",")]
 for rnd in range(2):
-    for serial, compact, probe, ns in [(0, c_, 0, ns_) for ns_ in (4, 3, 2) for c_ in (False, True)] + [(0, True, p_, 4) for p_ in probes if p_]:
-        if True:
-            ctx.set_option("pack_streams", ns)
-            ctx.set_option("pack_serial_fills", serial)
-            ctx.set_option("pack_compact_probe", probe)
-            ts = []
-            for rep in range(reps + 2):
-                t0 = time.perf_counter()
-                ctx.align_batch_packed(a2, b2, L, L, psa.LOCAL, 1, 2, True, items=items, ops=ops, compact=compact)
-                if rep >= 2:
-                    ts.append((time.perf_counter() - t0) * 1e3)
-            print(json.dumps({"serial_fills": serial, "compact": compact, "probe": probe, "streams": ns, "round": rnd, "median_ms": float(np.median(ts)), "min_ms": float(min(ts))}), flush=True)
-            if rnd == 1 and os.environ.get("TIMELINE") == "1":
-                print(f"---- serial_fills={serial} compact={compact} probe={probe} ----", file=sys.stderr, flush=True)
-                ctx.set_option("timing", 2)
-                ctx.align_batch_packed(a2, b2, L, L, psa.LOCAL, 1, 2, True, items=items, ops=ops, compact=compact)
-                ctx.set_option("timing", 0)
+    for serial, compact in [(s_, c_) for s_ in (0, 1) for c_ in (False, True)]:
+        ctx.set_option("pack_serial_fills", serial)
+        ts = []
+        for rep in range(reps + 2):
+            t0 = time.perf_counter()
+            ctx.align_batch_packed(a2, b2, L, L, psa.LOCAL, 1, 2, True, items=items, ops=ops, compact=compact)
+            if rep >= 2:
+                ts.append((time.perf_counter() - t0) * 1e3)
+        print(json.dumps({"serial_fills": serial, "compact": compact, "round": rnd, "median_ms": float(np.median(ts)), "min_ms": float(min(ts))}), flush=True)
+        if rnd == 1 and os.environ.get("TIMELINE") == "1":
+            print(f"---- serial_fills={serial} compact={compact} ----", file=sys.stderr, flush=True)
+            ctx.set_option("timing", 2)
+            ctx.align_batch_packed(a2, b2, L, L, psa.LOCAL, 1, 2, True, items=items, ops=ops, compact=compact)
+            ctx.set_option("timing", 0)
 ctx.close()
