@@ -10,7 +10,7 @@
 
 // In-kernel stand-in for the reference's -infinity (subproblem_alignment.cpp:214-223).  Far
 // enough from INT32_MIN that a few "- g - h" never wrap, far enough from real scores that it
-// never wins a max.  Converted to PSA_NEG_INF at the API boundary.
+// never wins a max.  Converted to PSA_NEG_INF at the API boundary (out_value, psa_result.cuh).
 #define PSA_KNEG (-(1 << 29))
 
 // Per-context tuning and measurement options (psa_internal.h: psa_ctx_set_option).  The shipped
