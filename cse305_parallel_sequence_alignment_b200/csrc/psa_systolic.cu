@@ -136,7 +136,7 @@ __device__ __forceinline__ void st_relaxed_2xu64(unsigned long long* p, unsigned
 
 // RB rows x KC columns per lane and step: the per-step overhead (shuffles, boundary hand-over, loop control) is shared by
 // RB*KC cells and the RB + KC - 1 anti-diagonals of the block give a lone warp the instruction-level parallelism a
-// one-row step lacks.  Lane t works on row block s - t at step s; row counts are padded to a multiple of RB
+// one-row step lacks.  Lane t works on row block s - t at step s; row counts are padded to a multiple of 4
 // (padding rows never reach the result: their keys are masked, the corner is captured on row m).
 template <int MODE, int KC, int RB>
 __global__ void __launch_bounds__(SWPB * 32) psa_systolic_kernel(SysJob J) {
@@ -149,7 +149,12 @@ __global__ void __launch_bounds__(SWPB * 32) psa_systolic_kernel(SysJob J) {
     const int sidx = blockIdx.x * SWPB + wib;
     if (sidx >= J.nstrips) return;
     const int m = J.m, g = J.g, h = J.h, go = g + h, ng = -g, ngo = -go;
-    const int mp = (m + RB - 1) / RB * RB;                // padded rows
+    // Padded rows: a multiple of 4 for every RB, the same count the ring totals advance by below.  Each ring row of
+    // this launch must be written: a slot a lap skips still holds the tag of two laps back, which is the tag the next
+    // lap waits for, so the consumer takes a stale entry as valid if it reads the slot before the producer rewrites it
+    // (with rows padded to RB only, a 1-row launch at m = 5 skipped rows 5-7, and a later call on the same context
+    // whose rows reached those slots one lap on could return a wrong corner).
+    const int mp = (m + 3) & ~3;
     const int nblk = mp / RB;
     const int c0 = sidx * W + lane * KC;                  // panel-local 0-based first column of this lane
     const int cg = J.col_begin + c0;                      // global index of the column left of it
@@ -316,7 +321,7 @@ __global__ void __launch_bounds__(SWPB * 32) psa_systolic_kernel(SysJob J) {
         for (; st < steps; ++st) step(st, std::false_type{});
     }
     // ---- totals for the next launch that uses these boundaries (padded to 4 rows so that entry pairs stay aligned) ----
-    const unsigned adv = (unsigned)((m + 3) & ~3);
+    const unsigned adv = (unsigned)mp;
     if (use_in && lane == 0) { st_relaxed_u32(bin.consumed_pub, cons_base + adv, in_sys); *bin.cons_total = cons_base + adv; }
     if (use_out && lane == 31) *bout.prod_total = prod_base + adv;
 
@@ -391,7 +396,9 @@ int psa_systolic_capacity(psa_ctx* ctx) {
 // a fresh or regrown allocation starts from all-zero, which is a consistent state).
 static int ensure_sys(psa_ctx* ctx, int strips, size_t self_rows, SysLayout* L) {
     // capacities are powers of two so that the cumulative row numbering survives the wrap of its 32-bit counters
-    size_t pow2 = 1;
+    // and at least 32: a launch writes its rows padded to 4, and the producer waits while they exceed the capacity (the
+    // consumer of a self boundary is the next panel's launch, so at m = 1 or 2 a 1- or 2-row buffer never drained)
+    size_t pow2 = 32;
     while (pow2 < self_rows) pow2 <<= 1;
     self_rows = pow2;
     const bool fits = ctx->d_sys != nullptr && strips <= ctx->sys_strips && self_rows <= ctx->sys_self_rows;
