@@ -114,6 +114,12 @@ def load_library() -> C.CDLL:
     lib.psa_align_batch_device.restype = C.c_int
     lib.psa_align_batch_device.argtypes = [vp, vp, vp, vp, vp, vp, vp, C.c_size_t, C.c_int, C.c_int, C.c_int,
                                            C.c_int, C.c_int, C.c_uint, vp, vp, C.c_size_t, vp]
+    lib.psa_align_batch_banded.restype = C.c_int
+    lib.psa_align_batch_banded.argtypes = [vp, vp, vp, vp, vp, vp, vp, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int,
+                                           C.c_int, C.c_int, C.c_int, C.c_uint, vp, vp, C.c_size_t]
+    lib.psa_align_batch_banded_device.restype = C.c_int
+    lib.psa_align_batch_banded_device.argtypes = [vp, vp, vp, vp, vp, vp, vp, C.c_size_t, C.c_int, C.c_int, C.c_int,
+                                                  C.c_int, C.c_int, C.c_int, C.c_uint, vp, vp, C.c_size_t, vp]
     lib.psa_align_long_device.restype = C.c_int
     lib.psa_align_long_device.argtypes = [vp, vp, vp, C.c_size_t, C.c_size_t, C.c_int, C.c_int, C.c_int, C.c_uint,
                                           vp, vp, C.c_size_t, vp]
@@ -145,7 +151,7 @@ def load_library() -> C.CDLL:
 
 
 EXPORTS = ["psa_ctx_create", "psa_ctx_destroy", "psa_last_error", "psa_launch_count", "psa_align_pair", "psa_align_pair_typed", "psa_align_partition", "psa_align_long_partitioned", "psa_similarity_batch", "psa_similarity_batch_device",
-           "psa_result_free", "psa_align_batch", "psa_align_batch_device", "psa_pack_bases", "psa_pack_reads", "psa_align_batch_packed", "psa_align_long_device", "psa_xbuf_bytes", "psa_xbuf_create", "psa_xbuf_open", "psa_xbuf_close",
+           "psa_result_free", "psa_align_batch", "psa_align_batch_device", "psa_align_batch_banded", "psa_align_batch_banded_device", "psa_pack_bases", "psa_pack_reads", "psa_align_batch_packed", "psa_align_long_device", "psa_xbuf_bytes", "psa_xbuf_create", "psa_xbuf_open", "psa_xbuf_close",
            "psa_xbuf_destroy", "psa_long_panel_strips", "psa_long_strip_columns", "psa_align_long_cyclic_device", "psa_ops_unpack", "psa_render_rows",
            "psa_peak_int_ops"]
 
@@ -383,6 +389,44 @@ class Context:
         self._check(self._lib.psa_align_batch_device(
             self._h, d_bases_a, d_off_a, d_len_a, d_bases_b, d_off_b, d_len_b, n_pairs, max_len_a, max_len_b,
             mode, g, h, flags, d_items, d_ops or None, ops_stride_words, stream or None))
+
+    def align_batch_banded(self, bases_a: np.ndarray, off_a: np.ndarray, len_a: np.ndarray, bases_b: np.ndarray,
+                           off_b: np.ndarray, len_b: np.ndarray, band: int, mode: int = GLOBAL, g: int = 1, h: int = 2,
+                           traceback: bool = True, ops: Optional[np.ndarray] = None, flags: Optional[int] = None):
+        """psa_align_batch_banded: align_batch inside the diagonal band of half-width `band`.  Returns (items, ops words
+        [n_pairs, stride] or None)."""
+        n = len(len_a)
+        bases_a = np.ascontiguousarray(bases_a, dtype=np.uint8)
+        bases_b = np.ascontiguousarray(bases_b, dtype=np.uint8)
+        off_a = np.ascontiguousarray(off_a, dtype=np.int64)
+        off_b = np.ascontiguousarray(off_b, dtype=np.int64)
+        len_a = np.ascontiguousarray(len_a, dtype=np.int32)
+        len_b = np.ascontiguousarray(len_b, dtype=np.int32)
+        items = np.zeros(n, dtype=ITEM_DTYPE)
+        stride = 0
+        if traceback:
+            if ops is None:
+                stride = (int(len_a.max(initial=0)) + int(len_b.max(initial=0)) + 15) // 16 + 1
+                ops = np.zeros((n, stride), dtype=np.uint32)
+            stride = ops.shape[1]
+        if flags is None:
+            flags = WANT_SCORE | (WANT_TRACEBACK if traceback else 0)
+        self._check(self._lib.psa_align_batch_banded(
+            self._h, bases_a.ctypes.data, off_a.ctypes.data, len_a.ctypes.data, bases_b.ctypes.data,
+            off_b.ctypes.data, len_b.ctypes.data, n, bases_a.size, bases_b.size, mode, g, h, band, flags,
+            items.ctypes.data, ops.ctypes.data if traceback else None, stride))
+        return items, (ops if traceback else None)
+
+    def align_batch_banded_device(self, d_bases_a: int, d_off_a: int, d_len_a: int, d_bases_b: int, d_off_b: int,
+                                  d_len_b: int, n_pairs: int, max_len_a: int, max_len_b: int, band: int, d_items: int,
+                                  d_ops: int = 0, ops_stride_words: int = 0, mode: int = GLOBAL, g: int = 1, h: int = 2,
+                                  traceback: bool = True, stream: int = 0, flags: Optional[int] = None):
+        """Device-resident banded batch call (psa_align_batch_banded_device): raw device pointers / cudaStream_t."""
+        if flags is None:
+            flags = WANT_SCORE | (WANT_TRACEBACK if traceback else 0)
+        self._check(self._lib.psa_align_batch_banded_device(
+            self._h, d_bases_a, d_off_a, d_len_a, d_bases_b, d_off_b, d_len_b, n_pairs, max_len_a, max_len_b,
+            mode, g, h, band, flags, d_items, d_ops or None, ops_stride_words, stream or None))
 
     def align_long_device(self, d_a: int, d_b: int, m: int, n: int, d_item: int, d_ops: int = 0, ops_words: int = 0,
                           mode: int = GLOBAL, g: int = 1, h: int = 2, traceback: bool = False, stream: int = 0):

@@ -205,10 +205,12 @@ int psa_align_batch_device(psa_ctx* ctx, const uint8_t* d_bases_a, const int64_t
 constexpr int kLongTbBatchMin = 16;
 
 // Host-buffer batch with an optional border variant per call or per pair; psa_align_batch is the -1/-1 case.
+// band >= 0: psa_align_batch_banded (every pair on the banded kernels).
 static int align_batch_host(psa_ctx* ctx, const uint8_t* bases_a, const int64_t* off_a, const int32_t* len_a,
                             const uint8_t* bases_b, const int64_t* off_b, const int32_t* len_b, size_t n_pairs,
                             size_t bytes_a, size_t bytes_b, int mode, int g, int h, unsigned flags,
-                            psa_batch_item* items, uint32_t* ops, size_t ops_stride_words, const psa_piece_types& ty) {
+                            psa_batch_item* items, uint32_t* ops, size_t ops_stride_words, const psa_piece_types& ty,
+                            int band = -1) {
     if (!ctx) return PSA_ERR_ARG;
     if (n_pairs == 0) return PSA_OK;
     if (!off_a || !off_b || !len_a || !len_b || !items || (!bases_a && bytes_a) || (!bases_b && bytes_b))
@@ -292,7 +294,7 @@ static int align_batch_host(psa_ctx* ctx, const uint8_t* bases_a, const int64_t*
     }
     const bool typed = ty.any();
     // large DNA batches laid out back to back: chunked copy/compute pipeline on the four aux streams
-    if (!typed && contiguous && n_pairs > (size_t)ctx->opt.pack_chunk && psa_short_supported(max_m, max_n, tb) &&
+    if (band < 0 && !typed && contiguous && n_pairs > (size_t)ctx->opt.pack_chunk && psa_short_supported(max_m, max_n, tb) &&
         psa_pack_supported(max_m, max_n, mode, g, h) && ctx->opt.pack && ctx->opt.pipeline) {
         psa_batch_args host{bases_a, off_a, len_a, bases_b, off_b, len_b, (int64_t)n_pairs, g, h, items, ops,
                             (int64_t)ops_stride_words};
@@ -317,11 +319,14 @@ static int align_batch_host(psa_ctx* ctx, const uint8_t* bases_a, const int64_t*
     // long pairs with traceback: from kLongTbBatchMin pairs on, one warp per pair (checkpointed batch fill + batched walk)
     // unless one pair's checkpoints exceed the memory budget
     long long tb_chunk = 0;
-    if (!is_short && tb && n_pairs >= (size_t)kLongTbBatchMin) {
+    if (band < 0 && !is_short && tb && n_pairs >= (size_t)kLongTbBatchMin) {
         rc = psa_long_batch_tb_chunk(ctx, (long long)n_pairs, max_m, max_n, mode, &tb_chunk);
         if (rc) return rc;
     }
-    if (is_short || (!typed && !tb && n_pairs > 8) || tb_chunk > 0) {
+    if (band >= 0) {
+        rc = psa_launch_banded(ctx, args, max_m, max_n, mode, band, tb, st);
+        if (rc) return rc;
+    } else if (is_short || (!typed && !tb && n_pairs > 8) || tb_chunk > 0) {
         rc = dispatch_batch(ctx, args, max_m, max_n, mode, flags, st);
         if (rc) return rc;
     } else {
@@ -359,6 +364,45 @@ int psa_align_batch(psa_ctx* ctx, const uint8_t* bases_a, const int64_t* off_a, 
                     psa_batch_item* items, uint32_t* ops, size_t ops_stride_words) {
     return align_batch_host(ctx, bases_a, off_a, len_a, bases_b, off_b, len_b, n_pairs, bytes_a, bytes_b, mode, g, h, flags,
                             items, ops, ops_stride_words, psa_piece_types{});
+}
+
+int psa_align_batch_banded(psa_ctx* ctx, const uint8_t* bases_a, const int64_t* off_a, const int32_t* len_a,
+                           const uint8_t* bases_b, const int64_t* off_b, const int32_t* len_b, size_t n_pairs,
+                           size_t bytes_a, size_t bytes_b, int mode, int g, int h, int band, unsigned flags,
+                           psa_batch_item* items, uint32_t* ops, size_t ops_stride_words) {
+    if (!ctx) return PSA_ERR_ARG;
+    if (band < 0) return psa_fail(ctx, PSA_ERR_ARG, "band must be >= 0");
+    if (flags & ~(PSA_WANT_SCORE | PSA_WANT_TRACEBACK)) return psa_fail(ctx, PSA_ERR_ARG, "flags: PSA_WANT_SCORE and PSA_WANT_TRACEBACK only");
+    return align_batch_host(ctx, bases_a, off_a, len_a, bases_b, off_b, len_b, n_pairs, bytes_a, bytes_b, mode, g, h, flags,
+                            items, ops, ops_stride_words, psa_piece_types{}, band);
+}
+
+int psa_align_batch_banded_device(psa_ctx* ctx, const uint8_t* d_bases_a, const int64_t* d_off_a, const int32_t* d_len_a,
+                                  const uint8_t* d_bases_b, const int64_t* d_off_b, const int32_t* d_len_b, size_t n_pairs,
+                                  int max_len_a, int max_len_b, int mode, int g, int h, int band, unsigned flags,
+                                  psa_batch_item* d_items, uint32_t* d_ops, size_t ops_stride_words, void* cuda_stream) {
+    if (!ctx) return PSA_ERR_ARG;
+    if (band < 0) return psa_fail(ctx, PSA_ERR_ARG, "band must be >= 0");
+    if (flags & ~(PSA_WANT_SCORE | PSA_WANT_TRACEBACK)) return psa_fail(ctx, PSA_ERR_ARG, "flags: PSA_WANT_SCORE and PSA_WANT_TRACEBACK only");
+    if (n_pairs == 0) return PSA_OK;
+    if (!d_bases_a || !d_bases_b || !d_off_a || !d_off_b || !d_len_a || !d_len_b || !d_items)
+        return psa_fail(ctx, PSA_ERR_ARG, "null device pointer");
+    if (max_len_a < 0 || max_len_b < 0) return psa_fail(ctx, PSA_ERR_ARG, "negative length bound");
+    int rc = check_scoring(ctx, mode, g, h, max_len_a, max_len_b);
+    if (rc) return rc;
+    const bool tb = (flags & PSA_WANT_TRACEBACK) != 0;
+    if (tb && !d_ops) return psa_fail(ctx, PSA_ERR_ARG, "traceback requested without an ops buffer");
+    if (tb && ops_stride_words * 16 < (size_t)max_len_a + max_len_b)
+        return psa_fail(ctx, PSA_ERR_CAPACITY, "ops_stride_words < ceil((max m + max n)/16)");
+    PSA_CUDA_OK(ctx, cudaSetDevice(ctx->device));
+    psa_batch_args args{d_bases_a, d_off_a, d_len_a, d_bases_b, d_off_b, d_len_b, (int64_t)n_pairs, g, h,
+                        d_items, tb ? d_ops : nullptr, (int64_t)ops_stride_words};
+    cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : ctx->stream;
+    rc = psa_stream_enter(ctx, st);
+    if (rc) return rc;
+    rc = psa_launch_banded(ctx, args, max_len_a, max_len_b, mode, band, tb, st);
+    if (rc) return rc;
+    return psa_stream_leave(ctx, st);
 }
 
 int psa_align_long_device(psa_ctx* ctx, const uint8_t* d_a, const uint8_t* d_b, size_t m, size_t n, int mode, int g, int h,

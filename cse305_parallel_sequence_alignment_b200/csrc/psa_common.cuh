@@ -163,5 +163,8 @@ int psa_launch_long_batch_at(psa_ctx* ctx, const psa_batch_args& args, int max_m
 // psa_long_batch_tb_chunk: pairs per chunk for this batch shape (0: one checkpoint slot exceeds the memory budget).
 int psa_long_batch_tb_chunk(psa_ctx* ctx, long long n_pairs, int max_m, int max_n, int mode, long long* chunk);
 int psa_launch_long_batch_tb(psa_ctx* ctx, const psa_batch_args& args, int max_m, int max_n, int mode, cudaStream_t st);
+// Banded batch (psa_align_batch_banded): every pair on the banded tile kernels, one warp per pair (psa_long.cu).
+int psa_launch_banded(psa_ctx* ctx, const psa_batch_args& args, int max_m, int max_n, int mode, int band, bool traceback,
+                      cudaStream_t st);
 bool psa_pack_long_supported(int max_m, int max_n, int mode, int g, int h);
 int psa_launch_pack_long(psa_ctx* ctx, const psa_batch_args& args, int max_m, int max_n, int mode, cudaStream_t st);

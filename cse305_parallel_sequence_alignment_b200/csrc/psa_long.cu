@@ -503,6 +503,390 @@ __global__ void __launch_bounds__(WALK_WPB * 32) psa_long_batch_tb_walk_kernel(L
     if ((threadIdx.x & 31) == 0) Bt.P.items[p] = r;
 }
 
+// ---- banded batches (psa_align_batch_banded) -----------------------------------------------------------------------
+// Cell (i, j) is in the band iff |j - c(i)| <= bw, c(i) = floor(i*n/m): the line from (0,0) to (m,n).  Outside the band
+// H = T1 = 0 in local mode (the value of the local borders, DESIGN.md section 3), the sentinel in global mode; E = F =
+// sentinel in both.  Row block rb sweeps only strips s_lo(rb) .. s_hi(rb), the strips its band rows touch (both
+// non-decreasing in rb); everything it reads from outside that range -- the top of strips rb - 1 did not compute, the
+// left column of strip s_lo > 0, border cells beyond the band -- is out of band.  Tiles that a band edge cuts take the
+// masked sweeps (sweep_score / sweep with BANDED), tiles wholly inside the band the plain ones.
+struct Band {
+    int m, n, bw;
+    __device__ __forceinline__ int c(int i) const { return (int)((long long)i * n / m); }
+    __device__ __forceinline__ int lo(int i) const { return max(0, c(i) - bw); }
+    __device__ __forceinline__ int hi(int i) const { return (int)min((long long)n, (long long)c(i) + bw); }
+    // strips of width WW touched by rows i0+1 .. i0+nrows
+    __device__ __forceinline__ int s_lo(int i0, int WW) const { return (max(1, lo(i0 + 1)) - 1) / WW; }
+    __device__ __forceinline__ int s_hi(int i0, int nrows, int WW) const { return max(s_lo(i0, WW), (max(1, hi(i0 + nrows)) - 1) / WW); }
+    // every cell of rows i0+1 .. i0+nrows, columns s*WW+1 .. min(n, (s+1)*WW) is in the band
+    __device__ __forceinline__ bool inside(int i0, int nrows, int s, int WW) const {
+        return lo(i0 + nrows) <= s * WW + 1 && hi(i0 + 1) >= min(n, (s + 1) * WW);
+    }
+};
+
+template <int MODE>
+__device__ __forceinline__ constexpr int oob_H() { return MODE == PSA_LOCAL ? 0 : PSA_KNEG; }
+
+// Checkpoints of a banded traceback fill, per computed tile (rb, s) of the <128, 8> grid: the tile's bottom row (H, F
+// over its W columns) and its right column (H, E over its R rows).  Row block rb's tiles are records
+// tile_base[rb] .. tile_base[rb] + s_hi - s_lo, in strip order.
+constexpr int REC = 2 * W + 2 * R;     // ints per tile record
+struct BandCk {
+    Band B;
+    int* rec;
+    long long* tile_base;              // [NB]
+};
+
+struct BandSmem {
+    WarpSmem<R> w;
+    int lo[R], hi[R];                  // band of each row of the row block
+};
+
+// H and F of row i0 (the top boundary of row block rb) at column j.  prev: row block rb-1's strips p_lo .. p_hi, kept in
+// the recycled row J.hbufH / J.hbufF (score only) or in the records from rec_prev on (traceback).
+template <int MODE, int WW, bool TB>
+__device__ __forceinline__ void band_top(const LongJob& J, const Band& B, const int* rec_prev, int rb, int i0, int p_lo, int p_hi,
+                                         int j, int& H, int& F) {
+    F = PSA_KNEG;
+    if (rb == 0) { H = j <= B.hi(0) ? border_row0_H<MODE>(j, J.g, J.h) : oob_H<MODE>(); return; }
+    if (j == 0) { H = B.lo(i0) == 0 ? border_col0_H<MODE>(i0, J.g, J.h) : oob_H<MODE>(); return; }
+    const int sj = (j - 1) / WW;
+    if (sj < p_lo || sj > p_hi) { H = oob_H<MODE>(); return; }
+    if (TB) {
+        const int* rr = rec_prev + (long long)(sj - p_lo) * REC;
+        H = __ldcg(rr + (j - 1 - sj * WW)); F = __ldcg(rr + W + (j - 1 - sj * WW));
+    } else {
+        H = __ldcg(J.hbufH + j); F = __ldcg(J.hbufF + j);
+    }
+}
+
+// One row block of a banded pair, warp-collective.  Score only (TB = false): <128, 16> grid, TF-form sweeps, bottom row
+// into the recycled row.  Traceback fill (TB = true): <128, 8> grid, sweep<> without codes, every tile's bottom row and
+// right column into the records rec_cur (row block rb) -- rec_prev are row block rb-1's.
+template <int MODE, int KK, bool TB>
+__device__ void process_rowblock_banded(const LongJob& J, const Band& B, int rb, BandSmem& sm, Track& tr, int* rec_cur,
+                                        const int* rec_prev) {
+    constexpr int WW = 32 * KK;
+    static_assert(!TB || WW == W, "traceback checkpoints use the walk's tile grid");
+    const int lane = threadIdx.x & 31;
+    const int m = J.m, n = J.n, g = J.g, h = J.h;
+    const int i0 = rb * R, nrows = min(R, m - i0);
+    const int s_lo = B.s_lo(i0, WW), s_hi = B.s_hi(i0, nrows, WW);
+    const int p_lo = rb > 0 ? B.s_lo(i0 - R, WW) : 0, p_hi = rb > 0 ? B.s_hi(i0 - R, R, WW) : -1;
+    for (int r = lane; r < nrows; r += 32) {
+        const int i = i0 + 1 + r;
+        sm.w.sA[r] = J.a[i0 + r];
+        sm.lo[r] = B.lo(i); sm.hi[r] = B.hi(i);
+        sm.w.bH[0][r] = (s_lo == 0 && sm.lo[r] == 0) ? border_col0_H<MODE>(i, g, h) : oob_H<MODE>();
+        sm.w.bE[0][r] = PSA_KNEG;
+    }
+    int corner, dummy;
+    band_top<MODE, WW, TB>(J, B, rec_prev, rb, i0, p_lo, p_hi, s_lo * WW, corner, dummy);
+    __syncwarp();
+    int cur = 0;
+    int cap1 = PSA_KNEG, cap2 = PSA_KNEG, cap3 = PSA_KNEG;
+    bool captured = false;
+    for (int s = s_lo; s <= s_hi; ++s) {
+        const int c0 = s * WW + lane * KK;
+        const bool inside = B.inside(i0, nrows, s, WW);
+        int hlast;
+        if constexpr (TB) {
+            Cols<KK> cs;
+#pragma unroll
+            for (int k = 0; k < KK; ++k) {
+                const int j = c0 + k + 1;
+                cs.b[k] = (j <= n) ? (int)J.b[j - 1] : 256;
+                if (j <= n) band_top<MODE, WW, TB>(J, B, rec_prev, rb, i0, p_lo, p_hi, j, cs.H[k], cs.F[k]);
+                else { cs.H[k] = PSA_KNEG; cs.F[k] = PSA_KNEG; }
+            }
+            hlast = cs.H[KK - 1];
+            int hd = __shfl_up_sync(0xffffffffu, hlast, 1);
+            if (lane == 0) hd = corner;
+            Track tt{0, 0, 0};
+            int* rc = rec_cur + (long long)(s - s_lo) * REC;
+            if (inside) sweep<KK, MODE, false>(cs, hd, sm.w.bH[cur], sm.w.bE[cur], rc + 2 * W, rc + 2 * W + R, sm.w.sA, nrows, i0, c0,
+                                               m, n, g, h, nullptr, tt, cap1, cap2, cap3);
+            else sweep<KK, MODE, false, true>(cs, hd, sm.w.bH[cur], sm.w.bE[cur], rc + 2 * W, rc + 2 * W + R, sm.w.sA, nrows, i0, c0,
+                                              m, n, g, h, nullptr, tt, cap1, cap2, cap3, sm.lo, sm.hi);
+            if (MODE == PSA_LOCAL && tt.best > 0) {      // first cell of the tile's best, in row-major order, against the earlier tiles'
+                const bool better = tt.best > tr.best || (tt.best == tr.best && (tt.bi < tr.bi || (tt.bi == tr.bi && tt.bj < tr.bj)));
+                if (better) tr = tt;
+            }
+#pragma unroll
+            for (int k = 0; k < KK; ++k) { rc[lane * KK + k] = cs.H[k]; rc[W + lane * KK + k] = cs.F[k]; }
+            __syncwarp();
+            // the right column went straight to the record; the next tile's left boundary is read from there
+            for (int r = lane; r < nrows; r += 32) { sm.w.bH[cur ^ 1][r] = rc[2 * W + r]; sm.w.bE[cur ^ 1][r] = rc[2 * W + R + r]; }
+        } else {
+            ColsS<KK> cs;
+#pragma unroll
+            for (int k = 0; k < KK; ++k) {
+                const int j = c0 + k + 1;
+                cs.b[k] = (j <= n) ? (int)J.b[j - 1] : 256;
+                int H0 = oob_H<MODE>(), F0 = PSA_KNEG;
+                if (j <= n) band_top<MODE, WW, TB>(J, B, rec_prev, rb, i0, p_lo, p_hi, j, H0, F0);
+                cs.set_top(k, H0, F0, g + h);
+                cs.set_key_addend(k, j <= n, g + h);
+            }
+            hlast = cs.top_H(KK - 1, g + h);
+            int hd = __shfl_up_sync(0xffffffffu, hlast, 1);
+            if (lane == 0) hd = corner;
+            int bestkey = 0, besti = 0;
+            if (inside) sweep_score<KK, MODE>(cs, hd, sm.w.bH[cur], sm.w.bE[cur], sm.w.bH[cur ^ 1], sm.w.bE[cur ^ 1], sm.w.sA, nrows, i0,
+                                              c0, m, n, g, h, J.mul8, bestkey, besti, cap1, cap2, cap3);
+            else sweep_score<KK, MODE, true>(cs, hd, sm.w.bH[cur], sm.w.bE[cur], sm.w.bH[cur ^ 1], sm.w.bE[cur ^ 1], sm.w.sA, nrows, i0,
+                                             c0, m, n, g, h, J.mul8, bestkey, besti, cap1, cap2, cap3, sm.lo, sm.hi);
+            if (MODE == PSA_LOCAL) {          // as process_rowblock
+                const int t1v = bestkey / key_mult(KK);
+                const int bj = c0 + (key_mult(KK) - 1 - (bestkey % key_mult(KK))) + 1;
+                if (t1v > 0 && bj <= n) {
+                    const bool better = t1v > tr.best || (t1v == tr.best && (besti < tr.bi || (besti == tr.bi && bj < tr.bj)));
+                    if (better) { tr.best = t1v; tr.bi = besti; tr.bj = bj; }
+                }
+            }
+#pragma unroll
+            for (int k = 0; k < KK; ++k) {
+                const int j = c0 + k + 1;
+                if (j <= n) { J.hbufH[j] = cs.top_H(k, g + h); J.hbufF[j] = cs.ff[k]; }
+            }
+        }
+        if ((i0 + nrows == m) && (n > s * WW) && (n <= (s + 1) * WW)) captured = true;
+        corner = __shfl_sync(0xffffffffu, hlast, 31);   // H[i0][(s+1)*WW]
+        cur ^= 1;
+        __syncwarp();
+    }
+    if (MODE == PSA_GLOBAL && captured) {
+        const int src = ((n - 1) % WW) / KK;
+        if (lane == src) { J.corner[0] = cap1; J.corner[1] = cap2; J.corner[2] = cap3; }
+    }
+}
+
+// Banded result record: a global call whose band admits no path reports -inf corners with end state 1 (the state
+// find_alignment picks among equal corners) and no columns.
+__device__ __forceinline__ psa_batch_item banded_item(psa_batch_item r) {
+    if (r.score == PSA_NEG_INF) r.end_state = 1;
+    return r;
+}
+
+struct BandedBatch {
+    psa_batch_args P;
+    int* hbuf;                 // per resident warp: 2*(max_n+1) ints
+    long long hbuf_warp_stride;
+    int* ticket;
+    int bw;
+};
+
+// Score only: one warp per pair, one recycled boundary row, <128, 16> tiles.
+template <int MODE>
+__global__ void __launch_bounds__(WPB * 32) psa_banded_batch_kernel(BandedBatch Bt) {
+    constexpr int KB = 16;
+    __shared__ BandSmem smem[WPB];
+    __shared__ unsigned long long s_best[WPB];
+    __shared__ int s_corner[WPB][4];
+    const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    BandSmem& sm = smem[w];
+    const long long gw = (long long)blockIdx.x * WPB + w;
+    for (;;) {
+        long long p = 0;
+        if (lane == 0) p = atomicAdd(Bt.ticket, 1);
+        p = __shfl_sync(0xffffffffu, p, 0);
+        if (p >= Bt.P.n_pairs) break;
+        LongJob J;
+        J.a = Bt.P.bases_a + Bt.P.off_a[p]; J.b = Bt.P.bases_b + Bt.P.off_b[p];
+        J.m = Bt.P.len_a[p]; J.n = Bt.P.len_b[p]; J.g = Bt.P.g; J.h = Bt.P.h; J.mul8 = key_mult(KB);
+        J.hbufH = Bt.hbuf + gw * Bt.hbuf_warp_stride; J.hbufF = J.hbufH + Bt.hbuf_warp_stride / 2; J.hb_stride = 0;
+        J.ckvH = nullptr; J.ckvE = nullptr; J.progress = nullptr; J.ticket = nullptr;
+        J.best = &s_best[w]; J.corner = s_corner[w];
+        J.col0 = 0; J.n_total = J.n; J.row_off = 0;
+        J.start_type = -1; J.end_type = -1;
+        if (lane == 0) { s_best[w] = 0ull; s_corner[w][0] = s_corner[w][1] = s_corner[w][2] = PSA_KNEG; }
+        __syncwarp();
+        if (J.m > 0 && J.n > 0) {
+            const Band B{J.m, J.n, Bt.bw};
+            Track tr{0, 0, 0};
+            const int NB = (J.m + R - 1) / R;
+            for (int rb = 0; rb < NB; ++rb) process_rowblock_banded<MODE, KB, false>(J, B, rb, sm, tr, nullptr, nullptr);
+            flush_track<MODE>(J, tr);
+            __syncwarp();
+        }
+        if (lane == 0) {
+            psa_batch_item r;
+            if (J.m <= 0 || J.n <= 0) r = empty_item<MODE>(J.m, J.n, J.g, J.h, -1, -1);
+            else if (MODE == PSA_LOCAL) r = local_item_from_key(s_best[w]);
+            else r = global_item(s_corner[w][0], s_corner[w][1], s_corner[w][2], J.m, J.n, J.h, -1);
+            Bt.P.items[p] = banded_item(r);
+        }
+        __syncwarp();
+    }
+}
+
+// Traceback: pair p of the chunk [p0, p0 + count) owns slot p - p0: [best (8 B) | corner (3 x 4 B) | pad to 256 B |
+// tile_base (NB x 8 B, padded to 256 B) | tile records (REC ints each)], inside slot_bytes (planned from max m, max n, bw).
+struct BandedTb {
+    psa_batch_args P;
+    long long p0, count;
+    uint8_t* region;
+    long long slot_bytes;
+    int* ticket;
+    int bw;
+};
+
+__device__ __forceinline__ LongJob banded_tb_job(const BandedTb& Bt, long long p, BandCk& bk) {
+    const psa_batch_args& P = Bt.P;
+    LongJob J;
+    J.a = P.bases_a + P.off_a[p]; J.b = P.bases_b + P.off_b[p];
+    J.m = P.len_a[p]; J.n = P.len_b[p]; J.g = P.g; J.h = P.h; J.mul8 = key_mult(K);
+    uint8_t* slot = Bt.region + (p - Bt.p0) * Bt.slot_bytes;
+    const int NB = (J.m + R - 1) / R;
+    J.best = (unsigned long long*)slot; J.corner = (int*)(slot + 8);
+    J.hbufH = nullptr; J.hbufF = nullptr; J.hb_stride = 0;
+    J.ckvH = nullptr; J.ckvE = nullptr; J.progress = nullptr; J.ticket = nullptr;
+    J.col0 = 0; J.n_total = J.n; J.row_off = 0; J.start_type = -1; J.end_type = -1;
+    bk.B = Band{J.m, J.n, Bt.bw};
+    bk.tile_base = (long long*)(slot + 256);
+    bk.rec = (int*)(slot + 256 + up256_d((long long)NB * 8));
+    return J;
+}
+
+template <int MODE>
+__global__ void __launch_bounds__(WPB * 32) psa_banded_tb_fill_kernel(BandedTb Bt) {
+    __shared__ BandSmem smem[WPB];
+    const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    BandSmem& sm = smem[w];
+    for (;;) {
+        long long q = 0;
+        if (lane == 0) q = atomicAdd(Bt.ticket, 1);
+        q = __shfl_sync(0xffffffffu, q, 0);
+        if (q >= Bt.count) break;
+        BandCk bk;
+        const LongJob J = banded_tb_job(Bt, Bt.p0 + q, bk);
+        if (J.m <= 0 || J.n <= 0) continue;          // borders only: the walk kernel writes the item
+        if (lane == 0) { *J.best = 0ull; J.corner[0] = J.corner[1] = J.corner[2] = PSA_KNEG; }
+        __syncwarp();
+        Track tr{0, 0, 0};
+        const int NB = (J.m + R - 1) / R;
+        long long base = 0, prev = 0;
+        for (int rb = 0; rb < NB; ++rb) {
+            if (lane == 0) bk.tile_base[rb] = base;
+            process_rowblock_banded<MODE, K, true>(J, bk.B, rb, sm, tr, bk.rec + base * REC, bk.rec + prev * REC);
+            prev = base;
+            base += bk.B.s_hi(rb * R, min(R, J.m - rb * R), W) - bk.B.s_lo(rb * R, W) + 1;
+        }
+        flush_track<MODE>(J, tr);
+        __syncwarp();
+    }
+}
+
+// recompute_tile for the banded layout: boundaries from the records, out-of-band values outside them, masked sweep.
+template <int MODE>
+__device__ void recompute_tile_banded(const LongJob& J, const BandCk& bk, int rb, int s, int nrows, uint32_t* dirs, int* lbH,
+                                      int* lbE, uint8_t* sA, int* bLo, int* bHi) {
+    const int lane = threadIdx.x & 31;
+    const int m = J.m, n = J.n, g = J.g, h = J.h;
+    const Band& B = bk.B;
+    const int i0 = rb * R, c0 = s * W + lane * K;
+    const int s_lo = B.s_lo(i0, W);
+    const int p_lo = rb > 0 ? B.s_lo(i0 - R, W) : 0, p_hi = rb > 0 ? B.s_hi(i0 - R, R, W) : -1;
+    const int* rec_prev = rb > 0 ? bk.rec + __ldcg(bk.tile_base + rb - 1) * REC : nullptr;
+    const int* rec_left = s > s_lo ? bk.rec + (__ldcg(bk.tile_base + rb) + (s - 1 - s_lo)) * REC : nullptr;
+    __syncwarp();
+    for (int q = lane; q < nrows; q += 32) {
+        const int i = i0 + 1 + q;
+        sA[q] = J.a[i0 + q];
+        bLo[q] = B.lo(i); bHi[q] = B.hi(i);
+        if (s > s_lo) { lbH[q] = __ldcg(rec_left + 2 * W + q); lbE[q] = __ldcg(rec_left + 2 * W + R + q); }
+        else { lbH[q] = (s == 0 && bLo[q] == 0) ? border_col0_H<MODE>(i, g, h) : oob_H<MODE>(); lbE[q] = PSA_KNEG; }
+    }
+    Cols<K> cs;
+#pragma unroll
+    for (int k = 0; k < K; ++k) {
+        const int jj = c0 + k + 1;
+        cs.b[k] = (jj <= n) ? (int)J.b[jj - 1] : 256;
+        if (jj <= n) band_top<MODE, W, true>(J, B, rec_prev, rb, i0, p_lo, p_hi, jj, cs.H[k], cs.F[k]);
+        else { cs.H[k] = PSA_KNEG; cs.F[k] = PSA_KNEG; }
+    }
+    int hd = __shfl_up_sync(0xffffffffu, cs.H[K - 1], 1);
+    int corner, dummy;
+    band_top<MODE, W, true>(J, B, rec_prev, rb, i0, p_lo, p_hi, s * W, corner, dummy);
+    if (lane == 0) hd = corner;
+    __syncwarp();
+    Track tr{0, 0, 0};
+    int d1 = 0, d2 = 0, d3 = 0;
+    sweep<K, MODE, true, true>(cs, hd, lbH, lbE, nullptr, nullptr, sA, nrows, i0, c0, m, n, g, h, dirs, tr, d1, d2, d3, bLo, bHi);
+    __syncwarp();
+}
+
+// tb_walk over the banded layout: the same steps, every tile the path enters recomputed by recompute_tile_banded.  (A
+// separate function so that the unbanded walks keep their code.)
+template <int MODE>
+__device__ void tb_walk_banded(const LongJob& J, const BandCk& bk, psa_batch_item& r, uint32_t* ops, uint32_t* dirs, int* lbH,
+                               int* lbE, uint8_t* sA, int* bLo, int* bHi) {
+    const int lane = threadIdx.x & 31;
+    const int m = J.m;
+    int i = r.end_i, j = r.end_j, state = r.end_state;
+    int trb = -1, ts = -1;      // tile currently held in `dirs`
+    int len = 0;
+    uint32_t acc = 0;
+    bool done = !(i > 0 && j > 0);
+    while (!done) {
+        int need_rb = -1, need_s = -1;
+        if (lane == 0) {
+            while (i > 0 && j > 0) {
+                const int si = (state == 2) ? i : i - 1;
+                const int sj = (state == 3) ? j : j - 1;
+                const bool border = (si == 0 || sj == 0);
+                int code = 0;
+                if (!border) {
+                    const int rb = (si - 1) / R, s = (sj - 1) / W;
+                    if (rb != trb || s != ts) { need_rb = rb; need_s = s; break; }
+                    const int cj = sj - 1 - s * W;
+                    code = (dirs[(si - 1 - rb * R) * 32 + cj / K] >> (4 * (cj % K))) & 15;
+                }
+                acc |= (uint32_t)state << (2 * (len & 15));
+                if ((len & 15) == 15) { ops[len >> 4] = acc; acc = 0; }
+                ++len;
+                r.start_i = i; r.start_j = j;
+                const int ns = next_state<MODE>(state, code, border);
+                if (ns == 0) { i = 0; break; }
+                state = ns; i = si; j = sj;
+            }
+        }
+        need_rb = __shfl_sync(0xffffffffu, need_rb, 0);
+        need_s = __shfl_sync(0xffffffffu, need_s, 0);
+        if (need_rb < 0) break;
+        const int need_row = __shfl_sync(0xffffffffu, (lane == 0) ? ((state == 2) ? i : i - 1) : 0, 0);
+        const int i0 = need_rb * R, nrows = min(min(R, m - i0), need_row - i0);
+        recompute_tile_banded<MODE>(J, bk, need_rb, need_s, nrows, dirs, lbH, lbE, sA, bLo, bHi);
+        trb = need_rb; ts = need_s;
+    }
+    if (lane == 0) {
+        if (len & 15) ops[len >> 4] = acc;
+        r.aln_len = len;
+    }
+}
+
+template <int MODE>
+__global__ void __launch_bounds__(WALK_WPB * 32) psa_banded_tb_walk_kernel(BandedTb Bt) {
+    __shared__ uint32_t dirs[WALK_WPB][R * 32];
+    __shared__ int lbH[WALK_WPB][R], lbE[WALK_WPB][R], bLo[WALK_WPB][R], bHi[WALK_WPB][R];
+    __shared__ uint8_t sA[WALK_WPB][R];
+    const int w = threadIdx.x >> 5;
+    const long long q = (long long)blockIdx.x * WALK_WPB + w;
+    if (q >= Bt.count) return;
+    const long long p = Bt.p0 + q;
+    BandCk bk;
+    const LongJob J = banded_tb_job(Bt, p, bk);
+    psa_batch_item r;
+    if (J.m <= 0 || J.n <= 0) {
+        r = empty_item<MODE>(J.m, J.n, J.g, J.h, -1, -1);
+    } else {
+        r = banded_item(tb_end<MODE>(J));
+        if (r.score != PSA_NEG_INF)
+            tb_walk_banded<MODE>(J, bk, r, Bt.P.ops + p * Bt.P.ops_stride_words, dirs[w], lbH[w], lbE[w], sA[w], bLo[w], bHi[w]);
+    }
+    if ((threadIdx.x & 31) == 0) Bt.P.items[p] = r;
+}
+
 }  // namespace
 
 // ---- host side ---------------------------------------------------------------------------
@@ -741,6 +1125,76 @@ int psa_launch_long_batch_tb(psa_ctx* ctx, const psa_batch_args& args, int max_m
         } else {
             psa_long_batch_tb_fill_kernel<PSA_GLOBAL><<<fill_grid, WPB * 32, 0, st>>>(Bt);
             psa_long_batch_tb_walk_kernel<PSA_GLOBAL><<<walk_grid, WALK_WPB * 32, 0, st>>>(Bt);
+        }
+        PSA_CUDA_OK(ctx, cudaGetLastError());
+        ctx->launches += 2;
+    }
+    return PSA_OK;
+}
+
+// ---- banded batches ------------------------------------------------------------------------------------------------
+// Every pair runs on the banded tile kernels, one warp per pair, whatever its length.  Score only: one launch, a
+// recycled boundary row per resident warp.  Traceback: chunks of fill -> walk as psa_launch_long_batch_tb, with slots
+// sized by the band: row block rb computes s_hi - s_lo + 1 <= (its band's column span) / W + 2 tiles, and the spans
+// summed over the NB row blocks are at most n + 2*bw*NB (c(i) rises by n over the matrix), so a pair of at most
+// max_m x max_n holds at most min(NB*S, (max_n + 2*bw*NB)/W + 2*NB) tiles -- a bound that needs no lengths.
+namespace {
+size_t banded_slot_bytes(int max_m, int max_n, int bw) {
+    const long long NB = ((long long)max_m + R - 1) / R, S = ((long long)max_n + W - 1) / W;
+    const long long tiles = std::min(NB * S, ((long long)max_n + 2LL * bw * NB) / W + 2 * NB);
+    return 256 + up256((size_t)NB * 8) + (size_t)tiles * REC * 4;
+}
+}  // namespace
+
+int psa_launch_banded(psa_ctx* ctx, const psa_batch_args& args, int max_m, int max_n, int mode, int band, bool traceback,
+                      cudaStream_t st) {
+    if (max_m >= 0x1FFFFF || max_n >= 0x1FFFFF) return psa_fail(ctx, PSA_ERR_RANGE, "long path: lengths must be < 2^21 - 1");
+    const int bw = (int)std::min<long long>(band, (long long)max_m + max_n);     // wider bands admit the same cells
+    const bool local = mode == PSA_LOCAL;
+    if (!traceback) {
+        const void* kern = local ? (const void*)psa_banded_batch_kernel<PSA_LOCAL> : (const void*)psa_banded_batch_kernel<PSA_GLOBAL>;
+        int grid = 1;
+        int rc = long_batch_grid(ctx, args.n_pairs, kern, &grid);
+        if (rc) return rc;
+        const size_t warp_stride = up256((size_t)(max_n + 1) * 4) / 4 * 2;       // ints: H row + F row
+        const size_t hb = (size_t)grid * WPB * warp_stride * 4;
+        rc = ensure_work(ctx, hb + 256);
+        if (rc) return rc;
+        uint8_t* d = (uint8_t*)ctx->d_work;
+        PSA_CUDA_OK(ctx, cudaMemsetAsync(d + hb, 0, 256, st));
+        BandedBatch Bt{args, (int*)d, (long long)warp_stride, (int*)(d + hb), bw};
+        void* kargs[] = {&Bt};
+        PSA_CUDA_OK(ctx, cudaLaunchKernel(kern, dim3(grid), dim3(WPB * 32), kargs, 0, st));
+        ctx->launches += 1;
+        return PSA_OK;
+    }
+    int per_sm = 0;
+    const void* fill = local ? (const void*)psa_banded_tb_fill_kernel<PSA_LOCAL> : (const void*)psa_banded_tb_fill_kernel<PSA_GLOBAL>;
+    PSA_CUDA_OK(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fill, WPB * 32, 0));
+    const long long ctas = std::max(1, std::min(per_sm, 4) * ctx->sm_count);
+    size_t free_b = 0, total_b = 0;
+    PSA_CUDA_OK(ctx, cudaMemGetInfo(&free_b, &total_b));
+    const size_t budget = (free_b + ctx->d_work_bytes) / 2;
+    const size_t slot = banded_slot_bytes(max_m, max_n, bw);
+    long long chunk = std::min<long long>(args.n_pairs, ctas * WPB);
+    chunk = std::min<long long>(chunk, (long long)((budget > 256 ? budget - 256 : 0) / slot));
+    if (ctx->opt.long_tb_chunk > 0) chunk = std::min<long long>(chunk, ctx->opt.long_tb_chunk);
+    chunk = std::max(1LL, chunk);          // one slot over the budget: try it anyway
+    int rc = ensure_work(ctx, 256 + (size_t)chunk * slot);
+    if (rc) return rc;
+    uint8_t* d = (uint8_t*)ctx->d_work;
+    for (long long p0 = 0; p0 < args.n_pairs; p0 += chunk) {
+        const long long cnt = std::min(chunk, args.n_pairs - p0);
+        BandedTb Bt{args, p0, cnt, d + 256, (long long)slot, (int*)d, bw};
+        PSA_CUDA_OK(ctx, cudaMemsetAsync(d, 0, 256, st));
+        const int fill_grid = (int)std::min<long long>((cnt + WPB - 1) / WPB, ctas);
+        const int walk_grid = (int)((cnt + WALK_WPB - 1) / WALK_WPB);
+        if (local) {
+            psa_banded_tb_fill_kernel<PSA_LOCAL><<<fill_grid, WPB * 32, 0, st>>>(Bt);
+            psa_banded_tb_walk_kernel<PSA_LOCAL><<<walk_grid, WALK_WPB * 32, 0, st>>>(Bt);
+        } else {
+            psa_banded_tb_fill_kernel<PSA_GLOBAL><<<fill_grid, WPB * 32, 0, st>>>(Bt);
+            psa_banded_tb_walk_kernel<PSA_GLOBAL><<<walk_grid, WALK_WPB * 32, 0, st>>>(Bt);
         }
         PSA_CUDA_OK(ctx, cudaGetLastError());
         ctx->launches += 2;

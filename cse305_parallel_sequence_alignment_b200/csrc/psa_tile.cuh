@@ -35,10 +35,13 @@ struct Track {    // local mode: best T1 seen by this lane and its first cell (r
 //   sA        row characters of the tile rows (index r)
 //   dirs      shared memory, 32 words per tile row, or null
 //   cap_*     global mode: receives T1/T2/T3 of cell (m, n) when the tile contains it
-template <int K, int MODE, bool DIRS>
+//   BANDED    a band edge cuts the tile: cell (i, j) of tile row r exists only for bLo[r] <= j <= bHi[r]; every other
+//             cell is forced to the out-of-band value (H = T1 = 0 in local mode, else the sentinel; E = F = sentinel)
+template <int K, int MODE, bool DIRS, bool BANDED = false>
 __device__ __forceinline__ void sweep(Cols<K>& cs, int hd, const int* lbH, const int* lbE, int* rbH, int* rbE,
                                       const uint8_t* sA, int nrows, int i0, int c0, int m, int n, int g, int h,
-                                      uint32_t* dirs, Track& tr, int& cap1, int& cap2, int& cap3) {
+                                      uint32_t* dirs, Track& tr, int& cap1, int& cap2, int& cap3,
+                                      const int* bLo = nullptr, const int* bHi = nullptr) {
     constexpr bool LOCAL = (MODE == PSA_LOCAL);
     const int lane = threadIdx.x & 31;
     const int go = g + h;
@@ -57,12 +60,14 @@ __device__ __forceinline__ void sweep(Cols<K>& cs, int hd, const int* lbH, const
             const int hl0 = hl;
             int diag = hd;
             uint32_t word = 0;
+            const int klo = BANDED ? bLo[r] - c0 - 1 : 0, khi = BANDED ? bHi[r] - c0 - 1 : 0;
 #pragma unroll
             for (int k = 0; k < K; ++k) {
-                const int t1 = (LOCAL ? imax(diag, 0) : diag) + (a == cs.b[k] ? 1 : 0);
-                const int e = imax(hl - go, el - g);
-                const int f = imax(cs.H[k] - go, cs.F[k] - g);
-                const int H = imax(t1, imax(e, f));
+                int t1 = (LOCAL ? imax(diag, 0) : diag) + (a == cs.b[k] ? 1 : 0);
+                int e = imax(hl - go, el - g);
+                int f = imax(cs.H[k] - go, cs.F[k] - g);
+                int H = imax(t1, imax(e, f));
+                if (BANDED && (k < klo || k > khi)) { t1 = H = LOCAL ? 0 : PSA_KNEG; e = f = PSA_KNEG; }
                 if (DIRS) {
                     int d1 = (t1 == H) ? 1 : (e >= f ? 2 : 3);
                     const int z2 = (d1 == 1) ? (e + h > H) : (e + h >= H);
@@ -128,9 +133,12 @@ struct ColsS {
     }
 };
 
-template <int K, bool LOCAL, bool CAP>
+// BANDED: columns k < klo and k > khi of the lane are outside the band; they leave (H, T1, E, F) = the out-of-band value
+// (TF form: hg = TF = H - go, E = F = sentinel).
+template <int K, bool LOCAL, bool CAP, bool BANDED = false>
 __device__ __forceinline__ void score_step_tf(ColsS<K>& cs, int& tf_io, int& e_io, int diag_hg, int a, int ng, int ngo, int go,
-                                              int mul8, int& rowkey, int kcap, int& cap1, int& cap2, int& cap3) {
+                                              int mul8, int& rowkey, int kcap, int& cap1, int& cap2, int& cap3,
+                                              int klo = 0, int khi = 0) {
     int t1g[K], tfn[K];
     // everything that depends only on the row above first (off the E chain)
 #pragma unroll
@@ -138,12 +146,14 @@ __device__ __forceinline__ void score_step_tf(ColsS<K>& cs, int& tf_io, int& e_i
         t1g[k] = (k == 0 ? diag_hg : cs.hg[k - 1]) + (a == cs.b[k] ? 1 : 0);
         cs.ff[k] = __viaddmax_s32(cs.ff[k], ng, cs.hg[k]);
         tfn[k] = __viaddmax_s32(cs.ff[k], ngo, t1g[k]);
+        if (BANDED && (k < klo || k > khi)) { cs.ff[k] = PSA_KNEG; t1g[k] = tfn[k] = (LOCAL ? 0 : PSA_KNEG) - go; }
     }
     int key_prev = 0;
     int e = e_io, tf = tf_io;
 #pragma unroll
     for (int k = 0; k < K; ++k) {
         e = __viaddmax_s32(e, ng, tf);
+        if (BANDED && (k < klo || k > khi)) e = PSA_KNEG;
         tf = tfn[k];
         const int hgk = __viaddmax_s32(e, ngo, tf);
         if (LOCAL) {
@@ -181,13 +191,16 @@ __device__ __forceinline__ void score_step_h(ColsS<K>& cs, int& hlgo, int& el, i
 
 // lbH/lbE, rbH/rbE hold H and E (external format); hd = H[i0][c0].  bestkey/besti: local-mode
 // tracker of this lane for this tile (key = T1*KM + KM-1-k, row), folded by the caller.
-template <int K, int MODE>
+// BANDED (TF form only): the band of tile row r is columns bLo[r] .. bHi[r], as in sweep<>.
+template <int K, int MODE, bool BANDED = false>
 __device__ __forceinline__ void sweep_score(ColsS<K>& cs, int hd, const int* lbH, const int* lbE, int* rbH, int* rbE,
                                             const uint8_t* sA, int nrows, int i0, int c0, int m, int n, int g, int h,
-                                            int mul8, int& bestkey, int& besti, int& cap1, int& cap2, int& cap3) {
+                                            int mul8, int& bestkey, int& besti, int& cap1, int& cap2, int& cap3,
+                                            const int* bLo = nullptr, const int* bHi = nullptr) {
     static_assert(K % 2 == 0, "the row key folds two cells per VIMNMX3");
     constexpr bool LOCAL = (MODE == PSA_LOCAL);
     constexpr bool TF = tf_form(K);
+    static_assert(TF || !BANDED, "the band mask is written for the TF form");
     constexpr int KM = key_mult(K);
     const int lane = threadIdx.x & 31;
     const int go = g + h, ng = -g, ngo = -go;
@@ -212,8 +225,9 @@ __device__ __forceinline__ void sweep_score(ColsS<K>& cs, int hd, const int* lbH
             int rowkey = 0;
             if (TF) {
                 const int hg_left = __viaddmax_s32(el, ngo, x);       // H[i][c0] - go: the next row's diagonal
-                if (!anycap) score_step_tf<K, LOCAL, false>(cs, x, el, diag, a, ng, ngo, go, mul8, rowkey, -1, cap1, cap2, cap3);
-                else score_step_tf<K, LOCAL, true>(cs, x, el, diag, a, ng, ngo, go, mul8, rowkey, capstep ? kcap : -1, cap1, cap2, cap3);
+                const int klo = BANDED ? bLo[r] - c0 - 1 : 0, khi = BANDED ? bHi[r] - c0 - 1 : 0;
+                if (!anycap) score_step_tf<K, LOCAL, false, BANDED>(cs, x, el, diag, a, ng, ngo, go, mul8, rowkey, -1, cap1, cap2, cap3, klo, khi);
+                else score_step_tf<K, LOCAL, true, BANDED>(cs, x, el, diag, a, ng, ngo, go, mul8, rowkey, capstep ? kcap : -1, cap1, cap2, cap3, klo, khi);
                 diag = hg_left;
             } else {
                 const int hin = x;

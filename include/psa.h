@@ -171,6 +171,29 @@ int psa_align_batch_device(psa_ctx* ctx, const uint8_t* d_bases_a, const int64_t
                            size_t n_pairs, int max_len_a, int max_len_b, int mode, int g, int h, unsigned flags,
                            psa_batch_item* d_items, uint32_t* d_ops, size_t ops_stride_words, void* cuda_stream);
 
+/* ---- banded batches ------------------------------------------------------------------------
+ * psa_align_batch / psa_align_batch_device restricted to a diagonal band of half-width `band` >= 0: for a pair of
+ * lengths m, n >= 1, cell (i, j) exists iff |j - floor(i*n/m)| <= band (the band around the line from (0,0) to (m,n));
+ * every other cell is -infinity.  Inside the band the recurrence, borders, scoring, end cell, tie rules and traceback
+ * order are psa_align_batch's, in both modes (a local alignment may start at any cell of the band).  Cell (m, n) is
+ * always in the band; if the band admits no complete global path the record reports PSA_NEG_INF corners and score,
+ * end state 1, aln_len 0, and no op words are written.  Members with m = 0 or n = 0 get psa_align_batch's record.
+ * With band >= max(m, n) every cell is in the band and the results equal psa_align_batch's exactly.
+ * For similar sequences (reads against their source window, overlaps, polishing) the fill and the traceback
+ * checkpoints shrink from m*n to about m*(2*band + 1) cells.  Same buffer layouts, op-word format and capacity rule as
+ * psa_align_batch; flags: PSA_WANT_SCORE and PSA_WANT_TRACEBACK only (anything else: PSA_ERR_ARG); lengths < 2^21 - 1.
+ * Every pair runs on the banded long-pair kernels, one warp per pair: short pairs are correct but gain nothing from
+ * the band over psa_align_batch.  The device form is asynchronous on cuda_stream (NULL = the context's stream) and
+ * plans its work from n_pairs, max_len_a, max_len_b and band alone. */
+int psa_align_batch_banded(psa_ctx* ctx, const uint8_t* bases_a, const int64_t* off_a, const int32_t* len_a,
+                           const uint8_t* bases_b, const int64_t* off_b, const int32_t* len_b, size_t n_pairs,
+                           size_t bytes_a, size_t bytes_b, int mode, int g, int h, int band, unsigned flags,
+                           psa_batch_item* items, uint32_t* ops, size_t ops_stride_words);
+int psa_align_batch_banded_device(psa_ctx* ctx, const uint8_t* d_bases_a, const int64_t* d_off_a, const int32_t* d_len_a,
+                                  const uint8_t* d_bases_b, const int64_t* d_off_b, const int32_t* d_len_b, size_t n_pairs,
+                                  int max_len_a, int max_len_b, int mode, int g, int h, int band, unsigned flags,
+                                  psa_batch_item* d_items, uint32_t* d_ops, size_t ops_stride_words, void* cuda_stream);
+
 /* ---- fixed-stride batches of 2-bit packed DNA reads ----------------------------------------
  * The short-read shape of config 2 as a production caller would hold it: every pair is len_a x len_b
  * (len_a <= 512, len_b <= 256), both sides packed 16 bases per 32-bit word (base r of a sequence in
