@@ -123,6 +123,12 @@ def load_library() -> C.CDLL:
     lib.psa_align_long_device.restype = C.c_int
     lib.psa_align_long_device.argtypes = [vp, vp, vp, C.c_size_t, C.c_size_t, C.c_int, C.c_int, C.c_int, C.c_uint,
                                           vp, vp, C.c_size_t, vp]
+    lib.psa_align_pair_banded.restype = C.c_int
+    lib.psa_align_pair_banded.argtypes = [vp, C.c_char_p, C.c_char_p, C.c_size_t, C.c_size_t, C.c_int, C.c_int, C.c_int, C.c_int,
+                                          C.c_uint, C.POINTER(_Result)]
+    lib.psa_align_long_banded_device.restype = C.c_int
+    lib.psa_align_long_banded_device.argtypes = [vp, vp, vp, C.c_size_t, C.c_size_t, C.c_int, C.c_int, C.c_int, C.c_int, C.c_uint,
+                                                 vp, vp, C.c_size_t, vp]
     lib.psa_xbuf_bytes.restype = C.c_size_t
     lib.psa_xbuf_bytes.argtypes = [C.c_size_t]
     lib.psa_xbuf_create.restype = C.c_int
@@ -151,7 +157,7 @@ def load_library() -> C.CDLL:
 
 
 EXPORTS = ["psa_ctx_create", "psa_ctx_destroy", "psa_last_error", "psa_launch_count", "psa_align_pair", "psa_align_pair_typed", "psa_align_partition", "psa_align_long_partitioned", "psa_similarity_batch", "psa_similarity_batch_device",
-           "psa_result_free", "psa_align_batch", "psa_align_batch_device", "psa_align_batch_banded", "psa_align_batch_banded_device", "psa_pack_bases", "psa_pack_reads", "psa_align_batch_packed", "psa_align_long_device", "psa_xbuf_bytes", "psa_xbuf_create", "psa_xbuf_open", "psa_xbuf_close",
+           "psa_result_free", "psa_align_batch", "psa_align_batch_device", "psa_align_batch_banded", "psa_align_batch_banded_device", "psa_pack_bases", "psa_pack_reads", "psa_align_batch_packed", "psa_align_long_device", "psa_align_pair_banded", "psa_align_long_banded_device", "psa_xbuf_bytes", "psa_xbuf_create", "psa_xbuf_open", "psa_xbuf_close",
            "psa_xbuf_destroy", "psa_long_panel_strips", "psa_long_strip_columns", "psa_align_long_cyclic_device", "psa_ops_unpack", "psa_render_rows",
            "psa_peak_int_ops"]
 
@@ -434,6 +440,24 @@ class Context:
         flags = WANT_SCORE | (WANT_TRACEBACK if traceback else 0)
         self._check(self._lib.psa_align_long_device(self._h, d_a, d_b, m, n, mode, g, h, flags, d_item, d_ops or None,
                                                     ops_words, stream or None))
+
+    def align_pair_banded(self, a: bytes, b: bytes, band: int, mode: int = GLOBAL, g: int = 1, h: int = 2,
+                          traceback: bool = True, flags: Optional[int] = None) -> PairResult:
+        """psa_align_pair_banded: one pair inside the diagonal band of half-width `band`, over the whole GPU."""
+        res = _Result()
+        if flags is None:
+            flags = WANT_SCORE | (WANT_TRACEBACK if traceback else 0)
+        self._check(self._lib.psa_align_pair_banded(self._h, a, b, len(a), len(b), mode, g, h, band, flags, C.byref(res)))
+        return self._take(res, traceback)
+
+    def align_long_banded_device(self, d_a: int, d_b: int, m: int, n: int, band: int, d_item: int, d_ops: int = 0,
+                                 ops_words: int = 0, mode: int = GLOBAL, g: int = 1, h: int = 2, traceback: bool = False,
+                                 stream: int = 0, flags: Optional[int] = None):
+        """psa_align_long_banded_device: one banded pair resident in device memory (raw pointers); asynchronous on `stream`."""
+        if flags is None:
+            flags = WANT_SCORE | (WANT_TRACEBACK if traceback else 0)
+        self._check(self._lib.psa_align_long_banded_device(self._h, d_a, d_b, m, n, mode, g, h, band, flags, d_item,
+                                                           d_ops or None, ops_words, stream or None))
 
     # ---- one long pair over several GPUs: block-cyclic systolic panels (config 4) ----
     def xbuf_create(self, m_cap: int):

@@ -405,6 +405,32 @@ int psa_align_batch_banded_device(psa_ctx* ctx, const uint8_t* d_bases_a, const 
     return psa_stream_leave(ctx, st);
 }
 
+// Argument rules shared by both forms of the one-pair banded entry (the host form handles m = 0 or n = 0 itself).
+static int check_banded_pair(psa_ctx* ctx, size_t m, size_t n, int mode, int g, int h, int band, unsigned flags) {
+    if (band < 0) return psa_fail(ctx, PSA_ERR_ARG, "band must be >= 0");
+    if (flags & ~(PSA_WANT_SCORE | PSA_WANT_TRACEBACK)) return psa_fail(ctx, PSA_ERR_ARG, "flags: PSA_WANT_SCORE and PSA_WANT_TRACEBACK only");
+    if (m >= 0x1FFFFF || n >= 0x1FFFFF) return psa_fail(ctx, PSA_ERR_RANGE, "long path: lengths must be < 2^21 - 1");
+    return check_scoring(ctx, mode, g, h, (int64_t)m, (int64_t)n);
+}
+
+int psa_align_long_banded_device(psa_ctx* ctx, const uint8_t* d_a, const uint8_t* d_b, size_t m, size_t n, int mode, int g,
+                                 int h, int band, unsigned flags, psa_batch_item* d_item, uint32_t* d_ops, size_t ops_words,
+                                 void* cuda_stream) {
+    if (!ctx) return PSA_ERR_ARG;
+    if (!d_a || !d_b || !d_item || m == 0 || n == 0) return psa_fail(ctx, PSA_ERR_ARG, "null pointer or empty sequence");
+    int rc = check_banded_pair(ctx, m, n, mode, g, h, band, flags);
+    if (rc) return rc;
+    const bool tb = (flags & PSA_WANT_TRACEBACK) != 0;
+    if (tb && (!d_ops || ops_words * 16 < m + n)) return psa_fail(ctx, PSA_ERR_CAPACITY, "ops buffer < ceil((m+n)/16) words");
+    PSA_CUDA_OK(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : ctx->stream;
+    rc = psa_stream_enter(ctx, st);
+    if (rc) return rc;
+    rc = psa_launch_banded_pair(ctx, d_a, d_b, (int)m, (int)n, mode, g, h, band, tb, d_item, d_ops, st);
+    if (rc) return rc;
+    return psa_stream_leave(ctx, st);
+}
+
 int psa_align_long_device(psa_ctx* ctx, const uint8_t* d_a, const uint8_t* d_b, size_t m, size_t n, int mode, int g, int h,
                           unsigned flags, psa_batch_item* d_item, uint32_t* d_ops, size_t ops_words, void* cuda_stream) {
     if (!ctx) return PSA_ERR_ARG;
@@ -568,6 +594,20 @@ static int alloc_alignment(psa_ctx* ctx, psa_result* out, int64_t len) {
     return PSA_OK;
 }
 
+// *out from one pair's record and, with traceback (words != null), its op words: ops, then rows through psa_render_rows.
+static int fill_result(psa_ctx* ctx, psa_result* out, const psa_batch_item& it, const uint32_t* words, const char* a, const char* b) {
+    out->t1 = it.t1; out->t2 = it.t2; out->t3 = it.t3; out->score = it.score; out->end_state = it.end_state;
+    out->end_i = it.end_i; out->end_j = it.end_j; out->start_i = it.start_i; out->start_j = it.start_j;
+    out->aln_len = it.aln_len;
+    if (words) {
+        int rc = alloc_alignment(ctx, out, it.aln_len);
+        if (rc) return rc;
+        psa_ops_unpack(words, it.aln_len, out->ops);
+        psa_render_rows(a, b, out->ops, it.aln_len, it.start_i, it.start_j, out->row_a, out->row_b);
+    }
+    return PSA_OK;
+}
+
 static bool ok_type(int t) { return t == -1 || t == -2 || t == -3 || t == 1 || t == 2 || t == 3; }
 
 static int align_pair_impl(psa_ctx* ctx, const char* a, const char* b, size_t m, size_t n, int mode, int g, int h,
@@ -585,16 +625,7 @@ static int align_pair_impl(psa_ctx* ctx, const char* a, const char* b, size_t m,
     int rc = align_batch_host(ctx, (const uint8_t*)a, &off, &lm, (const uint8_t*)b, &off, &ln, 1, m, n, mode, g, h,
                               flags, &it, tb ? words.data() : nullptr, stride, ty);
     if (rc) return rc;
-    out->t1 = it.t1; out->t2 = it.t2; out->t3 = it.t3; out->score = it.score; out->end_state = it.end_state;
-    out->end_i = it.end_i; out->end_j = it.end_j; out->start_i = it.start_i; out->start_j = it.start_j;
-    out->aln_len = it.aln_len;
-    if (tb) {
-        rc = alloc_alignment(ctx, out, it.aln_len);
-        if (rc) return rc;
-        psa_ops_unpack(words.data(), it.aln_len, out->ops);
-        psa_render_rows(a, b, out->ops, it.aln_len, it.start_i, it.start_j, out->row_a, out->row_b);
-    }
-    return PSA_OK;
+    return fill_result(ctx, out, it, tb ? words.data() : nullptr, a, b);
 }
 
 extern "C" {
@@ -602,6 +633,37 @@ extern "C" {
 int psa_align_pair(psa_ctx* ctx, const char* a, const char* b, size_t m, size_t n, int mode, int g, int h,
                    unsigned flags, psa_result* out) {
     return align_pair_impl(ctx, a, b, m, n, mode, g, h, flags, out, psa_piece_types{});
+}
+
+int psa_align_pair_banded(psa_ctx* ctx, const char* a, const char* b, size_t m, size_t n, int mode, int g, int h, int band,
+                          unsigned flags, psa_result* out) {
+    if (!ctx) return PSA_ERR_ARG;
+    if (!out || (!a && m) || (!b && n)) return psa_fail(ctx, PSA_ERR_ARG, "null pointer");
+    int rc = check_banded_pair(ctx, m, n, mode, g, h, band, flags);
+    if (rc) return rc;
+    if (m == 0 || n == 0) return align_pair_impl(ctx, a, b, m, n, mode, g, h, flags, out, psa_piece_types{});
+    memset(out, 0, sizeof(*out));
+    const bool tb = (flags & PSA_WANT_TRACEBACK) != 0;
+    const size_t words = (m + n + 15) / 16 + 1;
+    PSA_CUDA_OK(ctx, cudaSetDevice(ctx->device));
+    // an asynchronous device call of this context may still be using the shared scratch on a user stream
+    if (ctx->last_valid) { PSA_CUDA_OK(ctx, cudaEventSynchronize(ctx->last_event)); ctx->last_valid = false; }
+    const size_t o_a = 0, o_b = align_up(m, 256), o_it = o_b + align_up(n, 256), o_op = o_it + 256;
+    rc = ensure_scratch(ctx, o_op + (tb ? words * 4 : 0));
+    if (rc) return rc;
+    uint8_t* d = (uint8_t*)ctx->d_scratch;
+    cudaStream_t st = ctx->stream;
+    PSA_CUDA_OK(ctx, cudaMemcpyAsync(d + o_a, a, m, cudaMemcpyHostToDevice, st));
+    PSA_CUDA_OK(ctx, cudaMemcpyAsync(d + o_b, b, n, cudaMemcpyHostToDevice, st));
+    rc = psa_launch_banded_pair(ctx, d + o_a, d + o_b, (int)m, (int)n, mode, g, h, band, tb, (psa_batch_item*)(d + o_it),
+                                tb ? (uint32_t*)(d + o_op) : nullptr, st);
+    if (rc) return rc;
+    psa_batch_item it;
+    std::vector<uint32_t> w(tb ? words : 0);
+    PSA_CUDA_OK(ctx, cudaMemcpyAsync(&it, d + o_it, sizeof(it), cudaMemcpyDeviceToHost, st));
+    if (tb) PSA_CUDA_OK(ctx, cudaMemcpyAsync(w.data(), d + o_op, words * 4, cudaMemcpyDeviceToHost, st));
+    PSA_CUDA_OK(ctx, cudaStreamSynchronize(st));
+    return fill_result(ctx, out, it, tb ? w.data() : nullptr, a, b);
 }
 
 int psa_align_pair_typed(psa_ctx* ctx, const char* a, const char* b, size_t m, size_t n, int start_type, int end_type,

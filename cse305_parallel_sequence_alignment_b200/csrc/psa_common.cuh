@@ -166,5 +166,8 @@ int psa_launch_long_batch_tb(psa_ctx* ctx, const psa_batch_args& args, int max_m
 // Banded batch (psa_align_batch_banded): every pair on the banded tile kernels, one warp per pair (psa_long.cu).
 int psa_launch_banded(psa_ctx* ctx, const psa_batch_args& args, int max_m, int max_n, int mode, int band, bool traceback,
                       cudaStream_t st);
+// One banded pair over the whole GPU (psa_align_pair_banded, psa_align_long_banded_device; psa_long.cu).
+int psa_launch_banded_pair(psa_ctx* ctx, const uint8_t* d_a, const uint8_t* d_b, int m, int n, int mode, int g, int h, int band,
+                           bool traceback, psa_batch_item* d_item, uint32_t* d_ops, cudaStream_t st);
 bool psa_pack_long_supported(int max_m, int max_n, int mode, int g, int h);
 int psa_launch_pack_long(psa_ctx* ctx, const psa_batch_args& args, int max_m, int max_n, int mode, cudaStream_t st);

@@ -560,10 +560,11 @@ __device__ __forceinline__ void band_top(const LongJob& J, const Band& B, const 
     }
 }
 
-// One row block of a banded pair, warp-collective.  Score only (TB = false): <128, 16> grid, TF-form sweeps, bottom row
+// One row block of a banded pair, warp-collective.  Score only (TB = false): <128, KK> grid, TF-form sweeps, bottom row
 // into the recycled row.  Traceback fill (TB = true): <128, 8> grid, sweep<> without codes, every tile's bottom row and
 // right column into the records rec_cur (row block rb) -- rec_prev are row block rb-1's.
-template <int MODE, int KK, bool TB>
+// WAIT (one pair over many warps): row block rb-1 may still be running; J.progress[rb] = 1 + the last strip finished.
+template <int MODE, int KK, bool TB, bool WAIT = false>
 __device__ void process_rowblock_banded(const LongJob& J, const Band& B, int rb, BandSmem& sm, Track& tr, int* rec_cur,
                                         const int* rec_prev) {
     constexpr int WW = 32 * KK;
@@ -580,6 +581,19 @@ __device__ void process_rowblock_banded(const LongJob& J, const Band& B, int rb,
         sm.w.bH[0][r] = (s_lo == 0 && sm.lo[r] == 0) ? border_col0_H<MODE>(i, g, h) : oob_H<MODE>();
         sm.w.bE[0][r] = PSA_KNEG;
     }
+    // Row block rb-1 wrote strips p_lo .. p_hi of row i0; the top of strip s and the corner H[i0][s_lo*WW] (strip s_lo - 1)
+    // are ready once it has finished strip min(s, p_hi).  Polling as process_rowblock does.
+    auto wait_for = [&](int strip) {
+        if constexpr (WAIT) {
+            if (rb > 0) {
+                unsigned ns = 32;
+                while (ld_relaxed(J.progress + rb - 1) <= strip) { __nanosleep(ns); if (ns < 2048) ns <<= 1; }
+                __threadfence();
+                __syncwarp();
+            }
+        }
+    };
+    wait_for(min(s_lo, p_hi));
     int corner, dummy;
     band_top<MODE, WW, TB>(J, B, rec_prev, rb, i0, p_lo, p_hi, s_lo * WW, corner, dummy);
     __syncwarp();
@@ -587,6 +601,7 @@ __device__ void process_rowblock_banded(const LongJob& J, const Band& B, int rb,
     int cap1 = PSA_KNEG, cap2 = PSA_KNEG, cap3 = PSA_KNEG;
     bool captured = false;
     for (int s = s_lo; s <= s_hi; ++s) {
+        if (s > s_lo && s <= p_hi) wait_for(s);
         const int c0 = s * WW + lane * KK;
         const bool inside = B.inside(i0, nrows, s, WW);
         int hlast;
@@ -654,6 +669,11 @@ __device__ void process_rowblock_banded(const LongJob& J, const Band& B, int rb,
         corner = __shfl_sync(0xffffffffu, hlast, 31);   // H[i0][(s+1)*WW]
         cur ^= 1;
         __syncwarp();
+        if constexpr (WAIT) {
+            __threadfence();
+            __syncwarp();
+            if (lane == 0) st_release(J.progress + rb, s + 1);
+        }
     }
     if (MODE == PSA_GLOBAL && captured) {
         const int src = ((n - 1) % WW) / KK;
@@ -816,6 +836,33 @@ __device__ void recompute_tile_banded(const LongJob& J, const BandCk& bk, int rb
     __syncwarp();
 }
 
+// Lane 0's steps of a banded walk through tile (trb, ts), whose codes `dirs` holds: ops from (i, j, state) on until the
+// path ends (need_rb stays -1) or its next source cell lies in tile (need_rb, need_s).  The loop of tb_walk_banded,
+// which keeps its own copy so that the batch walk compiles unchanged.
+template <int MODE>
+__device__ __forceinline__ void walk_steps(const uint32_t* dirs, int trb, int ts, int& i, int& j, int& state, int& len,
+                                           uint32_t& acc, uint32_t* ops, psa_batch_item& r, int& need_rb, int& need_s) {
+    while (i > 0 && j > 0) {
+        const int si = (state == 2) ? i : i - 1;
+        const int sj = (state == 3) ? j : j - 1;
+        const bool border = (si == 0 || sj == 0);
+        int code = 0;
+        if (!border) {
+            const int rb = (si - 1) / R, s = (sj - 1) / W;
+            if (rb != trb || s != ts) { need_rb = rb; need_s = s; break; }
+            const int cj = sj - 1 - s * W;
+            code = (dirs[(si - 1 - rb * R) * 32 + cj / K] >> (4 * (cj % K))) & 15;
+        }
+        acc |= (uint32_t)state << (2 * (len & 15));
+        if ((len & 15) == 15) { ops[len >> 4] = acc; acc = 0; }
+        ++len;
+        r.start_i = i; r.start_j = j;
+        const int ns = next_state<MODE>(state, code, border);
+        if (ns == 0) { i = 0; break; }
+        state = ns; i = si; j = sj;
+    }
+}
+
 // tb_walk over the banded layout: the same steps, every tile the path enters recomputed by recompute_tile_banded.  (A
 // separate function so that the unbanded walks keep their code.)
 template <int MODE>
@@ -885,6 +932,165 @@ __global__ void __launch_bounds__(WALK_WPB * 32) psa_banded_tb_walk_kernel(Bande
             tb_walk_banded<MODE>(J, bk, r, Bt.P.ops + p * Bt.P.ops_stride_words, dirs[w], lbH[w], lbE[w], sA[w], bLo[w], bHi[w]);
     }
     if ((threadIdx.x & 31) == 0) Bt.P.items[p] = r;
+}
+
+// ---- one banded pair over the whole GPU (psa_align_pair_banded, psa_align_long_banded_device) --------------------------
+// Fill: the row blocks of the batch kernels above, handed out by ticket in increasing order to every warp of the grid, with
+// the progress handshake of process_rowblock_banded<..., WAIT>.  Score only: one recycled H/F row of n + 1 ints (row block
+// rb reads strip s of it before it overwrites it, rb + 1 reads it only afterwards).  Traceback: the per-tile records of
+// BandCk at tile_base[rb], computed beforehand by psa_banded_tile_base_kernel.
+struct BandedPair {
+    LongJob J;                 // progress, ticket, best, corner; hbufH / hbufF: the recycled row (score only)
+    BandCk bk;                 // traceback only
+};
+
+template <int MODE, int KK, bool TB>
+__global__ void __launch_bounds__(WPB * 32) psa_banded_pair_fill_kernel(BandedPair P) {
+    __shared__ BandSmem smem[WPB];
+    BandSmem& sm = smem[threadIdx.x >> 5];
+    const int lane = threadIdx.x & 31;
+    const LongJob& J = P.J;
+    const int NB = (J.m + R - 1) / R;
+    Track tr{0, 0, 0};
+    for (;;) {
+        int rb = 0;
+        if (lane == 0) rb = atomicAdd(J.ticket, 1);
+        rb = __shfl_sync(0xffffffffu, rb, 0);
+        if (rb >= NB) break;
+        int* cur = TB ? P.bk.rec + P.bk.tile_base[rb] * REC : nullptr;
+        const int* prev = (TB && rb > 0) ? P.bk.rec + P.bk.tile_base[rb - 1] * REC : nullptr;
+        process_rowblock_banded<MODE, KK, TB, true>(J, P.bk.B, rb, sm, tr, cur, prev);
+    }
+    flush_track<MODE>(J, tr);
+}
+
+// tile_base[rb] = tiles of row blocks 0 .. rb-1 (NB <= 16384: at most 16 row blocks per thread).
+__global__ void __launch_bounds__(1024) psa_banded_tile_base_kernel(Band B, long long* tile_base) {
+    __shared__ long long part[1024];
+    const int NB = (B.m + R - 1) / R, t = threadIdx.x;
+    const int per = (NB + 1023) / 1024, r0 = min(NB, t * per), r1 = min(NB, r0 + per);
+    auto tiles = [&](int rb) { return (long long)(B.s_hi(rb * R, min(R, B.m - rb * R), W) - B.s_lo(rb * R, W) + 1); };
+    long long sum = 0;
+    for (int rb = r0; rb < r1; ++rb) sum += tiles(rb);
+    part[t] = sum;
+    __syncthreads();
+    for (int off = 1; off < 1024; off <<= 1) {          // inclusive scan
+        const long long v = t >= off ? part[t - off] : 0;
+        __syncthreads();
+        part[t] += v;
+        __syncthreads();
+    }
+    long long base = part[t] - sum;
+    for (int rb = r0; rb < r1; ++rb) { tile_base[rb] = base; base += tiles(rb); }
+}
+
+// Walk: bottom-up in windows of row blocks rb_lo .. rb_hi-1.  For each window psa_banded_pair_codes_kernel first recomputes
+// the codes of every band tile of the window the path can still reach -- rows above the walk's current row, strips not
+// right of its current column -- all tiles in parallel; then the one-warp walk copies those codes in tile by tile (a tile
+// missing from the buffer is recomputed on demand) and leaves its state in BandedWalk for the next window.
+struct BandedWalk {
+    psa_batch_item r;          // the record being completed
+    int i, j, state, len;
+    uint32_t acc;              // partial op word
+    int done;
+};
+
+struct BandedPairTb {
+    LongJob J;
+    BandCk bk;
+    uint32_t* codes;           // [rb - rb_lo][tpr] tiles of R*32 code words
+    int tpr;                   // tile slots per row block (>= s_hi - s_lo + 1 of every row block)
+    int rb_lo, rb_hi;          // this window; rb_hi == NB: the first window
+    BandedWalk* walk;
+    psa_batch_item* item;
+    uint32_t* ops;             // null: score only (one window, which writes the record)
+};
+
+// Start of the walk: the end cell and end state of the banded record in the first window, else the saved state.
+template <int MODE>
+__device__ __forceinline__ BandedWalk walk_start(const BandedPairTb& T) {
+    if (T.rb_hi * R < T.J.m) return *T.walk;
+    BandedWalk w;
+    w.r = banded_item(tb_end<MODE>(T.J));
+    w.i = w.r.end_i; w.j = w.r.end_j; w.state = w.r.end_state; w.len = 0; w.acc = 0;
+    w.done = T.ops == nullptr || w.r.score == PSA_NEG_INF;
+    return w;
+}
+
+constexpr int CODES_WPB = 2;
+template <int MODE>
+__global__ void __launch_bounds__(CODES_WPB * 32) psa_banded_pair_codes_kernel(BandedPairTb T) {
+    __shared__ uint32_t dirs[CODES_WPB][R * 32];
+    __shared__ int lbH[CODES_WPB][R], lbE[CODES_WPB][R], bLo[CODES_WPB][R], bHi[CODES_WPB][R];
+    __shared__ uint8_t sA[CODES_WPB][R];
+    const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const long long u = (long long)blockIdx.x * CODES_WPB + w;
+    if (u >= (long long)(T.rb_hi - T.rb_lo) * T.tpr) return;
+    const int rb = T.rb_lo + (int)(u / T.tpr), t = (int)(u % T.tpr);
+    const BandedWalk st = walk_start<MODE>(T);
+    const Band& B = T.bk.B;
+    const int i0 = rb * R, nrows = min(R, T.J.m - i0), s = B.s_lo(i0, W) + t;
+    if (st.done || i0 >= st.i || s > B.s_hi(i0, nrows, W) || s * W >= st.j) return;
+    recompute_tile_banded<MODE>(T.J, T.bk, rb, s, nrows, dirs[w], lbH[w], lbE[w], sA[w], bLo[w], bHi[w]);
+    uint4* out = reinterpret_cast<uint4*>(T.codes + u * (R * 32));
+    const uint4* in = reinterpret_cast<const uint4*>(dirs[w]);
+    for (int q = lane; q < nrows * 8; q += 32) out[q] = in[q];
+}
+
+template <int MODE>
+__global__ void __launch_bounds__(32) psa_banded_pair_walk_kernel(BandedPairTb T) {
+    __shared__ uint32_t dirs[R * 32];
+    __shared__ int lbH[R], lbE[R], bLo[R], bHi[R];
+    __shared__ uint8_t sA[R];
+    const int lane = threadIdx.x;
+    const LongJob& J = T.J;
+    const Band& B = T.bk.B;
+    BandedWalk st = walk_start<MODE>(T);
+    const bool first = T.rb_hi * R >= J.m;
+    if (st.done && !first) return;                        // finished in an earlier window
+    int i = st.i, j = st.j, state = st.state, len = st.len;
+    uint32_t acc = st.acc;
+    bool done = st.done || !(i > 0 && j > 0);
+    int trb = -1, ts = -1;
+    while (!done) {
+        int need_rb = -1, need_s = -1;
+        if (lane == 0) walk_steps<MODE>(dirs, trb, ts, i, j, state, len, acc, T.ops, st.r, need_rb, need_s);
+        need_rb = __shfl_sync(0xffffffffu, need_rb, 0);
+        need_s = __shfl_sync(0xffffffffu, need_s, 0);
+        if (need_rb < 0) { done = true; break; }
+        if (need_rb < T.rb_lo) break;                     // the next window's rows
+        const int need_row = __shfl_sync(0xffffffffu, (lane == 0) ? ((state == 2) ? i : i - 1) : 0, 0);
+        const int i0 = need_rb * R, full = min(R, J.m - i0), nrows = min(full, need_row - i0);
+        const int t = need_s - B.s_lo(i0, W);
+        if (t >= 0 && t < T.tpr && need_s <= B.s_hi(i0, full, W)) {
+            const uint4* in = reinterpret_cast<const uint4*>(T.codes + ((long long)(need_rb - T.rb_lo) * T.tpr + t) * (R * 32));
+            uint4* out = reinterpret_cast<uint4*>(dirs);
+            const int total = nrows * 8;
+            __syncwarp();
+            for (int q0 = 0; q0 < total; q0 += 256) {       // as tb_walk: eight 16-byte loads in flight per lane
+                uint4 v[8];
+#pragma unroll
+                for (int x = 0; x < 8; ++x) { const int q = q0 + x * 32 + lane; if (q < total) v[x] = __ldcg(in + q); }
+#pragma unroll
+                for (int x = 0; x < 8; ++x) { const int q = q0 + x * 32 + lane; if (q < total) out[q] = v[x]; }
+            }
+            __syncwarp();
+        } else {
+            recompute_tile_banded<MODE>(J, T.bk, need_rb, need_s, nrows, dirs, lbH, lbE, sA, bLo, bHi);
+        }
+        trb = need_rb; ts = need_s;
+    }
+    if (lane == 0) {
+        if (done) {
+            if (T.ops != nullptr && st.r.score != PSA_NEG_INF) {     // as tb_walk_banded
+                if (len & 15) T.ops[len >> 4] = acc;
+                st.r.aln_len = len;
+            }
+            *T.item = st.r;
+        }
+        st.i = i; st.j = j; st.state = state; st.len = len; st.acc = acc; st.done = done;
+        *T.walk = st;
+    }
 }
 
 }  // namespace
@@ -1195,6 +1401,115 @@ int psa_launch_banded(psa_ctx* ctx, const psa_batch_args& args, int max_m, int m
         } else {
             psa_banded_tb_fill_kernel<PSA_GLOBAL><<<fill_grid, WPB * 32, 0, st>>>(Bt);
             psa_banded_tb_walk_kernel<PSA_GLOBAL><<<walk_grid, WALK_WPB * 32, 0, st>>>(Bt);
+        }
+        PSA_CUDA_OK(ctx, cudaGetLastError());
+        ctx->launches += 2;
+    }
+    return PSA_OK;
+}
+
+// ---- one banded pair over the whole GPU ----------------------------------------------------------------------------
+// Planned from (m, n, band, mode, traceback) alone.  Launches (include/psa.h): score only 2 (fill, record); traceback
+// 2 + 2 * windows (tile_base scan, fill, then per window of row blocks the code recompute and the walk).
+namespace {
+constexpr size_t kBandedCodeBytes = (size_t)256 << 20;      // window code buffer (16 KiB per tile)
+
+// Tiles of width WW one row block of a banded pair can hold: its band rows span at most 2*bw + (R-1)*n/m + 1 columns.
+long long banded_pair_tpr(int m, int n, int bw, int WW) {
+    const long long S = ((long long)n + WW - 1) / WW;
+    return std::min(S, (2LL * bw + (long long)R * n / m + 2) / WW + 2);
+}
+
+long long banded_pair_rows_per_window(int m, int n, int bw) {
+    const long long NB = ((long long)m + R - 1) / R, tpr = banded_pair_tpr(m, n, bw, W);
+    return std::min(NB, std::max(1LL, (long long)(kBandedCodeBytes / ((size_t)tpr * R * 32 * 4))));
+}
+}  // namespace
+
+int psa_launch_banded_pair(psa_ctx* ctx, const uint8_t* d_a, const uint8_t* d_b, int m, int n, int mode, int g, int h, int band,
+                           bool traceback, psa_batch_item* d_item, uint32_t* d_ops, cudaStream_t st) {
+    if (m <= 0 || n <= 0) return psa_fail(ctx, PSA_ERR_ARG, "banded pair path needs m, n >= 1");
+    if (m >= 0x1FFFFF || n >= 0x1FFFFF) return psa_fail(ctx, PSA_ERR_RANGE, "long path: lengths must be < 2^21 - 1");
+    const int bw = (int)std::min<long long>(band, (long long)m + n);
+    const bool local = mode == PSA_LOCAL;
+    const long long NB = ((long long)m + R - 1) / R;
+    const long long resident = (long long)ctx->sm_count * 4 * WPB;
+    // Score-only lane width: about (band span)/W row blocks run at once, so narrow <128, 4> tiles (W = 128) keep 4x as many
+    // warps busy as <128, 16> ones; the wider lanes (less overhead per cell) only pay once the span gives even them
+    // half of the resident warps, i.e. from a span of 256 columns per resident warp.
+    const long long span = 2LL * bw + (long long)R * n / m;
+    const int KK = traceback ? K : (span / 512 >= resident / 2 ? 16 : 4);
+    const long long tpr = banded_pair_tpr(m, n, bw, 32 * KK);
+    // memory: [misc 256: ticket | best @8 | corner @16 | walk state @64] [progress NB ints] then
+    //   score only: the recycled H and F rows;  traceback: [tile_base NB x 8 B] [records, banded_slot_bytes' bound] [codes]
+    const size_t row = up256((size_t)(n + 1) * 4);
+    const size_t o_pr = 256, o_body = o_pr + up256((size_t)NB * 4);
+    size_t ck = 0, codes = 0, total = o_body + 2 * row;
+    long long rpw = 0;
+    if (traceback) {
+        ck = banded_slot_bytes(m, n, bw) - 256;              // tile_base + records
+        rpw = banded_pair_rows_per_window(m, n, bw);
+        codes = (size_t)rpw * tpr * R * 32 * 4;
+        total = o_body + ck + codes;
+        size_t free_b = 0, total_b = 0;
+        PSA_CUDA_OK(ctx, cudaMemGetInfo(&free_b, &total_b));
+        const size_t budget = (free_b + ctx->d_work_bytes) / 2;
+        if (total > budget)
+            return psa_fail(ctx, PSA_ERR_NOMEM, "banded traceback needs " + std::to_string(total >> 20) + " MiB of checkpoints and codes, more than half of the free device memory (" + std::to_string(budget >> 20) + " MiB)");
+    }
+    int rc = ensure_work(ctx, total);
+    if (rc) return rc;
+    uint8_t* d = (uint8_t*)ctx->d_work;
+    PSA_CUDA_OK(ctx, cudaMemsetAsync(d, 0, o_body, st));
+    BandedPair P;
+    LongJob& J = P.J;
+    J.a = d_a; J.b = d_b; J.m = m; J.n = n; J.g = g; J.h = h; J.mul8 = key_mult(KK);
+    J.hbufH = traceback ? nullptr : (int*)(d + o_body); J.hbufF = traceback ? nullptr : (int*)(d + o_body + row); J.hb_stride = 0;
+    J.ckvH = nullptr; J.ckvE = nullptr;
+    J.progress = (int*)(d + o_pr); J.ticket = (int*)d;
+    J.best = (unsigned long long*)(d + 8); J.corner = (int*)(d + 16);
+    J.col0 = 0; J.n_total = n; J.row_off = 0; J.start_type = -1; J.end_type = -1;
+    P.bk.B = Band{m, n, bw};
+    P.bk.tile_base = traceback ? (long long*)(d + o_body) : nullptr;
+    P.bk.rec = traceback ? (int*)(d + o_body + up256((size_t)NB * 8)) : nullptr;
+    if (traceback) {
+        psa_banded_tile_base_kernel<<<1, 1024, 0, st>>>(P.bk.B, P.bk.tile_base);
+        PSA_CUDA_OK(ctx, cudaGetLastError());
+        ctx->launches += 1;
+    }
+    const void* fill;
+    if (traceback) fill = local ? (const void*)psa_banded_pair_fill_kernel<PSA_LOCAL, K, true> : (const void*)psa_banded_pair_fill_kernel<PSA_GLOBAL, K, true>;
+    else if (KK == 16) fill = local ? (const void*)psa_banded_pair_fill_kernel<PSA_LOCAL, 16, false> : (const void*)psa_banded_pair_fill_kernel<PSA_GLOBAL, 16, false>;
+    else fill = local ? (const void*)psa_banded_pair_fill_kernel<PSA_LOCAL, 4, false> : (const void*)psa_banded_pair_fill_kernel<PSA_GLOBAL, 4, false>;
+    int per_sm = 0;
+    PSA_CUDA_OK(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fill, WPB * 32, 0));
+    if (ctx->opt.long_ctas_per_sm > 0) per_sm = std::max(1, std::min(per_sm, ctx->opt.long_ctas_per_sm));
+    else if (per_sm > 4) per_sm = 4;
+    // about tpr row blocks are in flight at once; twice as many warps keep the next ones waiting at their first strip
+    const long long warps = std::min(NB, 2 * tpr + 4);
+    const int grid = (int)std::max(1LL, std::min((warps + WPB - 1) / WPB, (long long)per_sm * ctx->sm_count));
+    void* fargs[] = {&P};
+    PSA_CUDA_OK(ctx, cudaLaunchKernel(fill, dim3(grid), dim3(WPB * 32), fargs, 0, st));
+    ctx->launches += 1;
+    BandedPairTb T{J, P.bk, traceback ? (uint32_t*)(d + o_body + ck) : nullptr, (int)tpr, 0, (int)NB,
+                   (BandedWalk*)(d + 64), d_item, traceback ? d_ops : nullptr};
+    if (!traceback) {
+        if (local) psa_banded_pair_walk_kernel<PSA_LOCAL><<<1, 32, 0, st>>>(T);
+        else psa_banded_pair_walk_kernel<PSA_GLOBAL><<<1, 32, 0, st>>>(T);
+        PSA_CUDA_OK(ctx, cudaGetLastError());
+        ctx->launches += 1;
+        return PSA_OK;
+    }
+    for (long long hi = NB; hi > 0; hi -= rpw) {
+        T.rb_hi = (int)hi; T.rb_lo = (int)std::max(0LL, hi - rpw);
+        const long long units = (long long)(T.rb_hi - T.rb_lo) * tpr;
+        const unsigned blocks = (unsigned)((units + CODES_WPB - 1) / CODES_WPB);
+        if (local) {
+            psa_banded_pair_codes_kernel<PSA_LOCAL><<<blocks, CODES_WPB * 32, 0, st>>>(T);
+            psa_banded_pair_walk_kernel<PSA_LOCAL><<<1, 32, 0, st>>>(T);
+        } else {
+            psa_banded_pair_codes_kernel<PSA_GLOBAL><<<blocks, CODES_WPB * 32, 0, st>>>(T);
+            psa_banded_pair_walk_kernel<PSA_GLOBAL><<<1, 32, 0, st>>>(T);
         }
         PSA_CUDA_OK(ctx, cudaGetLastError());
         ctx->launches += 2;

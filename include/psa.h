@@ -238,6 +238,31 @@ int psa_align_long_device(psa_ctx* ctx, const uint8_t* d_a, const uint8_t* d_b, 
                           int h, unsigned flags, psa_batch_item* d_item, uint32_t* d_ops, size_t ops_words,
                           void* cuda_stream);
 
+/* ---- one banded pair over the whole GPU ------------------------------------------------------
+ * One pair inside the diagonal band of psa_align_batch_banded (|j - floor(i*n/m)| <= band), computed by every SM: the
+ * row blocks of the banded tile kernels run as a wavefront over all resident warps (progress counters per strip), and
+ * the traceback walk is fed by a parallel recompute of the band tiles it can still reach.  Results are a one-pair
+ * psa_align_batch_banded's, byte for byte: the same record and op words, the same no-path record in global mode
+ * (PSA_NEG_INF corners, end state 1, aln_len 0, no op words written), and with band >= max(m, n) those of
+ * psa_align_pair / psa_align_long_device.  flags: PSA_WANT_SCORE and PSA_WANT_TRACEBACK only; band < 0 or any other
+ * flag is PSA_ERR_ARG; lengths >= 2^21 - 1 are PSA_ERR_RANGE.  With traceback the fill keeps tile checkpoints of at most
+ * 3 KiB x min(NB*S, (n + 2*bw*NB)/256 + 2*NB) bytes (NB = ceil(m/128), S = ceil(n/256), bw = min(band, m + n)) plus a
+ * code buffer of at most 256 MiB; if they exceed half of the free device memory the call fails with PSA_ERR_NOMEM.
+ *
+ * psa_align_pair_banded: host strings; fills *out as psa_align_pair does (m = 0 or n = 0: psa_align_pair's record).
+ * psa_align_long_banded_device: sequences in device memory, m, n >= 1, psa_align_long_device's null / capacity rules
+ * (ops_words >= ceil((m+n)/16) with traceback).  Asynchronous on cuda_stream (NULL = the context's stream); the plan
+ * is a function of (m, n, band, mode, flags) alone, nothing is read back, and the call issues
+ *     score only:  2 kernel launches (fill, record)
+ *     traceback:   2 + 2 * ceil(NB / rpw) launches (tile offsets, fill, then a recompute and a walk per window), with
+ *                  rpw = min(NB, max(1, floor(2^28 / (tpr * 16384)))),
+ *                  tpr = min(S, floor((2*bw + floor(128*n/m) + 2) / 256) + 2). */
+int psa_align_pair_banded(psa_ctx* ctx, const char* a, const char* b, size_t m, size_t n, int mode, int g, int h,
+                          int band, unsigned flags, psa_result* out);
+int psa_align_long_banded_device(psa_ctx* ctx, const uint8_t* d_a, const uint8_t* d_b, size_t m, size_t n, int mode,
+                                 int g, int h, int band, unsigned flags, psa_batch_item* d_item, uint32_t* d_ops,
+                                 size_t ops_words, void* cuda_stream);
+
 /* ---- one long pair over several GPUs (config 4) ---------------------------------------------
  * Score-only fill of ONE pair by the column-stationary systolic kernel: the matrix is cut into panels of
  * panel_strips * psa_long_strip_columns() columns (one warp per strip -- 256 columns, 8 per lane -- every strip
