@@ -41,6 +41,22 @@ int check_scoring(psa_ctx* ctx, int mode, int g, int h, int64_t max_m, int64_t m
     return PSA_OK;
 }
 
+// check_scoring for the banded entries.  Its bound counts three gap openings, which holds for the full matrix only: a
+// band can force an opening on every row (n = 3m at band 1 needs a horizontal run of 2 per row).  An optimal path never
+// puts a vertical run next to a horizontal one (one diagonal step replaces the corner, inside the band, for 2g less and
+// a match or nothing), so its gap runs are separated by diagonals: at most min(m, n) + 1 of them, one more for a T2 / T3
+// value that ends in a gap and one for the border run.  Global mode with band < max(m, n) therefore admits
+// g(m+n+2) + h(min(m, n) + 3) + m + n < 2^28, which keeps out_value's threshold argument (psa_result.cuh) true.  Local
+// values never fall below -(g+h), a band >= max(m, n) holds every cell and an empty side leaves no cell for the band
+// to cut: those keep check_scoring's bound.  A batch is checked with its largest m and n.
+int check_banded_scoring(psa_ctx* ctx, int mode, int g, int h, int band, int64_t max_m, int64_t max_n) {
+    int rc = check_scoring(ctx, mode, g, h, max_m, max_n);
+    if (rc || mode != PSA_GLOBAL || band >= std::max(max_m, max_n) || std::min(max_m, max_n) == 0) return rc;
+    const int64_t span = (int64_t)g * (max_m + max_n + 2) + (int64_t)h * (std::min(max_m, max_n) + 3) + max_m + max_n;
+    if (span >= (1 << 28)) return psa_fail(ctx, PSA_ERR_RANGE, "banded score range exceeds int32 lanes");
+    return PSA_OK;
+}
+
 int dispatch_batch(psa_ctx* ctx, const psa_batch_args& args, int max_m, int max_n, int mode, unsigned flags,
                    cudaStream_t stream) {
     const bool tb = (flags & PSA_WANT_TRACEBACK) != 0;
@@ -261,7 +277,7 @@ static int align_batch_host(psa_ctx* ctx, const uint8_t* bases_a, const int64_t*
                     return psa_fail(ctx, PSA_ERR_ARG, "pair " + std::to_string(k) + ": offset/length outside the base arrays");
         }
     }
-    int rc = check_scoring(ctx, mode, g, h, max_m, max_n);
+    int rc = band >= 0 ? check_banded_scoring(ctx, mode, g, h, band, max_m, max_n) : check_scoring(ctx, mode, g, h, max_m, max_n);
     if (rc) return rc;
     if (tb && ops_stride_words * 16 < (size_t)max_m + max_n)
         return psa_fail(ctx, PSA_ERR_CAPACITY, "ops_stride_words < ceil((max m + max n)/16)");
@@ -388,7 +404,7 @@ int psa_align_batch_banded_device(psa_ctx* ctx, const uint8_t* d_bases_a, const 
     if (!d_bases_a || !d_bases_b || !d_off_a || !d_off_b || !d_len_a || !d_len_b || !d_items)
         return psa_fail(ctx, PSA_ERR_ARG, "null device pointer");
     if (max_len_a < 0 || max_len_b < 0) return psa_fail(ctx, PSA_ERR_ARG, "negative length bound");
-    int rc = check_scoring(ctx, mode, g, h, max_len_a, max_len_b);
+    int rc = check_banded_scoring(ctx, mode, g, h, band, max_len_a, max_len_b);
     if (rc) return rc;
     const bool tb = (flags & PSA_WANT_TRACEBACK) != 0;
     if (tb && !d_ops) return psa_fail(ctx, PSA_ERR_ARG, "traceback requested without an ops buffer");
@@ -410,7 +426,7 @@ static int check_banded_pair(psa_ctx* ctx, size_t m, size_t n, int mode, int g, 
     if (band < 0) return psa_fail(ctx, PSA_ERR_ARG, "band must be >= 0");
     if (flags & ~(PSA_WANT_SCORE | PSA_WANT_TRACEBACK)) return psa_fail(ctx, PSA_ERR_ARG, "flags: PSA_WANT_SCORE and PSA_WANT_TRACEBACK only");
     if (m >= 0x1FFFFF || n >= 0x1FFFFF) return psa_fail(ctx, PSA_ERR_RANGE, "long path: lengths must be < 2^21 - 1");
-    return check_scoring(ctx, mode, g, h, (int64_t)m, (int64_t)n);
+    return check_banded_scoring(ctx, mode, g, h, band, (int64_t)m, (int64_t)n);
 }
 
 int psa_align_long_banded_device(psa_ctx* ctx, const uint8_t* d_a, const uint8_t* d_b, size_t m, size_t n, int mode, int g,

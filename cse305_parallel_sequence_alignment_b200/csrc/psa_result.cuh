@@ -7,11 +7,13 @@
 __device__ __forceinline__ int imax(int a, int b) { return a > b ? a : b; }
 
 // The in-kernel sentinel (and anything that drifted from it) is the ABI's -infinity.  The threshold is -3 * 2^27.
-// check_scoring admits span = g(m+n+2) + 2h + m + n < 2^28.  A finite value needs at most three gap openings (a start
-// type forces the first gap, an orthogonal gap follows, and the end state needs one more) and at most m + n gap
-// columns, so it is >= -(3h + g(m+n)) > -1.5 * span > -3 * 2^27.  A value that descends from the sentinel gains at
-// most +1 per diagonal step, so it is <= PSA_KNEG + min(m, n) < -2^29 + 2^27 = -3 * 2^27.  The old threshold
-// PSA_KNEG / 2 = -2^28 cut off finite typed corners such as -3h + 113 at g = 0, h = 134 217 577.
+// check_scoring admits span = g(m+n+2) + 2h + m + n < 2^28.  In the full matrix a finite value needs at most three gap
+// openings (a start type forces the first gap, an orthogonal gap follows, and the end state needs one more) and at most
+// m + n gap columns, so it is >= -(3h + g(m+n)) > -1.5 * span > -3 * 2^27.  A band can force an opening on every row:
+// banded global calls are held to check_banded_scoring's g(m+n+2) + h(min(m, n) + 3) + m + n < 2^28 (psa_capi.cu),
+// which keeps them >= -2^28.  A value that descends from the sentinel gains at most +1 per diagonal step, so it is
+// <= PSA_KNEG + min(m, n) < -2^29 + 2^27 = -3 * 2^27.  The old threshold PSA_KNEG / 2 = -2^28 cut off finite typed
+// corners such as -3h + 113 at g = 0, h = 134 217 577.
 __device__ __forceinline__ int out_value(int v) { return v < PSA_KNEG / 4 * 3 ? PSA_NEG_INF : v; }
 
 // End state of a global alignment (find_alignment, cpp:112-146): forced by a positive end type, else the first of

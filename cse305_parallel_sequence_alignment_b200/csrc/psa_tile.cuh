@@ -124,12 +124,15 @@ struct ColsS {
     int ff[K];    // F[i-1][j]
     int H[K];     // H form only: H[i-1][j]
     int b[K];
-    int ka[K];    // local mode: key addend KM-1-k (TF form: + (g+h)*KM, its key is built from T1 - (g+h)), or a large
-                  // negative number for padding columns (j > n)
+    int ka[K];    // local mode: key addend KM-1-k, or -2^30 for padding columns (j > n); TF form: + (g+h)*KM, its key is
+                  // built from T1 - (g+h).  A padding key is then T1*KM - 2^30 < 0.  Without the + (g+h)*KM there,
+                  // (T1 - (g+h))*KM - 2^30 wrapped to a large positive key once (g+h)*KM > 2^30 (local mode admits g+h up
+                  // to about 2^27): it outranked the real columns of the lane holding column n, and the lane's best was
+                  // then dropped as lying past n.
     __device__ __forceinline__ void set_top(int k, int H0, int F0, int go) { hg[k] = H0 - go; ff[k] = F0; if (!tf_form(K)) H[k] = H0; }
     __device__ __forceinline__ int top_H(int k, int go) const { return tf_form(K) ? hg[k] + go : H[k]; }
     __device__ __forceinline__ void set_key_addend(int k, bool real, int go) {
-        ka[k] = real ? (key_mult(K) - 1 - k) + (tf_form(K) ? go * key_mult(K) : 0) : -(1 << 30);
+        ka[k] = (real ? key_mult(K) - 1 - k : -(1 << 30)) + (tf_form(K) ? go * key_mult(K) : 0);
     }
 };
 

@@ -182,6 +182,10 @@ int psa_align_batch_device(psa_ctx* ctx, const uint8_t* d_bases_a, const int64_t
  * For similar sequences (reads against their source window, overlaps, polishing) the fill and the traceback
  * checkpoints shrink from m*n to about m*(2*band + 1) cells.  Same buffer layouts, op-word format and capacity rule as
  * psa_align_batch; flags: PSA_WANT_SCORE and PSA_WANT_TRACEBACK only (anything else: PSA_ERR_ARG); lengths < 2^21 - 1.
+ * Score range: a band can force a gap opening on every row, so a global call with band < max(M, N) and M, N >= 1
+ * (M, N = the largest lengths of the call) needs g(M+N+2) + h(min(M, N) + 3) + M + N < 2^28, else PSA_ERR_RANGE
+ * ("banded score range exceeds int32 lanes").  Local calls and bands >= max(M, N) keep psa_align_batch's
+ * g(M+N+2) + 2h + M + N < 2^28.  At g = 0 a 1 Mbp x 1 Mbp global pair admits h <= 266.
  * Every pair runs on the banded long-pair kernels, one warp per pair: short pairs are correct but gain nothing from
  * the band over psa_align_batch.  The device form is asynchronous on cuda_stream (NULL = the context's stream) and
  * plans its work from n_pairs, max_len_a, max_len_b and band alone. */
@@ -245,7 +249,8 @@ int psa_align_long_device(psa_ctx* ctx, const uint8_t* d_a, const uint8_t* d_b, 
  * psa_align_batch_banded's, byte for byte: the same record and op words, the same no-path record in global mode
  * (PSA_NEG_INF corners, end state 1, aln_len 0, no op words written), and with band >= max(m, n) those of
  * psa_align_pair / psa_align_long_device.  flags: PSA_WANT_SCORE and PSA_WANT_TRACEBACK only; band < 0 or any other
- * flag is PSA_ERR_ARG; lengths >= 2^21 - 1 are PSA_ERR_RANGE.  With traceback the fill keeps tile checkpoints of at most
+ * flag is PSA_ERR_ARG; lengths >= 2^21 - 1 are PSA_ERR_RANGE, and so are (g, h) outside psa_align_batch_banded's score
+ * range rule (global with band < max(m, n): g(m+n+2) + h(min(m, n) + 3) + m + n < 2^28).  With traceback the fill keeps tile checkpoints of at most
  * 3 KiB x min(NB*S, (n + 2*bw*NB)/256 + 2*NB) bytes (NB = ceil(m/128), S = ceil(n/256), bw = min(band, m + n)) plus a
  * code buffer of at most 256 MiB; if they exceed half of the free device memory the call fails with PSA_ERR_NOMEM.
  *
