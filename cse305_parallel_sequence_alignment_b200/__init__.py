@@ -5,7 +5,7 @@ Python doorway used by the tests, bench.py and __graft_entry__: it loads the sha
 ctypes and fails loudly if the library or a CUDA device is missing -- there is no CPU fallback.
 """
 from .capi import (GLOBAL, LOCAL, WANT_SCORE, WANT_TRACEBACK, OPS_COMPACT, compact_ops_offsets, BatchItem, Context, PsaError, build_library,
-                   library_path, load_library, pack_pairs, unpack_ops, render_rows, pack_bases, pack_reads, pack_reads_2bit)
+                   library_path, load_library, pack_anchors, pack_pairs, unpack_ops, render_rows, pack_bases, pack_reads, pack_reads_2bit)
 
 __all__ = ["GLOBAL", "LOCAL", "WANT_SCORE", "WANT_TRACEBACK", "OPS_COMPACT", "compact_ops_offsets", "BatchItem", "Context", "PsaError",
-           "build_library", "library_path", "load_library", "pack_pairs", "unpack_ops", "render_rows", "pack_bases", "pack_reads", "pack_reads_2bit"]
+           "build_library", "library_path", "load_library", "pack_anchors", "pack_pairs", "unpack_ops", "render_rows", "pack_bases", "pack_reads", "pack_reads_2bit"]

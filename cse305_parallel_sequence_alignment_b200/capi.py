@@ -129,6 +129,15 @@ def load_library() -> C.CDLL:
     lib.psa_align_long_banded_device.restype = C.c_int
     lib.psa_align_long_banded_device.argtypes = [vp, vp, vp, C.c_size_t, C.c_size_t, C.c_int, C.c_int, C.c_int, C.c_int, C.c_uint,
                                                  vp, vp, C.c_size_t, vp]
+    lib.psa_align_batch_guided.restype = C.c_int
+    lib.psa_align_batch_guided.argtypes = [vp, vp, vp, vp, vp, vp, vp, C.c_size_t, C.c_size_t, C.c_size_t, vp, vp, vp, C.c_size_t,
+                                           C.c_int, C.c_int, C.c_int, C.c_int, C.c_uint, vp, vp, C.c_size_t]
+    lib.psa_align_batch_guided_device.restype = C.c_int
+    lib.psa_align_batch_guided_device.argtypes = [vp, vp, vp, vp, vp, vp, vp, C.c_size_t, C.c_int, C.c_int, vp, vp, vp, C.c_int,
+                                                  C.c_int, C.c_int, C.c_int, C.c_uint, vp, vp, C.c_size_t, vp]
+    lib.psa_align_pair_guided.restype = C.c_int
+    lib.psa_align_pair_guided.argtypes = [vp, C.c_char_p, C.c_char_p, C.c_size_t, C.c_size_t, vp, C.c_size_t, C.c_int, C.c_int,
+                                          C.c_int, C.c_int, C.c_uint, C.POINTER(_Result)]
     lib.psa_xbuf_bytes.restype = C.c_size_t
     lib.psa_xbuf_bytes.argtypes = [C.c_size_t]
     lib.psa_xbuf_create.restype = C.c_int
@@ -157,7 +166,8 @@ def load_library() -> C.CDLL:
 
 
 EXPORTS = ["psa_ctx_create", "psa_ctx_destroy", "psa_last_error", "psa_launch_count", "psa_align_pair", "psa_align_pair_typed", "psa_align_partition", "psa_align_long_partitioned", "psa_similarity_batch", "psa_similarity_batch_device",
-           "psa_result_free", "psa_align_batch", "psa_align_batch_device", "psa_align_batch_banded", "psa_align_batch_banded_device", "psa_pack_bases", "psa_pack_reads", "psa_align_batch_packed", "psa_align_long_device", "psa_align_pair_banded", "psa_align_long_banded_device", "psa_xbuf_bytes", "psa_xbuf_create", "psa_xbuf_open", "psa_xbuf_close",
+           "psa_result_free", "psa_align_batch", "psa_align_batch_device", "psa_align_batch_banded", "psa_align_batch_banded_device", "psa_pack_bases", "psa_pack_reads", "psa_align_batch_packed", "psa_align_long_device", "psa_align_pair_banded", "psa_align_long_banded_device",
+           "psa_align_batch_guided", "psa_align_batch_guided_device", "psa_align_pair_guided", "psa_xbuf_bytes", "psa_xbuf_create", "psa_xbuf_open", "psa_xbuf_close",
            "psa_xbuf_destroy", "psa_long_panel_strips", "psa_long_strip_columns", "psa_align_long_cyclic_device", "psa_ops_unpack", "psa_render_rows",
            "psa_peak_int_ops"]
 
@@ -214,6 +224,20 @@ def compact_ops_offsets(items: np.ndarray) -> np.ndarray:
     out = np.zeros(len(items) + 1, dtype=np.int64)
     np.cumsum(words, out=out[1:])
     return out
+
+
+def pack_anchors(anchors: Sequence) -> tuple:
+    """Per-pair anchor chains ((K_k, 2) arrays of (i, j), or lists of pairs) -> (psa_anchor array [total, 2] int32,
+    int64 offsets, int32 counts), the layout psa_align_batch_guided takes."""
+    chains = [np.asarray(c, dtype=np.int64).reshape(-1, 2) for c in anchors]
+    cnt = np.array([len(c) for c in chains], dtype=np.int32)
+    off = np.zeros(len(chains), dtype=np.int64)
+    if len(chains) > 1:
+        np.cumsum(cnt[:-1], out=off[1:])
+    flat = np.concatenate(chains) if chains and cnt.sum() else np.zeros((0, 2), np.int64)
+    if flat.size and (flat.min() < -2 ** 31 or flat.max() >= 2 ** 31):
+        raise ValueError("anchor coordinates must fit int32")
+    return np.ascontiguousarray(flat, dtype=np.int32), off, cnt
 
 
 def unpack_ops(words: np.ndarray, aln_len: int) -> bytes:
@@ -433,6 +457,63 @@ class Context:
         self._check(self._lib.psa_align_batch_banded_device(
             self._h, d_bases_a, d_off_a, d_len_a, d_bases_b, d_off_b, d_len_b, n_pairs, max_len_a, max_len_b,
             mode, g, h, band, flags, d_items, d_ops or None, ops_stride_words, stream or None))
+
+    def align_batch_guided(self, bases_a: np.ndarray, off_a: np.ndarray, len_a: np.ndarray, bases_b: np.ndarray,
+                           off_b: np.ndarray, len_b: np.ndarray, anchors: Sequence, band: int, mode: int = GLOBAL, g: int = 1,
+                           h: int = 2, traceback: bool = True, ops: Optional[np.ndarray] = None, flags: Optional[int] = None):
+        """psa_align_batch_guided: align_batch_banded with each pair's band around its anchor chain; anchors[k] is pair k's
+        chain, a (K_k, 2) array of (i, j).  Returns (items, ops words [n_pairs, stride] or None)."""
+        n = len(len_a)
+        bases_a = np.ascontiguousarray(bases_a, dtype=np.uint8)
+        bases_b = np.ascontiguousarray(bases_b, dtype=np.uint8)
+        off_a = np.ascontiguousarray(off_a, dtype=np.int64)
+        off_b = np.ascontiguousarray(off_b, dtype=np.int64)
+        len_a = np.ascontiguousarray(len_a, dtype=np.int32)
+        len_b = np.ascontiguousarray(len_b, dtype=np.int32)
+        anc, off_anc, n_anc = pack_anchors(anchors)
+        if len(n_anc) != n:
+            raise ValueError("one anchor chain per pair")
+        items = np.zeros(n, dtype=ITEM_DTYPE)
+        stride = 0
+        if traceback:
+            if ops is None:
+                stride = (int(len_a.max(initial=0)) + int(len_b.max(initial=0)) + 15) // 16 + 1
+                ops = np.zeros((n, stride), dtype=np.uint32)
+            stride = ops.shape[1]
+        if flags is None:
+            flags = WANT_SCORE | (WANT_TRACEBACK if traceback else 0)
+        self._check(self._lib.psa_align_batch_guided(
+            self._h, bases_a.ctypes.data, off_a.ctypes.data, len_a.ctypes.data, bases_b.ctypes.data,
+            off_b.ctypes.data, len_b.ctypes.data, n, bases_a.size, bases_b.size, anc.ctypes.data if len(anc) else None,
+            off_anc.ctypes.data, n_anc.ctypes.data, len(anc), mode, g, h, band, flags,
+            items.ctypes.data, ops.ctypes.data if traceback else None, stride))
+        return items, (ops if traceback else None)
+
+    def align_batch_guided_device(self, d_bases_a: int, d_off_a: int, d_len_a: int, d_bases_b: int, d_off_b: int,
+                                  d_len_b: int, n_pairs: int, max_len_a: int, max_len_b: int, d_anchors: int, d_off_anc: int,
+                                  d_n_anc: int, band: int, d_items: int, d_ops: int = 0, ops_stride_words: int = 0,
+                                  mode: int = GLOBAL, g: int = 1, h: int = 2, traceback: bool = True, stream: int = 0,
+                                  flags: Optional[int] = None):
+        """psa_align_batch_guided_device: raw device pointers / cudaStream_t; anchors as pack_anchors lays them out.  A pair
+        whose chain is invalid gets the rejected record (end_state 0)."""
+        if flags is None:
+            flags = WANT_SCORE | (WANT_TRACEBACK if traceback else 0)
+        self._check(self._lib.psa_align_batch_guided_device(
+            self._h, d_bases_a, d_off_a, d_len_a, d_bases_b, d_off_b, d_len_b, n_pairs, max_len_a, max_len_b,
+            d_anchors or None, d_off_anc or None, d_n_anc or None, mode, g, h, band, flags, d_items, d_ops or None,
+            ops_stride_words, stream or None))
+
+    def align_pair_guided(self, a: bytes, b: bytes, anchors, band: int, mode: int = GLOBAL, g: int = 1, h: int = 2,
+                          traceback: bool = True, flags: Optional[int] = None) -> PairResult:
+        """psa_align_pair_guided: one pair inside the band around its anchor chain ((K, 2) array of (i, j)), over the whole
+        GPU."""
+        anc, _, cnt = pack_anchors([anchors])
+        res = _Result()
+        if flags is None:
+            flags = WANT_SCORE | (WANT_TRACEBACK if traceback else 0)
+        self._check(self._lib.psa_align_pair_guided(self._h, a, b, len(a), len(b), anc.ctypes.data if len(anc) else None,
+                                                    int(cnt[0]), mode, g, h, band, flags, C.byref(res)))
+        return self._take(res, traceback)
 
     def align_long_device(self, d_a: int, d_b: int, m: int, n: int, d_item: int, d_ops: int = 0, ops_words: int = 0,
                           mode: int = GLOBAL, g: int = 1, h: int = 2, traceback: bool = False, stream: int = 0):

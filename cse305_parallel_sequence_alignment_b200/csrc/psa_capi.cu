@@ -48,12 +48,32 @@ int check_scoring(psa_ctx* ctx, int mode, int g, int h, int64_t max_m, int64_t m
 // value that ends in a gap and one for the border run.  Global mode with band < max(m, n) therefore admits
 // g(m+n+2) + h(min(m, n) + 3) + m + n < 2^28, which keeps out_value's threshold argument (psa_result.cuh) true.  Local
 // values never fall below -(g+h), a band >= max(m, n) holds every cell and an empty side leaves no cell for the band
-// to cut: those keep check_scoring's bound.  A batch is checked with its largest m and n.
+// to cut: those keep check_scoring's bound.  A batch is checked with its largest m and n.  The argument uses only that
+// a corner's two end cells are in the band, so it covers the bands of anchor chains (psa_align_batch_guided) as well.
 int check_banded_scoring(psa_ctx* ctx, int mode, int g, int h, int band, int64_t max_m, int64_t max_n) {
     int rc = check_scoring(ctx, mode, g, h, max_m, max_n);
     if (rc || mode != PSA_GLOBAL || band >= std::max(max_m, max_n) || std::min(max_m, max_n) == 0) return rc;
     const int64_t span = (int64_t)g * (max_m + max_n + 2) + (int64_t)h * (std::min(max_m, max_n) + 3) + max_m + max_n;
     if (span >= (1 << 28)) return psa_fail(ctx, PSA_ERR_RANGE, "banded score range exceeds int32 lanes");
+    return PSA_OK;
+}
+
+// The host forms' chain check (psa_align_batch_guided, psa_align_pair_guided): pair k's anchors
+// anchors[off[k] .. off[k] + cnt[k]) lie inside the array and form a valid chain for its lengths (include/psa.h).
+int check_chains(psa_ctx* ctx, const psa_anchor* anchors, const int64_t* off, const int32_t* cnt, size_t total,
+                 const int32_t* len_a, const int32_t* len_b, size_t n_pairs) {
+    for (size_t k = 0; k < n_pairs; ++k) {
+        const std::string pair = "pair " + std::to_string(k) + ": ";
+        if (cnt[k] < 0 || off[k] < 0 || (uint64_t)off[k] + (uint64_t)cnt[k] > total)
+            return psa_fail(ctx, PSA_ERR_ARG, pair + "anchor range outside the anchor array");
+        const psa_anchor* c = anchors + off[k];
+        for (int32_t q = 0; q < cnt[k]; ++q) {
+            if (c[q].i < 0 || c[q].i > len_a[k] || c[q].j < 0 || c[q].j > len_b[k])
+                return psa_fail(ctx, PSA_ERR_ARG, pair + "anchor " + std::to_string(q) + " outside the matrix");
+            if (q > 0 && (c[q].i < c[q - 1].i || c[q].j < c[q - 1].j))
+                return psa_fail(ctx, PSA_ERR_ARG, pair + "anchor " + std::to_string(q) + " decreases a coordinate of the chain");
+        }
+    }
     return PSA_OK;
 }
 
@@ -221,12 +241,13 @@ int psa_align_batch_device(psa_ctx* ctx, const uint8_t* d_bases_a, const int64_t
 constexpr int kLongTbBatchMin = 16;
 
 // Host-buffer batch with an optional border variant per call or per pair; psa_align_batch is the -1/-1 case.
-// band >= 0: psa_align_batch_banded (every pair on the banded kernels).
+// band >= 0: psa_align_batch_banded (every pair on the banded kernels); with guide (host arrays of total_anc anchors)
+// psa_align_batch_guided.
 static int align_batch_host(psa_ctx* ctx, const uint8_t* bases_a, const int64_t* off_a, const int32_t* len_a,
                             const uint8_t* bases_b, const int64_t* off_b, const int32_t* len_b, size_t n_pairs,
                             size_t bytes_a, size_t bytes_b, int mode, int g, int h, unsigned flags,
                             psa_batch_item* items, uint32_t* ops, size_t ops_stride_words, const psa_piece_types& ty,
-                            int band = -1) {
+                            int band = -1, const psa_guide* guide = nullptr, size_t total_anc = 0) {
     if (!ctx) return PSA_ERR_ARG;
     if (n_pairs == 0) return PSA_OK;
     if (!off_a || !off_b || !len_a || !len_b || !items || (!bases_a && bytes_a) || (!bases_b && bytes_b))
@@ -279,6 +300,11 @@ static int align_batch_host(psa_ctx* ctx, const uint8_t* bases_a, const int64_t*
     }
     int rc = band >= 0 ? check_banded_scoring(ctx, mode, g, h, band, max_m, max_n) : check_scoring(ctx, mode, g, h, max_m, max_n);
     if (rc) return rc;
+    if (guide) {
+        if (!guide->off || !guide->n || (!guide->anchors && total_anc)) return psa_fail(ctx, PSA_ERR_ARG, "null anchor array");
+        rc = check_chains(ctx, guide->anchors, guide->off, guide->n, total_anc, len_a, len_b, n_pairs);
+        if (rc) return rc;
+    }
     if (tb && ops_stride_words * 16 < (size_t)max_m + max_n)
         return psa_fail(ctx, PSA_ERR_CAPACITY, "ops_stride_words < ceil((max m + max n)/16)");
     PSA_CUDA_OK(ctx, cudaSetDevice(ctx->device));
@@ -296,6 +322,10 @@ static int align_batch_host(psa_ctx* ctx, const uint8_t* bases_a, const int64_t*
     const size_t o_it = o; o = align_up(o + n_pairs * sizeof(psa_batch_item), 256);
     const size_t o_op = o; o = align_up(o + (tb ? n_pairs * ops_stride_words * 4 : 0), 256);
     const size_t o_ty = o; o = align_up(o + (ty.per_pair ? n_pairs : 0), 256);
+    // guided: [anchors | off_anc | n_anc]
+    const size_t o_an = o; o = align_up(o + (guide ? total_anc * sizeof(psa_anchor) : 0), 256);
+    const size_t o_ao = o; o = align_up(o + (guide ? n_pairs * 8 : 0), 256);
+    const size_t o_ac = o; o = align_up(o + (guide ? n_pairs * 4 : 0), 256);
     rc = ensure_scratch(ctx, o);
     if (rc) return rc;
     uint8_t* d = (uint8_t*)ctx->d_scratch;
@@ -330,6 +360,12 @@ static int align_batch_host(psa_ctx* ctx, const uint8_t* bases_a, const int64_t*
     PSA_CUDA_OK(ctx, cudaMemcpyAsync(d + o_ob, off_b, n_pairs * 8, cudaMemcpyHostToDevice, st));
     PSA_CUDA_OK(ctx, cudaMemcpyAsync(d + o_la, len_a, n_pairs * 4, cudaMemcpyHostToDevice, st));
     PSA_CUDA_OK(ctx, cudaMemcpyAsync(d + o_lb, len_b, n_pairs * 4, cudaMemcpyHostToDevice, st));
+    const psa_guide d_guide{(const psa_anchor*)(d + o_an), (const int64_t*)(d + o_ao), (const int32_t*)(d + o_ac)};
+    if (guide) {
+        if (total_anc) PSA_CUDA_OK(ctx, cudaMemcpyAsync(d + o_an, guide->anchors, total_anc * sizeof(psa_anchor), cudaMemcpyHostToDevice, st));
+        PSA_CUDA_OK(ctx, cudaMemcpyAsync(d + o_ao, guide->off, n_pairs * 8, cudaMemcpyHostToDevice, st));
+        PSA_CUDA_OK(ctx, cudaMemcpyAsync(d + o_ac, guide->n, n_pairs * 4, cudaMemcpyHostToDevice, st));
+    }
     const bool is_short = psa_short_supported(max_m, max_n, tb);
     if (typed && mode != PSA_GLOBAL) return psa_fail(ctx, PSA_ERR_ARG, "start/end types apply to global alignment only");
     // long pairs with traceback: from kLongTbBatchMin pairs on, one warp per pair (checkpointed batch fill + batched walk)
@@ -340,7 +376,7 @@ static int align_batch_host(psa_ctx* ctx, const uint8_t* bases_a, const int64_t*
         if (rc) return rc;
     }
     if (band >= 0) {
-        rc = psa_launch_banded(ctx, args, max_m, max_n, mode, band, tb, st);
+        rc = psa_launch_banded(ctx, args, max_m, max_n, mode, band, tb, st, guide ? &d_guide : nullptr);
         if (rc) return rc;
     } else if (is_short || (!typed && !tb && n_pairs > 8) || tb_chunk > 0) {
         rc = dispatch_batch(ctx, args, max_m, max_n, mode, flags, st);
@@ -417,6 +453,49 @@ int psa_align_batch_banded_device(psa_ctx* ctx, const uint8_t* d_bases_a, const 
     rc = psa_stream_enter(ctx, st);
     if (rc) return rc;
     rc = psa_launch_banded(ctx, args, max_len_a, max_len_b, mode, band, tb, st);
+    if (rc) return rc;
+    return psa_stream_leave(ctx, st);
+}
+
+int psa_align_batch_guided(psa_ctx* ctx, const uint8_t* bases_a, const int64_t* off_a, const int32_t* len_a,
+                           const uint8_t* bases_b, const int64_t* off_b, const int32_t* len_b, size_t n_pairs,
+                           size_t bytes_a, size_t bytes_b, const psa_anchor* anchors, const int64_t* off_anc,
+                           const int32_t* n_anc, size_t total_anc, int mode, int g, int h, int band, unsigned flags,
+                           psa_batch_item* items, uint32_t* ops, size_t ops_stride_words) {
+    if (!ctx) return PSA_ERR_ARG;
+    if (band < 0) return psa_fail(ctx, PSA_ERR_ARG, "band must be >= 0");
+    if (flags & ~(PSA_WANT_SCORE | PSA_WANT_TRACEBACK)) return psa_fail(ctx, PSA_ERR_ARG, "flags: PSA_WANT_SCORE and PSA_WANT_TRACEBACK only");
+    const psa_guide guide{anchors, off_anc, n_anc};
+    return align_batch_host(ctx, bases_a, off_a, len_a, bases_b, off_b, len_b, n_pairs, bytes_a, bytes_b, mode, g, h, flags,
+                            items, ops, ops_stride_words, psa_piece_types{}, band, &guide, total_anc);
+}
+
+int psa_align_batch_guided_device(psa_ctx* ctx, const uint8_t* d_bases_a, const int64_t* d_off_a, const int32_t* d_len_a,
+                                  const uint8_t* d_bases_b, const int64_t* d_off_b, const int32_t* d_len_b, size_t n_pairs,
+                                  int max_len_a, int max_len_b, const psa_anchor* d_anchors, const int64_t* d_off_anc,
+                                  const int32_t* d_n_anc, int mode, int g, int h, int band, unsigned flags,
+                                  psa_batch_item* d_items, uint32_t* d_ops, size_t ops_stride_words, void* cuda_stream) {
+    if (!ctx) return PSA_ERR_ARG;
+    if (band < 0) return psa_fail(ctx, PSA_ERR_ARG, "band must be >= 0");
+    if (flags & ~(PSA_WANT_SCORE | PSA_WANT_TRACEBACK)) return psa_fail(ctx, PSA_ERR_ARG, "flags: PSA_WANT_SCORE and PSA_WANT_TRACEBACK only");
+    if (n_pairs == 0) return PSA_OK;
+    if (!d_bases_a || !d_bases_b || !d_off_a || !d_off_b || !d_len_a || !d_len_b || !d_items || !d_anchors || !d_off_anc || !d_n_anc)
+        return psa_fail(ctx, PSA_ERR_ARG, "null device pointer");
+    if (max_len_a < 0 || max_len_b < 0) return psa_fail(ctx, PSA_ERR_ARG, "negative length bound");
+    int rc = check_banded_scoring(ctx, mode, g, h, band, max_len_a, max_len_b);
+    if (rc) return rc;
+    const bool tb = (flags & PSA_WANT_TRACEBACK) != 0;
+    if (tb && !d_ops) return psa_fail(ctx, PSA_ERR_ARG, "traceback requested without an ops buffer");
+    if (tb && ops_stride_words * 16 < (size_t)max_len_a + max_len_b)
+        return psa_fail(ctx, PSA_ERR_CAPACITY, "ops_stride_words < ceil((max m + max n)/16)");
+    PSA_CUDA_OK(ctx, cudaSetDevice(ctx->device));
+    psa_batch_args args{d_bases_a, d_off_a, d_len_a, d_bases_b, d_off_b, d_len_b, (int64_t)n_pairs, g, h,
+                        d_items, tb ? d_ops : nullptr, (int64_t)ops_stride_words};
+    const psa_guide guide{d_anchors, d_off_anc, d_n_anc};
+    cudaStream_t st = cuda_stream ? (cudaStream_t)cuda_stream : ctx->stream;
+    rc = psa_stream_enter(ctx, st);
+    if (rc) return rc;
+    rc = psa_launch_banded(ctx, args, max_len_a, max_len_b, mode, band, tb, st, &guide);
     if (rc) return rc;
     return psa_stream_leave(ctx, st);
 }
@@ -673,6 +752,44 @@ int psa_align_pair_banded(psa_ctx* ctx, const char* a, const char* b, size_t m, 
     PSA_CUDA_OK(ctx, cudaMemcpyAsync(d + o_b, b, n, cudaMemcpyHostToDevice, st));
     rc = psa_launch_banded_pair(ctx, d + o_a, d + o_b, (int)m, (int)n, mode, g, h, band, tb, (psa_batch_item*)(d + o_it),
                                 tb ? (uint32_t*)(d + o_op) : nullptr, st);
+    if (rc) return rc;
+    psa_batch_item it;
+    std::vector<uint32_t> w(tb ? words : 0);
+    PSA_CUDA_OK(ctx, cudaMemcpyAsync(&it, d + o_it, sizeof(it), cudaMemcpyDeviceToHost, st));
+    if (tb) PSA_CUDA_OK(ctx, cudaMemcpyAsync(w.data(), d + o_op, words * 4, cudaMemcpyDeviceToHost, st));
+    PSA_CUDA_OK(ctx, cudaStreamSynchronize(st));
+    return fill_result(ctx, out, it, tb ? w.data() : nullptr, a, b);
+}
+
+int psa_align_pair_guided(psa_ctx* ctx, const char* a, const char* b, size_t m, size_t n, const psa_anchor* anchors,
+                          size_t n_anchors, int mode, int g, int h, int band, unsigned flags, psa_result* out) {
+    if (!ctx) return PSA_ERR_ARG;
+    if (!out || (!a && m) || (!b && n) || (!anchors && n_anchors)) return psa_fail(ctx, PSA_ERR_ARG, "null pointer");
+    int rc = check_banded_pair(ctx, m, n, mode, g, h, band, flags);
+    if (rc) return rc;
+    if (n_anchors > (size_t)INT32_MAX) return psa_fail(ctx, PSA_ERR_ARG, "more than 2^31 - 1 anchors");
+    const int64_t off0 = 0;
+    const int32_t cnt = (int32_t)n_anchors, lm = (int32_t)m, ln = (int32_t)n;
+    rc = check_chains(ctx, anchors, &off0, &cnt, n_anchors, &lm, &ln, 1);
+    if (rc) return rc;
+    if (m == 0 || n == 0) return align_pair_impl(ctx, a, b, m, n, mode, g, h, flags, out, psa_piece_types{});
+    memset(out, 0, sizeof(*out));
+    const bool tb = (flags & PSA_WANT_TRACEBACK) != 0;
+    const size_t words = (m + n + 15) / 16 + 1;
+    PSA_CUDA_OK(ctx, cudaSetDevice(ctx->device));
+    // an asynchronous device call of this context may still be using the shared scratch on a user stream
+    if (ctx->last_valid) { PSA_CUDA_OK(ctx, cudaEventSynchronize(ctx->last_event)); ctx->last_valid = false; }
+    const size_t o_a = 0, o_b = align_up(m, 256), o_an = o_b + align_up(n, 256);
+    const size_t o_it = o_an + align_up(n_anchors * sizeof(psa_anchor), 256), o_op = o_it + 256;
+    rc = ensure_scratch(ctx, o_op + (tb ? words * 4 : 0));
+    if (rc) return rc;
+    uint8_t* d = (uint8_t*)ctx->d_scratch;
+    cudaStream_t st = ctx->stream;
+    PSA_CUDA_OK(ctx, cudaMemcpyAsync(d + o_a, a, m, cudaMemcpyHostToDevice, st));
+    PSA_CUDA_OK(ctx, cudaMemcpyAsync(d + o_b, b, n, cudaMemcpyHostToDevice, st));
+    if (n_anchors) PSA_CUDA_OK(ctx, cudaMemcpyAsync(d + o_an, anchors, n_anchors * sizeof(psa_anchor), cudaMemcpyHostToDevice, st));
+    rc = psa_launch_guided_pair(ctx, d + o_a, d + o_b, (int)m, (int)n, mode, g, h, band, anchors, (const psa_anchor*)(d + o_an),
+                                cnt, tb, (psa_batch_item*)(d + o_it), tb ? (uint32_t*)(d + o_op) : nullptr, st);
     if (rc) return rc;
     psa_batch_item it;
     std::vector<uint32_t> w(tb ? words : 0);

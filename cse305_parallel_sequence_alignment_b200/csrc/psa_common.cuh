@@ -125,6 +125,13 @@ struct psa_batch_args {
     const uint8_t* types = nullptr;   // optional, per pair: (start_type + 3) | (end_type + 3) << 4; overrides the two above
 };
 
+// Anchor chains of a guided batch (psa_align_batch_guided): pair k's chain is anchors[off[k] .. off[k] + n[k]).
+struct psa_guide {
+    const psa_anchor* anchors;
+    const int64_t* off;
+    const int32_t* n;
+};
+
 // launchers (each returns a psa_status and bumps ctx->launches)
 int psa_launch_short(psa_ctx* ctx, const psa_batch_args& args, int max_m, int max_n, int mode, bool traceback,
                      cudaStream_t stream);
@@ -163,11 +170,16 @@ int psa_launch_long_batch_at(psa_ctx* ctx, const psa_batch_args& args, int max_m
 // psa_long_batch_tb_chunk: pairs per chunk for this batch shape (0: one checkpoint slot exceeds the memory budget).
 int psa_long_batch_tb_chunk(psa_ctx* ctx, long long n_pairs, int max_m, int max_n, int mode, long long* chunk);
 int psa_launch_long_batch_tb(psa_ctx* ctx, const psa_batch_args& args, int max_m, int max_n, int mode, cudaStream_t st);
-// Banded batch (psa_align_batch_banded): every pair on the banded tile kernels, one warp per pair (psa_long.cu).
+// Banded batch (psa_align_batch_banded): every pair on the banded tile kernels, one warp per pair (psa_long.cu).  With a
+// guide (device arrays) each pair's band follows its anchor chain (psa_align_batch_guided[_device]).
 int psa_launch_banded(psa_ctx* ctx, const psa_batch_args& args, int max_m, int max_n, int mode, int band, bool traceback,
-                      cudaStream_t st);
+                      cudaStream_t st, const psa_guide* guide = nullptr);
 // One banded pair over the whole GPU (psa_align_pair_banded, psa_align_long_banded_device; psa_long.cu).
 int psa_launch_banded_pair(psa_ctx* ctx, const uint8_t* d_a, const uint8_t* d_b, int m, int n, int mode, int g, int h, int band,
                            bool traceback, psa_batch_item* d_item, uint32_t* d_ops, cudaStream_t st);
+// The same around a valid anchor chain (psa_align_pair_guided): planned from the host copy, run on the device copy.
+int psa_launch_guided_pair(psa_ctx* ctx, const uint8_t* d_a, const uint8_t* d_b, int m, int n, int mode, int g, int h, int band,
+                           const psa_anchor* h_anchors, const psa_anchor* d_anchors, int n_anchors, bool traceback,
+                           psa_batch_item* d_item, uint32_t* d_ops, cudaStream_t st);
 bool psa_pack_long_supported(int max_m, int max_n, int mode, int g, int h);
 int psa_launch_pack_long(psa_ctx* ctx, const psa_batch_args& args, int max_m, int max_n, int mode, cudaStream_t st);

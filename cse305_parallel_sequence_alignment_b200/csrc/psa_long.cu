@@ -524,6 +524,94 @@ struct Band {
     }
 };
 
+// The band around a caller's anchor chain (psa_align_batch_guided, psa_align_pair_guided; include/psa.h).  The guide is
+// the polyline P_0 = (0, 0), P_1 .. P_K (the anchors), P_{K+1} = (m, n).  Row i's guide columns [cmin(i), cmax(i)] are
+// the j of the first and of the last chain point on row i, else the point at floor of the segment P_k -> P_{k+1} that
+// crosses row i; lo(i) = max(0, cmin(i) - bw), hi(i) = min(n, cmax(i) + bw).  A valid chain (coordinates in range and
+// non-decreasing) gives cmin(i + 1) >= cmax(i), so lo and hi are non-decreasing and s_lo / s_hi / inside keep Band's
+// formulas.  Each row costs a binary search over the chain; nothing is evaluated per cell.  K = 0 gives Band's rows.
+struct ChainBand {
+    int m, n, bw;
+    const psa_anchor* anc;     // the pair's K anchors, a valid chain
+    int K;
+    __host__ __device__ __forceinline__ int2 pt(int k) const {          // P_k, k = 0 .. K + 1
+        return k == 0 ? make_int2(0, 0) : k > K ? make_int2(m, n) : make_int2(anc[k - 1].i, anc[k - 1].j);
+    }
+    // first k with P_k.i > i (strict) or P_k.i >= i
+    __host__ __device__ __forceinline__ int bound(int i, bool strict) const {
+        int a = 0, b = K + 2;
+        while (a < b) {
+            const int mid = (a + b) >> 1, pi = pt(mid).x;
+            if (pi < i || (strict && pi == i)) a = mid + 1; else b = mid;
+        }
+        return a;
+    }
+    // column of the segment P_k -> P_{k+1} on row i, P_k.i < i < P_{k+1}.i
+    __host__ __device__ __forceinline__ int seg(int k, int i) const {
+        const int2 p = pt(k), q = pt(k + 1);
+        return p.y + (int)((long long)(i - p.x) * (q.y - p.y) / (q.x - p.x));
+    }
+    __host__ __device__ __forceinline__ int cmin(int i) const {
+        const int k = bound(i, false);
+        return pt(k).x == i ? pt(k).y : seg(k - 1, i);
+    }
+    __host__ __device__ __forceinline__ int cmax(int i) const {
+        const int k = bound(i, true);
+        return pt(k - 1).x == i ? pt(k - 1).y : seg(k - 1, i);
+    }
+    __host__ __device__ __forceinline__ int lo(int i) const { const int v = cmin(i) - bw; return v < 0 ? 0 : v; }
+    __host__ __device__ __forceinline__ int hi(int i) const { const long long v = (long long)cmax(i) + bw; return v > n ? n : (int)v; }
+    __host__ __device__ __forceinline__ int s_lo(int i0, int WW) const { const int l = lo(i0 + 1); return ((l > 1 ? l : 1) - 1) / WW; }
+    __host__ __device__ __forceinline__ int s_hi(int i0, int nrows, int WW) const {
+        const int h = hi(i0 + nrows), s = ((h > 1 ? h : 1) - 1) / WW, sl = s_lo(i0, WW);
+        return s > sl ? s : sl;
+    }
+    __host__ __device__ __forceinline__ bool inside(int i0, int nrows, int s, int WW) const {
+        const int right = n < (s + 1) * WW ? n : (s + 1) * WW;
+        return lo(i0 + nrows) <= s * WW + 1 && hi(i0 + 1) >= right;
+    }
+};
+
+// Warp-collective: anchors[0 .. K) form a valid chain for an m x n pair (K >= 0, 0 <= i <= m, 0 <= j <= n, both
+// coordinates non-decreasing).  Reads nothing when K < 0.
+__device__ bool chain_ok(const psa_anchor* anc, int K, int m, int n) {
+    if (K < 0) return false;
+    bool bad = false;
+    for (int k = threadIdx.x & 31; k < K; k += 32) {
+        const psa_anchor a = anc[k];
+        bad |= a.i < 0 || a.i > m || a.j < 0 || a.j > n;
+        if (k > 0) { const psa_anchor p = anc[k - 1]; bad |= a.i < p.i || a.j < p.j; }
+    }
+    return !__any_sync(0xffffffffu, bad);
+}
+
+// Where the batch kernels take each pair's band from: the diagonal of psa_align_batch_banded, or the pair's chain.
+struct DiagGuide {
+    using BandT = Band;
+    __device__ __forceinline__ Band band(long long, int m, int n, int bw) const { return Band{m, n, bw}; }
+    __device__ __forceinline__ bool ok(long long, int, int) const { return true; }
+};
+struct ChainGuide {
+    using BandT = ChainBand;
+    const psa_anchor* anc;     // pair p: anc[off[p] .. off[p] + cnt[p])
+    const int64_t* off;
+    const int32_t* cnt;
+    __device__ __forceinline__ ChainBand band(long long p, int m, int n, int bw) const { return ChainBand{m, n, bw, anc + off[p], cnt[p]}; }
+    __device__ __forceinline__ bool ok(long long p, int m, int n) const {
+        const int k = cnt[p];
+        return chain_ok(k >= 0 ? anc + off[p] : nullptr, k, m, n);
+    }
+};
+
+// Record of a pair whose chain the device form rejects: -inf corners and score, end state 0 (no other path produces
+// it), every cell 0, aln_len 0.
+__device__ __forceinline__ psa_batch_item rejected_item() {
+    psa_batch_item r;
+    r.t1 = r.t2 = r.t3 = r.score = PSA_NEG_INF;
+    r.end_state = 0; r.end_i = r.end_j = r.start_i = r.start_j = 0; r.aln_len = 0;
+    return r;
+}
+
 template <int MODE>
 __device__ __forceinline__ constexpr int oob_H() { return MODE == PSA_LOCAL ? 0 : PSA_KNEG; }
 
@@ -531,11 +619,13 @@ __device__ __forceinline__ constexpr int oob_H() { return MODE == PSA_LOCAL ? 0 
 // over its W columns) and its right column (H, E over its R rows).  Row block rb's tiles are records
 // tile_base[rb] .. tile_base[rb] + s_hi - s_lo, in strip order.
 constexpr int REC = 2 * W + 2 * R;     // ints per tile record
-struct BandCk {
-    Band B;
+template <class BandT>
+struct BandCkT {
+    BandT B;
     int* rec;
     long long* tile_base;              // [NB]
 };
+using BandCk = BandCkT<Band>;
 
 struct BandSmem {
     WarpSmem<R> w;
@@ -544,8 +634,8 @@ struct BandSmem {
 
 // H and F of row i0 (the top boundary of row block rb) at column j.  prev: row block rb-1's strips p_lo .. p_hi, kept in
 // the recycled row J.hbufH / J.hbufF (score only) or in the records from rec_prev on (traceback).
-template <int MODE, int WW, bool TB>
-__device__ __forceinline__ void band_top(const LongJob& J, const Band& B, const int* rec_prev, int rb, int i0, int p_lo, int p_hi,
+template <int MODE, int WW, bool TB, class BandT>
+__device__ __forceinline__ void band_top(const LongJob& J, const BandT& B, const int* rec_prev, int rb, int i0, int p_lo, int p_hi,
                                          int j, int& H, int& F) {
     F = PSA_KNEG;
     if (rb == 0) { H = j <= B.hi(0) ? border_row0_H<MODE>(j, J.g, J.h) : oob_H<MODE>(); return; }
@@ -564,8 +654,8 @@ __device__ __forceinline__ void band_top(const LongJob& J, const Band& B, const 
 // into the recycled row.  Traceback fill (TB = true): <128, 8> grid, sweep<> without codes, every tile's bottom row and
 // right column into the records rec_cur (row block rb) -- rec_prev are row block rb-1's.
 // WAIT (one pair over many warps): row block rb-1 may still be running; J.progress[rb] = 1 + the last strip finished.
-template <int MODE, int KK, bool TB, bool WAIT = false>
-__device__ void process_rowblock_banded(const LongJob& J, const Band& B, int rb, BandSmem& sm, Track& tr, int* rec_cur,
+template <int MODE, int KK, bool TB, bool WAIT = false, class BandT>
+__device__ void process_rowblock_banded(const LongJob& J, const BandT& B, int rb, BandSmem& sm, Track& tr, int* rec_cur,
                                         const int* rec_prev) {
     constexpr int WW = 32 * KK;
     static_assert(!TB || WW == W, "traceback checkpoints use the walk's tile grid");
@@ -696,9 +786,10 @@ struct BandedBatch {
     int bw;
 };
 
-// Score only: one warp per pair, one recycled boundary row, <128, 16> tiles.
-template <int MODE>
-__global__ void __launch_bounds__(WPB * 32) psa_banded_batch_kernel(BandedBatch Bt) {
+// Score only: one warp per pair, one recycled boundary row, <128, 16> tiles.  G: each pair's band (DiagGuide /
+// ChainGuide); a pair whose chain G rejects gets rejected_item() and touches nothing else.
+template <int MODE, class Guide>
+__device__ __forceinline__ void banded_batch(const BandedBatch& Bt, const Guide& G) {
     constexpr int KB = 16;
     __shared__ BandSmem smem[WPB];
     __shared__ unsigned long long s_best[WPB];
@@ -721,8 +812,9 @@ __global__ void __launch_bounds__(WPB * 32) psa_banded_batch_kernel(BandedBatch 
         J.start_type = -1; J.end_type = -1;
         if (lane == 0) { s_best[w] = 0ull; s_corner[w][0] = s_corner[w][1] = s_corner[w][2] = PSA_KNEG; }
         __syncwarp();
-        if (J.m > 0 && J.n > 0) {
-            const Band B{J.m, J.n, Bt.bw};
+        const bool ok = G.ok(p, J.m, J.n);
+        if (ok && J.m > 0 && J.n > 0) {
+            const auto B = G.band(p, J.m, J.n, Bt.bw);
             Track tr{0, 0, 0};
             const int NB = (J.m + R - 1) / R;
             for (int rb = 0; rb < NB; ++rb) process_rowblock_banded<MODE, KB, false>(J, B, rb, sm, tr, nullptr, nullptr);
@@ -734,11 +826,16 @@ __global__ void __launch_bounds__(WPB * 32) psa_banded_batch_kernel(BandedBatch 
             if (J.m <= 0 || J.n <= 0) r = empty_item<MODE>(J.m, J.n, J.g, J.h, -1, -1);
             else if (MODE == PSA_LOCAL) r = local_item_from_key(s_best[w]);
             else r = global_item(s_corner[w][0], s_corner[w][1], s_corner[w][2], J.m, J.n, J.h, -1);
-            Bt.P.items[p] = banded_item(r);
+            Bt.P.items[p] = ok ? banded_item(r) : rejected_item();
         }
         __syncwarp();
     }
 }
+
+template <int MODE>
+__global__ void __launch_bounds__(WPB * 32) psa_banded_batch_kernel(BandedBatch Bt) { banded_batch<MODE>(Bt, DiagGuide{}); }
+template <int MODE>
+__global__ void __launch_bounds__(WPB * 32) psa_guided_batch_kernel(BandedBatch Bt, ChainGuide G) { banded_batch<MODE>(Bt, G); }
 
 // Traceback: pair p of the chunk [p0, p0 + count) owns slot p - p0: [best (8 B) | corner (3 x 4 B) | pad to 256 B |
 // tile_base (NB x 8 B, padded to 256 B) | tile records (REC ints each)], inside slot_bytes (planned from max m, max n, bw).
@@ -751,7 +848,8 @@ struct BandedTb {
     int bw;
 };
 
-__device__ __forceinline__ LongJob banded_tb_job(const BandedTb& Bt, long long p, BandCk& bk) {
+template <class Guide>
+__device__ __forceinline__ LongJob banded_tb_job(const BandedTb& Bt, const Guide& G, long long p, BandCkT<typename Guide::BandT>& bk) {
     const psa_batch_args& P = Bt.P;
     LongJob J;
     J.a = P.bases_a + P.off_a[p]; J.b = P.bases_b + P.off_b[p];
@@ -762,14 +860,14 @@ __device__ __forceinline__ LongJob banded_tb_job(const BandedTb& Bt, long long p
     J.hbufH = nullptr; J.hbufF = nullptr; J.hb_stride = 0;
     J.ckvH = nullptr; J.ckvE = nullptr; J.progress = nullptr; J.ticket = nullptr;
     J.col0 = 0; J.n_total = J.n; J.row_off = 0; J.start_type = -1; J.end_type = -1;
-    bk.B = Band{J.m, J.n, Bt.bw};
+    bk.B = G.band(p, J.m, J.n, Bt.bw);
     bk.tile_base = (long long*)(slot + 256);
     bk.rec = (int*)(slot + 256 + up256_d((long long)NB * 8));
     return J;
 }
 
-template <int MODE>
-__global__ void __launch_bounds__(WPB * 32) psa_banded_tb_fill_kernel(BandedTb Bt) {
+template <int MODE, class Guide>
+__device__ __forceinline__ void banded_tb_fill(const BandedTb& Bt, const Guide& G) {
     __shared__ BandSmem smem[WPB];
     const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
     BandSmem& sm = smem[w];
@@ -778,9 +876,10 @@ __global__ void __launch_bounds__(WPB * 32) psa_banded_tb_fill_kernel(BandedTb B
         if (lane == 0) q = atomicAdd(Bt.ticket, 1);
         q = __shfl_sync(0xffffffffu, q, 0);
         if (q >= Bt.count) break;
-        BandCk bk;
-        const LongJob J = banded_tb_job(Bt, Bt.p0 + q, bk);
+        BandCkT<typename Guide::BandT> bk;
+        const LongJob J = banded_tb_job(Bt, G, Bt.p0 + q, bk);
         if (J.m <= 0 || J.n <= 0) continue;          // borders only: the walk kernel writes the item
+        if (!G.ok(Bt.p0 + q, J.m, J.n)) continue;    // rejected chain: its slot stays untouched, the walk writes the item
         if (lane == 0) { *J.best = 0ull; J.corner[0] = J.corner[1] = J.corner[2] = PSA_KNEG; }
         __syncwarp();
         Track tr{0, 0, 0};
@@ -797,13 +896,18 @@ __global__ void __launch_bounds__(WPB * 32) psa_banded_tb_fill_kernel(BandedTb B
     }
 }
 
-// recompute_tile for the banded layout: boundaries from the records, out-of-band values outside them, masked sweep.
 template <int MODE>
-__device__ void recompute_tile_banded(const LongJob& J, const BandCk& bk, int rb, int s, int nrows, uint32_t* dirs, int* lbH,
+__global__ void __launch_bounds__(WPB * 32) psa_banded_tb_fill_kernel(BandedTb Bt) { banded_tb_fill<MODE>(Bt, DiagGuide{}); }
+template <int MODE>
+__global__ void __launch_bounds__(WPB * 32) psa_guided_tb_fill_kernel(BandedTb Bt, ChainGuide G) { banded_tb_fill<MODE>(Bt, G); }
+
+// recompute_tile for the banded layout: boundaries from the records, out-of-band values outside them, masked sweep.
+template <int MODE, class BandT>
+__device__ void recompute_tile_banded(const LongJob& J, const BandCkT<BandT>& bk, int rb, int s, int nrows, uint32_t* dirs, int* lbH,
                                       int* lbE, uint8_t* sA, int* bLo, int* bHi) {
     const int lane = threadIdx.x & 31;
     const int m = J.m, n = J.n, g = J.g, h = J.h;
-    const Band& B = bk.B;
+    const BandT& B = bk.B;
     const int i0 = rb * R, c0 = s * W + lane * K;
     const int s_lo = B.s_lo(i0, W);
     const int p_lo = rb > 0 ? B.s_lo(i0 - R, W) : 0, p_hi = rb > 0 ? B.s_hi(i0 - R, R, W) : -1;
@@ -865,8 +969,8 @@ __device__ __forceinline__ void walk_steps(const uint32_t* dirs, int trb, int ts
 
 // tb_walk over the banded layout: the same steps, every tile the path enters recomputed by recompute_tile_banded.  (A
 // separate function so that the unbanded walks keep their code.)
-template <int MODE>
-__device__ void tb_walk_banded(const LongJob& J, const BandCk& bk, psa_batch_item& r, uint32_t* ops, uint32_t* dirs, int* lbH,
+template <int MODE, class BandT>
+__device__ void tb_walk_banded(const LongJob& J, const BandCkT<BandT>& bk, psa_batch_item& r, uint32_t* ops, uint32_t* dirs, int* lbH,
                                int* lbE, uint8_t* sA, int* bLo, int* bHi) {
     const int lane = threadIdx.x & 31;
     const int m = J.m;
@@ -912,26 +1016,38 @@ __device__ void tb_walk_banded(const LongJob& J, const BandCk& bk, psa_batch_ite
     }
 }
 
-template <int MODE>
-__global__ void __launch_bounds__(WALK_WPB * 32) psa_banded_tb_walk_kernel(BandedTb Bt) {
+// tid, bid: threadIdx.x, blockIdx.x, read by the kernel itself (which knows their range from its launch bounds)
+template <int MODE, class Guide>
+__device__ __forceinline__ void banded_tb_walk(const BandedTb& Bt, const Guide& G, unsigned tid, unsigned bid) {
     __shared__ uint32_t dirs[WALK_WPB][R * 32];
     __shared__ int lbH[WALK_WPB][R], lbE[WALK_WPB][R], bLo[WALK_WPB][R], bHi[WALK_WPB][R];
     __shared__ uint8_t sA[WALK_WPB][R];
-    const int w = threadIdx.x >> 5;
-    const long long q = (long long)blockIdx.x * WALK_WPB + w;
+    const int w = tid >> 5;
+    const long long q = (long long)bid * WALK_WPB + w;
     if (q >= Bt.count) return;
     const long long p = Bt.p0 + q;
-    BandCk bk;
-    const LongJob J = banded_tb_job(Bt, p, bk);
+    BandCkT<typename Guide::BandT> bk;
+    const LongJob J = banded_tb_job(Bt, G, p, bk);
     psa_batch_item r;
-    if (J.m <= 0 || J.n <= 0) {
+    if (!G.ok(p, J.m, J.n)) {
+        r = rejected_item();
+    } else if (J.m <= 0 || J.n <= 0) {
         r = empty_item<MODE>(J.m, J.n, J.g, J.h, -1, -1);
     } else {
         r = banded_item(tb_end<MODE>(J));
         if (r.score != PSA_NEG_INF)
             tb_walk_banded<MODE>(J, bk, r, Bt.P.ops + p * Bt.P.ops_stride_words, dirs[w], lbH[w], lbE[w], sA[w], bLo[w], bHi[w]);
     }
-    if ((threadIdx.x & 31) == 0) Bt.P.items[p] = r;
+    if ((tid & 31) == 0) Bt.P.items[p] = r;
+}
+
+template <int MODE>
+__global__ void __launch_bounds__(WALK_WPB * 32) psa_banded_tb_walk_kernel(BandedTb Bt) {
+    banded_tb_walk<MODE>(Bt, DiagGuide{}, threadIdx.x, blockIdx.x);
+}
+template <int MODE>
+__global__ void __launch_bounds__(WALK_WPB * 32) psa_guided_tb_walk_kernel(BandedTb Bt, ChainGuide G) {
+    banded_tb_walk<MODE>(Bt, G, threadIdx.x, blockIdx.x);
 }
 
 // ---- one banded pair over the whole GPU (psa_align_pair_banded, psa_align_long_banded_device) --------------------------
@@ -939,13 +1055,16 @@ __global__ void __launch_bounds__(WALK_WPB * 32) psa_banded_tb_walk_kernel(Bande
 // the progress handshake of process_rowblock_banded<..., WAIT>.  Score only: one recycled H/F row of n + 1 ints (row block
 // rb reads strip s of it before it overwrites it, rb + 1 reads it only afterwards).  Traceback: the per-tile records of
 // BandCk at tile_base[rb], computed beforehand by psa_banded_tile_base_kernel.
-struct BandedPair {
+template <class BandT>
+struct PairFillT {
     LongJob J;                 // progress, ticket, best, corner; hbufH / hbufF: the recycled row (score only)
-    BandCk bk;                 // traceback only
+    BandCkT<BandT> bk;         // traceback only
 };
+struct BandedPair : PairFillT<Band> {};
+struct GuidedPair : PairFillT<ChainBand> {};   // psa_align_pair_guided: the chain, validated on the host
 
-template <int MODE, int KK, bool TB>
-__global__ void __launch_bounds__(WPB * 32) psa_banded_pair_fill_kernel(BandedPair P) {
+template <int MODE, int KK, bool TB, class BandT>
+__device__ __forceinline__ void banded_pair_fill(const PairFillT<BandT>& P) {
     __shared__ BandSmem smem[WPB];
     BandSmem& sm = smem[threadIdx.x >> 5];
     const int lane = threadIdx.x & 31;
@@ -964,8 +1083,14 @@ __global__ void __launch_bounds__(WPB * 32) psa_banded_pair_fill_kernel(BandedPa
     flush_track<MODE>(J, tr);
 }
 
+template <int MODE, int KK, bool TB>
+__global__ void __launch_bounds__(WPB * 32) psa_banded_pair_fill_kernel(BandedPair P) { banded_pair_fill<MODE, KK, TB>(P); }
+template <int MODE, int KK, bool TB>
+__global__ void __launch_bounds__(WPB * 32) psa_guided_pair_fill_kernel(GuidedPair P) { banded_pair_fill<MODE, KK, TB>(P); }
+
 // tile_base[rb] = tiles of row blocks 0 .. rb-1 (NB <= 16384: at most 16 row blocks per thread).
-__global__ void __launch_bounds__(1024) psa_banded_tile_base_kernel(Band B, long long* tile_base) {
+template <class BandT>
+__device__ __forceinline__ void banded_tile_base(const BandT& B, long long* tile_base) {
     __shared__ long long part[1024];
     const int NB = (B.m + R - 1) / R, t = threadIdx.x;
     const int per = (NB + 1023) / 1024, r0 = min(NB, t * per), r1 = min(NB, r0 + per);
@@ -983,6 +1108,9 @@ __global__ void __launch_bounds__(1024) psa_banded_tile_base_kernel(Band B, long
     long long base = part[t] - sum;
     for (int rb = r0; rb < r1; ++rb) { tile_base[rb] = base; base += tiles(rb); }
 }
+
+__global__ void __launch_bounds__(1024) psa_banded_tile_base_kernel(Band B, long long* tile_base) { banded_tile_base(B, tile_base); }
+__global__ void __launch_bounds__(1024) psa_guided_tile_base_kernel(ChainBand B, long long* tile_base) { banded_tile_base(B, tile_base); }
 
 // Walk: bottom-up in windows of row blocks rb_lo .. rb_hi-1.  For each window psa_banded_pair_codes_kernel first recomputes
 // the codes of every band tile of the window the path can still reach -- rows above the walk's current row, strips not
@@ -1005,10 +1133,20 @@ struct BandedPairTb {
     psa_batch_item* item;
     uint32_t* ops;             // null: score only (one window, which writes the record)
 };
+struct GuidedPairTb {
+    LongJob J;
+    BandCkT<ChainBand> bk;
+    uint32_t* codes;           // [rb - rb_lo][tpr] tiles of R*32 code words
+    int tpr;                   // tile slots per row block (>= s_hi - s_lo + 1 of every row block)
+    int rb_lo, rb_hi;          // this window; rb_hi == NB: the first window
+    BandedWalk* walk;
+    psa_batch_item* item;
+    uint32_t* ops;             // null: score only (one window, which writes the record)
+};
 
 // Start of the walk: the end cell and end state of the banded record in the first window, else the saved state.
-template <int MODE>
-__device__ __forceinline__ BandedWalk walk_start(const BandedPairTb& T) {
+template <int MODE, class TbT>
+__device__ __forceinline__ BandedWalk walk_start(const TbT& T) {
     if (T.rb_hi * R < T.J.m) return *T.walk;
     BandedWalk w;
     w.r = banded_item(tb_end<MODE>(T.J));
@@ -1018,17 +1156,17 @@ __device__ __forceinline__ BandedWalk walk_start(const BandedPairTb& T) {
 }
 
 constexpr int CODES_WPB = 2;
-template <int MODE>
-__global__ void __launch_bounds__(CODES_WPB * 32) psa_banded_pair_codes_kernel(BandedPairTb T) {
+template <int MODE, class TbT>
+__device__ __forceinline__ void banded_pair_codes(const TbT& T, unsigned tid, unsigned bid) {   // as banded_tb_walk
     __shared__ uint32_t dirs[CODES_WPB][R * 32];
     __shared__ int lbH[CODES_WPB][R], lbE[CODES_WPB][R], bLo[CODES_WPB][R], bHi[CODES_WPB][R];
     __shared__ uint8_t sA[CODES_WPB][R];
-    const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const long long u = (long long)blockIdx.x * CODES_WPB + w;
+    const int w = tid >> 5, lane = tid & 31;
+    const long long u = (long long)bid * CODES_WPB + w;
     if (u >= (long long)(T.rb_hi - T.rb_lo) * T.tpr) return;
     const int rb = T.rb_lo + (int)(u / T.tpr), t = (int)(u % T.tpr);
     const BandedWalk st = walk_start<MODE>(T);
-    const Band& B = T.bk.B;
+    const auto& B = T.bk.B;
     const int i0 = rb * R, nrows = min(R, T.J.m - i0), s = B.s_lo(i0, W) + t;
     if (st.done || i0 >= st.i || s > B.s_hi(i0, nrows, W) || s * W >= st.j) return;
     recompute_tile_banded<MODE>(T.J, T.bk, rb, s, nrows, dirs[w], lbH[w], lbE[w], sA[w], bLo[w], bHi[w]);
@@ -1038,6 +1176,11 @@ __global__ void __launch_bounds__(CODES_WPB * 32) psa_banded_pair_codes_kernel(B
 }
 
 template <int MODE>
+__global__ void __launch_bounds__(CODES_WPB * 32) psa_banded_pair_codes_kernel(BandedPairTb T) { banded_pair_codes<MODE>(T, threadIdx.x, blockIdx.x); }
+template <int MODE>
+__global__ void __launch_bounds__(CODES_WPB * 32) psa_guided_pair_codes_kernel(GuidedPairTb T) { banded_pair_codes<MODE>(T, threadIdx.x, blockIdx.x); }
+
+template <int MODE>
 __global__ void __launch_bounds__(32) psa_banded_pair_walk_kernel(BandedPairTb T) {
     __shared__ uint32_t dirs[R * 32];
     __shared__ int lbH[R], lbE[R], bLo[R], bHi[R];
@@ -1045,6 +1188,65 @@ __global__ void __launch_bounds__(32) psa_banded_pair_walk_kernel(BandedPairTb T
     const int lane = threadIdx.x;
     const LongJob& J = T.J;
     const Band& B = T.bk.B;
+    BandedWalk st = walk_start<MODE>(T);
+    const bool first = T.rb_hi * R >= J.m;
+    if (st.done && !first) return;                        // finished in an earlier window
+    int i = st.i, j = st.j, state = st.state, len = st.len;
+    uint32_t acc = st.acc;
+    bool done = st.done || !(i > 0 && j > 0);
+    int trb = -1, ts = -1;
+    while (!done) {
+        int need_rb = -1, need_s = -1;
+        if (lane == 0) walk_steps<MODE>(dirs, trb, ts, i, j, state, len, acc, T.ops, st.r, need_rb, need_s);
+        need_rb = __shfl_sync(0xffffffffu, need_rb, 0);
+        need_s = __shfl_sync(0xffffffffu, need_s, 0);
+        if (need_rb < 0) { done = true; break; }
+        if (need_rb < T.rb_lo) break;                     // the next window's rows
+        const int need_row = __shfl_sync(0xffffffffu, (lane == 0) ? ((state == 2) ? i : i - 1) : 0, 0);
+        const int i0 = need_rb * R, full = min(R, J.m - i0), nrows = min(full, need_row - i0);
+        const int t = need_s - B.s_lo(i0, W);
+        if (t >= 0 && t < T.tpr && need_s <= B.s_hi(i0, full, W)) {
+            const uint4* in = reinterpret_cast<const uint4*>(T.codes + ((long long)(need_rb - T.rb_lo) * T.tpr + t) * (R * 32));
+            uint4* out = reinterpret_cast<uint4*>(dirs);
+            const int total = nrows * 8;
+            __syncwarp();
+            for (int q0 = 0; q0 < total; q0 += 256) {       // as tb_walk: eight 16-byte loads in flight per lane
+                uint4 v[8];
+#pragma unroll
+                for (int x = 0; x < 8; ++x) { const int q = q0 + x * 32 + lane; if (q < total) v[x] = __ldcg(in + q); }
+#pragma unroll
+                for (int x = 0; x < 8; ++x) { const int q = q0 + x * 32 + lane; if (q < total) out[q] = v[x]; }
+            }
+            __syncwarp();
+        } else {
+            recompute_tile_banded<MODE>(J, T.bk, need_rb, need_s, nrows, dirs, lbH, lbE, sA, bLo, bHi);
+        }
+        trb = need_rb; ts = need_s;
+    }
+    if (lane == 0) {
+        if (done) {
+            if (T.ops != nullptr && st.r.score != PSA_NEG_INF) {     // as tb_walk_banded
+                if (len & 15) T.ops[len >> 4] = acc;
+                st.r.aln_len = len;
+            }
+            *T.item = st.r;
+        }
+        st.i = i; st.j = j; st.state = state; st.len = len; st.acc = acc; st.done = done;
+        *T.walk = st;
+    }
+}
+
+
+// The guided pair's walk: psa_banded_pair_walk_kernel's body over ChainBand.  A copy, not a shared template: inlined into
+// a helper the diagonal kernel compiles to different SASS.
+template <int MODE>
+__global__ void __launch_bounds__(32) psa_guided_pair_walk_kernel(GuidedPairTb T) {
+    __shared__ uint32_t dirs[R * 32];
+    __shared__ int lbH[R], lbE[R], bLo[R], bHi[R];
+    __shared__ uint8_t sA[R];
+    const int lane = threadIdx.x;
+    const LongJob& J = T.J;
+    const auto& B = T.bk.B;
     BandedWalk st = walk_start<MODE>(T);
     const bool first = T.rb_hi * R >= J.m;
     if (st.done && !first) return;                        // finished in an earlier window
@@ -1352,13 +1554,18 @@ size_t banded_slot_bytes(int max_m, int max_n, int bw) {
 }
 }  // namespace
 
+// guide (device arrays) selects the guided kernels: each pair's band follows its anchor chain.  The slot bound holds for
+// every valid chain too: a chain's rows are monotone (cmin(i + 1) >= cmax(i)), so the row blocks' spans still sum to at
+// most n + 2*bw*NB.
 int psa_launch_banded(psa_ctx* ctx, const psa_batch_args& args, int max_m, int max_n, int mode, int band, bool traceback,
-                      cudaStream_t st) {
+                      cudaStream_t st, const psa_guide* guide) {
     if (max_m >= 0x1FFFFF || max_n >= 0x1FFFFF) return psa_fail(ctx, PSA_ERR_RANGE, "long path: lengths must be < 2^21 - 1");
     const int bw = (int)std::min<long long>(band, (long long)max_m + max_n);     // wider bands admit the same cells
     const bool local = mode == PSA_LOCAL;
+    ChainGuide G{guide ? guide->anchors : nullptr, guide ? guide->off : nullptr, guide ? guide->n : nullptr};
     if (!traceback) {
-        const void* kern = local ? (const void*)psa_banded_batch_kernel<PSA_LOCAL> : (const void*)psa_banded_batch_kernel<PSA_GLOBAL>;
+        const void* kern = guide ? (local ? (const void*)psa_guided_batch_kernel<PSA_LOCAL> : (const void*)psa_guided_batch_kernel<PSA_GLOBAL>)
+                                 : (local ? (const void*)psa_banded_batch_kernel<PSA_LOCAL> : (const void*)psa_banded_batch_kernel<PSA_GLOBAL>);
         int grid = 1;
         int rc = long_batch_grid(ctx, args.n_pairs, kern, &grid);
         if (rc) return rc;
@@ -1369,13 +1576,16 @@ int psa_launch_banded(psa_ctx* ctx, const psa_batch_args& args, int max_m, int m
         uint8_t* d = (uint8_t*)ctx->d_work;
         PSA_CUDA_OK(ctx, cudaMemsetAsync(d + hb, 0, 256, st));
         BandedBatch Bt{args, (int*)d, (long long)warp_stride, (int*)(d + hb), bw};
-        void* kargs[] = {&Bt};
+        void* kargs[] = {&Bt, &G};
         PSA_CUDA_OK(ctx, cudaLaunchKernel(kern, dim3(grid), dim3(WPB * 32), kargs, 0, st));
         ctx->launches += 1;
         return PSA_OK;
     }
     int per_sm = 0;
-    const void* fill = local ? (const void*)psa_banded_tb_fill_kernel<PSA_LOCAL> : (const void*)psa_banded_tb_fill_kernel<PSA_GLOBAL>;
+    const void* fill = guide ? (local ? (const void*)psa_guided_tb_fill_kernel<PSA_LOCAL> : (const void*)psa_guided_tb_fill_kernel<PSA_GLOBAL>)
+                             : (local ? (const void*)psa_banded_tb_fill_kernel<PSA_LOCAL> : (const void*)psa_banded_tb_fill_kernel<PSA_GLOBAL>);
+    const void* walk = guide ? (local ? (const void*)psa_guided_tb_walk_kernel<PSA_LOCAL> : (const void*)psa_guided_tb_walk_kernel<PSA_GLOBAL>)
+                             : (local ? (const void*)psa_banded_tb_walk_kernel<PSA_LOCAL> : (const void*)psa_banded_tb_walk_kernel<PSA_GLOBAL>);
     PSA_CUDA_OK(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fill, WPB * 32, 0));
     const long long ctas = std::max(1, std::min(per_sm, 4) * ctx->sm_count);
     size_t free_b = 0, total_b = 0;
@@ -1395,22 +1605,18 @@ int psa_launch_banded(psa_ctx* ctx, const psa_batch_args& args, int max_m, int m
         PSA_CUDA_OK(ctx, cudaMemsetAsync(d, 0, 256, st));
         const int fill_grid = (int)std::min<long long>((cnt + WPB - 1) / WPB, ctas);
         const int walk_grid = (int)((cnt + WALK_WPB - 1) / WALK_WPB);
-        if (local) {
-            psa_banded_tb_fill_kernel<PSA_LOCAL><<<fill_grid, WPB * 32, 0, st>>>(Bt);
-            psa_banded_tb_walk_kernel<PSA_LOCAL><<<walk_grid, WALK_WPB * 32, 0, st>>>(Bt);
-        } else {
-            psa_banded_tb_fill_kernel<PSA_GLOBAL><<<fill_grid, WPB * 32, 0, st>>>(Bt);
-            psa_banded_tb_walk_kernel<PSA_GLOBAL><<<walk_grid, WALK_WPB * 32, 0, st>>>(Bt);
-        }
-        PSA_CUDA_OK(ctx, cudaGetLastError());
+        void* kargs[] = {&Bt, &G};
+        PSA_CUDA_OK(ctx, cudaLaunchKernel(fill, dim3(fill_grid), dim3(WPB * 32), kargs, 0, st));
+        PSA_CUDA_OK(ctx, cudaLaunchKernel(walk, dim3(walk_grid), dim3(WALK_WPB * 32), kargs, 0, st));
         ctx->launches += 2;
     }
     return PSA_OK;
 }
 
 // ---- one banded pair over the whole GPU ----------------------------------------------------------------------------
-// Planned from (m, n, band, mode, traceback) alone.  Launches (include/psa.h): score only 2 (fill, record); traceback
-// 2 + 2 * windows (tile_base scan, fill, then per window of row blocks the code recompute and the walk).
+// Planned from (m, n, band, mode, traceback) alone -- and, for a guided pair, its chain, which the host holds.  Launches
+// (include/psa.h): score only 2 (fill, record); traceback 2 + 2 * windows (tile_base scan, fill, then per window of row
+// blocks the code recompute and the walk).
 namespace {
 constexpr size_t kBandedCodeBytes = (size_t)256 << 20;      // window code buffer (16 KiB per tile)
 
@@ -1420,26 +1626,66 @@ long long banded_pair_tpr(int m, int n, int bw, int WW) {
     return std::min(S, (2LL * bw + (long long)R * n / m + 2) / WW + 2);
 }
 
-long long banded_pair_rows_per_window(int m, int n, int bw) {
-    const long long NB = ((long long)m + R - 1) / R, tpr = banded_pair_tpr(m, n, bw, W);
+long long rows_per_window(long long NB, long long tpr) {
     return std::min(NB, std::max(1LL, (long long)(kBandedCodeBytes / ((size_t)tpr * R * 32 * 4))));
 }
-}  // namespace
 
-int psa_launch_banded_pair(psa_ctx* ctx, const uint8_t* d_a, const uint8_t* d_b, int m, int n, int mode, int g, int h, int band,
-                           bool traceback, psa_batch_item* d_item, uint32_t* d_ops, cudaStream_t st) {
-    if (m <= 0 || n <= 0) return psa_fail(ctx, PSA_ERR_ARG, "banded pair path needs m, n >= 1");
-    if (m >= 0x1FFFFF || n >= 0x1FFFFF) return psa_fail(ctx, PSA_ERR_RANGE, "long path: lengths must be < 2^21 - 1");
-    const int bw = (int)std::min<long long>(band, (long long)m + n);
+// The plan's band-dependent numbers: tiles per row block at the walk's width W and at the score-only width 32*KK, and
+// the column span that picks KK.
+struct PairPlan { long long span, tpr_w, tpr16, tpr4; };
+
+PairPlan pair_plan(const Band& B) {
+    return {2LL * B.bw + (long long)R * B.n / B.m, banded_pair_tpr(B.m, B.n, B.bw, W), banded_pair_tpr(B.m, B.n, B.bw, 512),
+            banded_pair_tpr(B.m, B.n, B.bw, 128)};
+}
+
+// A chain's plan is exact: the largest tile count and column span over its row blocks.  The empty chain plans as the
+// diagonal band, so that both take the same launches.
+PairPlan pair_plan(const ChainBand& B) {
+    if (B.K == 0) return pair_plan(Band{B.m, B.n, B.bw});
+    PairPlan p{0, 0, 0, 0};
+    for (int i0 = 0; i0 < B.m; i0 += R) {
+        const int nrows = std::min(R, B.m - i0);
+        p.span = std::max(p.span, (long long)B.hi(i0 + nrows) - B.lo(i0 + 1));
+        p.tpr_w = std::max(p.tpr_w, (long long)B.s_hi(i0, nrows, W) - B.s_lo(i0, W) + 1);
+        p.tpr16 = std::max(p.tpr16, (long long)B.s_hi(i0, nrows, 512) - B.s_lo(i0, 512) + 1);
+        p.tpr4 = std::max(p.tpr4, (long long)B.s_hi(i0, nrows, 128) - B.s_lo(i0, 128) + 1);
+    }
+    return p;
+}
+
+// The kernels of one band type: the diagonal band's, or the chain's.
+template <class BandT> struct PairKernels;
+template <> struct PairKernels<Band> {
+    using Fill = BandedPair;
+    using Tb = BandedPairTb;
+    template <int MODE, int KK, bool TB> static const void* fill() { return (const void*)psa_banded_pair_fill_kernel<MODE, KK, TB>; }
+    template <int MODE> static const void* codes() { return (const void*)psa_banded_pair_codes_kernel<MODE>; }
+    template <int MODE> static const void* walk() { return (const void*)psa_banded_pair_walk_kernel<MODE>; }
+    static const void* tile_base() { return (const void*)psa_banded_tile_base_kernel; }
+};
+template <> struct PairKernels<ChainBand> {
+    using Fill = GuidedPair;
+    using Tb = GuidedPairTb;
+    template <int MODE, int KK, bool TB> static const void* fill() { return (const void*)psa_guided_pair_fill_kernel<MODE, KK, TB>; }
+    template <int MODE> static const void* codes() { return (const void*)psa_guided_pair_codes_kernel<MODE>; }
+    template <int MODE> static const void* walk() { return (const void*)psa_guided_pair_walk_kernel<MODE>; }
+    static const void* tile_base() { return (const void*)psa_guided_tile_base_kernel; }
+};
+
+template <class BandT>
+int launch_banded_pair(psa_ctx* ctx, const uint8_t* d_a, const uint8_t* d_b, int m, int n, int mode, int g, int h, const BandT& band,
+                       const PairPlan& plan, bool traceback, psa_batch_item* d_item, uint32_t* d_ops, cudaStream_t st) {
+    using Ker = PairKernels<BandT>;
+    const int bw = band.bw;
     const bool local = mode == PSA_LOCAL;
     const long long NB = ((long long)m + R - 1) / R;
     const long long resident = (long long)ctx->sm_count * 4 * WPB;
     // Score-only lane width: about (band span)/W row blocks run at once, so narrow <128, 4> tiles (W = 128) keep 4x as many
     // warps busy as <128, 16> ones; the wider lanes (less overhead per cell) only pay once the span gives even them
     // half of the resident warps, i.e. from a span of 256 columns per resident warp.
-    const long long span = 2LL * bw + (long long)R * n / m;
-    const int KK = traceback ? K : (span / 512 >= resident / 2 ? 16 : 4);
-    const long long tpr = banded_pair_tpr(m, n, bw, 32 * KK);
+    const int KK = traceback ? K : (plan.span / 512 >= resident / 2 ? 16 : 4);
+    const long long tpr = traceback ? plan.tpr_w : (KK == 16 ? plan.tpr16 : plan.tpr4);
     // memory: [misc 256: ticket | best @8 | corner @16 | walk state @64] [progress NB ints] then
     //   score only: the recycled H and F rows;  traceback: [tile_base NB x 8 B] [records, banded_slot_bytes' bound] [codes]
     const size_t row = up256((size_t)(n + 1) * 4);
@@ -1448,7 +1694,7 @@ int psa_launch_banded_pair(psa_ctx* ctx, const uint8_t* d_a, const uint8_t* d_b,
     long long rpw = 0;
     if (traceback) {
         ck = banded_slot_bytes(m, n, bw) - 256;              // tile_base + records
-        rpw = banded_pair_rows_per_window(m, n, bw);
+        rpw = rows_per_window(NB, tpr);
         codes = (size_t)rpw * tpr * R * 32 * 4;
         total = o_body + ck + codes;
         size_t free_b = 0, total_b = 0;
@@ -1461,7 +1707,7 @@ int psa_launch_banded_pair(psa_ctx* ctx, const uint8_t* d_a, const uint8_t* d_b,
     if (rc) return rc;
     uint8_t* d = (uint8_t*)ctx->d_work;
     PSA_CUDA_OK(ctx, cudaMemsetAsync(d, 0, o_body, st));
-    BandedPair P;
+    typename Ker::Fill P;
     LongJob& J = P.J;
     J.a = d_a; J.b = d_b; J.m = m; J.n = n; J.g = g; J.h = h; J.mul8 = key_mult(KK);
     J.hbufH = traceback ? nullptr : (int*)(d + o_body); J.hbufF = traceback ? nullptr : (int*)(d + o_body + row); J.hb_stride = 0;
@@ -1469,18 +1715,18 @@ int psa_launch_banded_pair(psa_ctx* ctx, const uint8_t* d_a, const uint8_t* d_b,
     J.progress = (int*)(d + o_pr); J.ticket = (int*)d;
     J.best = (unsigned long long*)(d + 8); J.corner = (int*)(d + 16);
     J.col0 = 0; J.n_total = n; J.row_off = 0; J.start_type = -1; J.end_type = -1;
-    P.bk.B = Band{m, n, bw};
+    P.bk.B = band;
     P.bk.tile_base = traceback ? (long long*)(d + o_body) : nullptr;
     P.bk.rec = traceback ? (int*)(d + o_body + up256((size_t)NB * 8)) : nullptr;
     if (traceback) {
-        psa_banded_tile_base_kernel<<<1, 1024, 0, st>>>(P.bk.B, P.bk.tile_base);
-        PSA_CUDA_OK(ctx, cudaGetLastError());
+        void* targs[] = {&P.bk.B, &P.bk.tile_base};
+        PSA_CUDA_OK(ctx, cudaLaunchKernel(Ker::tile_base(), dim3(1), dim3(1024), targs, 0, st));
         ctx->launches += 1;
     }
     const void* fill;
-    if (traceback) fill = local ? (const void*)psa_banded_pair_fill_kernel<PSA_LOCAL, K, true> : (const void*)psa_banded_pair_fill_kernel<PSA_GLOBAL, K, true>;
-    else if (KK == 16) fill = local ? (const void*)psa_banded_pair_fill_kernel<PSA_LOCAL, 16, false> : (const void*)psa_banded_pair_fill_kernel<PSA_GLOBAL, 16, false>;
-    else fill = local ? (const void*)psa_banded_pair_fill_kernel<PSA_LOCAL, 4, false> : (const void*)psa_banded_pair_fill_kernel<PSA_GLOBAL, 4, false>;
+    if (traceback) fill = local ? Ker::template fill<PSA_LOCAL, K, true>() : Ker::template fill<PSA_GLOBAL, K, true>();
+    else if (KK == 16) fill = local ? Ker::template fill<PSA_LOCAL, 16, false>() : Ker::template fill<PSA_GLOBAL, 16, false>();
+    else fill = local ? Ker::template fill<PSA_LOCAL, 4, false>() : Ker::template fill<PSA_GLOBAL, 4, false>();
     int per_sm = 0;
     PSA_CUDA_OK(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fill, WPB * 32, 0));
     if (ctx->opt.long_ctas_per_sm > 0) per_sm = std::max(1, std::min(per_sm, ctx->opt.long_ctas_per_sm));
@@ -1491,12 +1737,13 @@ int psa_launch_banded_pair(psa_ctx* ctx, const uint8_t* d_a, const uint8_t* d_b,
     void* fargs[] = {&P};
     PSA_CUDA_OK(ctx, cudaLaunchKernel(fill, dim3(grid), dim3(WPB * 32), fargs, 0, st));
     ctx->launches += 1;
-    BandedPairTb T{J, P.bk, traceback ? (uint32_t*)(d + o_body + ck) : nullptr, (int)tpr, 0, (int)NB,
-                   (BandedWalk*)(d + 64), d_item, traceback ? d_ops : nullptr};
+    typename Ker::Tb T{J, P.bk, traceback ? (uint32_t*)(d + o_body + ck) : nullptr, (int)tpr, 0, (int)NB,
+                        (BandedWalk*)(d + 64), d_item, traceback ? d_ops : nullptr};
+    void* wargs[] = {&T};
+    const void* codes_k = local ? Ker::template codes<PSA_LOCAL>() : Ker::template codes<PSA_GLOBAL>();
+    const void* walk_k = local ? Ker::template walk<PSA_LOCAL>() : Ker::template walk<PSA_GLOBAL>();
     if (!traceback) {
-        if (local) psa_banded_pair_walk_kernel<PSA_LOCAL><<<1, 32, 0, st>>>(T);
-        else psa_banded_pair_walk_kernel<PSA_GLOBAL><<<1, 32, 0, st>>>(T);
-        PSA_CUDA_OK(ctx, cudaGetLastError());
+        PSA_CUDA_OK(ctx, cudaLaunchKernel(walk_k, dim3(1), dim3(32), wargs, 0, st));
         ctx->launches += 1;
         return PSA_OK;
     }
@@ -1504,17 +1751,31 @@ int psa_launch_banded_pair(psa_ctx* ctx, const uint8_t* d_a, const uint8_t* d_b,
         T.rb_hi = (int)hi; T.rb_lo = (int)std::max(0LL, hi - rpw);
         const long long units = (long long)(T.rb_hi - T.rb_lo) * tpr;
         const unsigned blocks = (unsigned)((units + CODES_WPB - 1) / CODES_WPB);
-        if (local) {
-            psa_banded_pair_codes_kernel<PSA_LOCAL><<<blocks, CODES_WPB * 32, 0, st>>>(T);
-            psa_banded_pair_walk_kernel<PSA_LOCAL><<<1, 32, 0, st>>>(T);
-        } else {
-            psa_banded_pair_codes_kernel<PSA_GLOBAL><<<blocks, CODES_WPB * 32, 0, st>>>(T);
-            psa_banded_pair_walk_kernel<PSA_GLOBAL><<<1, 32, 0, st>>>(T);
-        }
-        PSA_CUDA_OK(ctx, cudaGetLastError());
+        PSA_CUDA_OK(ctx, cudaLaunchKernel(codes_k, dim3(blocks), dim3(CODES_WPB * 32), wargs, 0, st));
+        PSA_CUDA_OK(ctx, cudaLaunchKernel(walk_k, dim3(1), dim3(32), wargs, 0, st));
         ctx->launches += 2;
     }
     return PSA_OK;
+}
+}  // namespace
+
+int psa_launch_banded_pair(psa_ctx* ctx, const uint8_t* d_a, const uint8_t* d_b, int m, int n, int mode, int g, int h, int band,
+                           bool traceback, psa_batch_item* d_item, uint32_t* d_ops, cudaStream_t st) {
+    if (m <= 0 || n <= 0) return psa_fail(ctx, PSA_ERR_ARG, "banded pair path needs m, n >= 1");
+    if (m >= 0x1FFFFF || n >= 0x1FFFFF) return psa_fail(ctx, PSA_ERR_RANGE, "long path: lengths must be < 2^21 - 1");
+    const Band B{m, n, (int)std::min<long long>(band, (long long)m + n)};
+    return launch_banded_pair(ctx, d_a, d_b, m, n, mode, g, h, B, pair_plan(B), traceback, d_item, d_ops, st);
+}
+
+int psa_launch_guided_pair(psa_ctx* ctx, const uint8_t* d_a, const uint8_t* d_b, int m, int n, int mode, int g, int h, int band,
+                           const psa_anchor* h_anchors, const psa_anchor* d_anchors, int n_anchors, bool traceback,
+                           psa_batch_item* d_item, uint32_t* d_ops, cudaStream_t st) {
+    if (m <= 0 || n <= 0) return psa_fail(ctx, PSA_ERR_ARG, "guided pair path needs m, n >= 1");
+    if (m >= 0x1FFFFF || n >= 0x1FFFFF) return psa_fail(ctx, PSA_ERR_RANGE, "long path: lengths must be < 2^21 - 1");
+    const int bw = (int)std::min<long long>(band, (long long)m + n);
+    const PairPlan plan = pair_plan(ChainBand{m, n, bw, h_anchors, n_anchors});
+    return launch_banded_pair(ctx, d_a, d_b, m, n, mode, g, h, ChainBand{m, n, bw, d_anchors, n_anchors}, plan, traceback, d_item,
+                              d_ops, st);
 }
 
 // ---- partition finder (SURVEY 8 f-3; the role of sequence_alignment/partial.cpp:81-163) ---------------------------

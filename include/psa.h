@@ -268,6 +268,60 @@ int psa_align_long_banded_device(psa_ctx* ctx, const uint8_t* d_a, const uint8_t
                                  int g, int h, int band, unsigned flags, psa_batch_item* d_item, uint32_t* d_ops,
                                  size_t ops_words, void* cuda_stream);
 
+/* ---- banded alignment along an anchor chain -------------------------------------------------------
+ * The band of psa_align_batch_banded / psa_align_pair_banded, centred on a caller-supplied chain of anchors instead of
+ * the straight line from (0,0) to (m,n): what a mapper knows after seeding and chaining.  An anchor (i, j) is the
+ * boundary point after A[1..i] and B[1..j], the coordinates of the DP cells: a seed match of length L at 0-based
+ * positions x in A and y in B gives the anchors (x, y) and (x+L, y+L).
+ * For a pair with m, n >= 1 and anchors P_1 .. P_K the guide is the polyline P_0 = (0,0), P_1, ..., P_K, P_{K+1} = (m,n).
+ *   valid chain:  0 <= i_k <= m and 0 <= j_k <= n, both coordinates non-decreasing along the chain (equal points,
+ *                 horizontal runs (equal i) and vertical runs (equal j) are allowed)
+ *   guide columns of row i, [cmin(i), cmax(i)]: if chain points lie on row i, the j of the first and the j of the last
+ *                 of them; otherwise i lies strictly inside one segment P_k -> P_{k+1} (i_k < i < i_{k+1}) and
+ *                 cmin(i) = cmax(i) = j_k + floor((i - i_k)(j_{k+1} - j_k) / (i_{k+1} - i_k))
+ *   band:         lo(i) = max(0, cmin(i) - band), hi(i) = min(n, cmax(i) + band); cell (i, j) exists iff lo(i) <= j <= hi(i)
+ * Everything else is psa_align_batch_banded's: out-of-band cells, borders (row 0's gap border up to hi(0), column 0's
+ * where lo(i) = 0), both modes, tie rules, traceback order, op words, the no-path record (PSA_NEG_INF corners and score,
+ * end state 1, aln_len 0, no op words) and, for m = 0 or n = 0, psa_align_batch's record.  An empty chain (K = 0) is
+ * the diagonal band: results byte-identical to psa_align_batch_banded / psa_align_pair_banded.  A horizontal run widens
+ * its row to cover the jump, so an insertion of any size is representable at any band; with band >= max(m, n) every
+ * cell exists and the results equal psa_align_batch's whatever the chain.  Flags, band >= 0, lengths < 2^21 - 1, buffer
+ * layouts, the capacity rule and the score-range rule (global with band < max(M, N): g(M+N+2) + h(min(M, N) + 3) + M + N
+ * < 2^28) are psa_align_batch_banded's.  Checkpoint memory keeps that entry's bound for every valid chain.
+ *
+ * psa_align_batch_guided: host buffers; pair k uses anchors[off_anc[k] .. off_anc[k] + n_anc[k]).  Every chain is
+ *   checked on the host (n_anc[k] >= 0, off_anc[k] >= 0, off_anc[k] + n_anc[k] <= total_anc, a valid chain for the
+ *   pair's lengths, m = 0 or n = 0 included); a failure is PSA_ERR_ARG naming the pair and the anchor.
+ * psa_align_batch_guided_device: every array in device memory (d_anchors, d_off_anc and d_n_anc non-null), asynchronous
+ *   on cuda_stream, planned from n_pairs, max_len_a, max_len_b and band alone.  It cannot return a chain error: a pair
+ *   whose chain is invalid gets the REJECTED record -- t1 = t2 = t3 = score = PSA_NEG_INF, end_state 0 (which no other
+ *   record has), end / start cells 0, aln_len 0, no op words written -- and reads or writes nothing of the other pairs.
+ * psa_align_pair_guided: host strings, fills *out as psa_align_pair_banded does, on the same whole-GPU kernels; the
+ *   chain is checked on the host (PSA_ERR_ARG naming the anchor; anchors may be NULL when n_anchors = 0) and plans the
+ *   call exactly.  The call issues
+ *     score only:  2 kernel launches (fill, record)
+ *     traceback:   2 + 2 * ceil(NB / rpw) launches, rpw = min(NB, max(1, floor(2^28 / (tpr * 16384)))), NB = ceil(m/128),
+ *                  with tpr = psa_align_pair_banded's for an empty chain and otherwise the largest number of 256-column
+ *                  tiles a row block touches: the maximum over row blocks (rows i0+1 .. i0+r, r = min(128, m - i0)) of
+ *                  s_hi - s_lo + 1, s_lo = floor((max(1, lo(i0+1)) - 1) / 256), s_hi = max(s_lo, floor((max(1, hi(i0+r)) - 1) / 256)).
+ *   PSA_ERR_NOMEM as psa_align_pair_banded: if checkpoints and codes exceed half of the free device memory. */
+typedef struct {
+    int32_t i, j;
+} psa_anchor;
+
+int psa_align_batch_guided(psa_ctx* ctx, const uint8_t* bases_a, const int64_t* off_a, const int32_t* len_a,
+                           const uint8_t* bases_b, const int64_t* off_b, const int32_t* len_b, size_t n_pairs,
+                           size_t bytes_a, size_t bytes_b, const psa_anchor* anchors, const int64_t* off_anc,
+                           const int32_t* n_anc, size_t total_anc, int mode, int g, int h, int band, unsigned flags,
+                           psa_batch_item* items, uint32_t* ops, size_t ops_stride_words);
+int psa_align_batch_guided_device(psa_ctx* ctx, const uint8_t* d_bases_a, const int64_t* d_off_a, const int32_t* d_len_a,
+                                  const uint8_t* d_bases_b, const int64_t* d_off_b, const int32_t* d_len_b, size_t n_pairs,
+                                  int max_len_a, int max_len_b, const psa_anchor* d_anchors, const int64_t* d_off_anc,
+                                  const int32_t* d_n_anc, int mode, int g, int h, int band, unsigned flags,
+                                  psa_batch_item* d_items, uint32_t* d_ops, size_t ops_stride_words, void* cuda_stream);
+int psa_align_pair_guided(psa_ctx* ctx, const char* a, const char* b, size_t m, size_t n, const psa_anchor* anchors,
+                          size_t n_anchors, int mode, int g, int h, int band, unsigned flags, psa_result* out);
+
 /* ---- one long pair over several GPUs (config 4) ---------------------------------------------
  * Score-only fill of ONE pair by the column-stationary systolic kernel: the matrix is cut into panels of
  * panel_strips * psa_long_strip_columns() columns (one warp per strip -- 256 columns, 8 per lane -- every strip
